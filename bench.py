@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the octree hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload): the "Sponza 1024^3 @4K" configuration of BASELINE.json
 on the procedural atrium stand-in (sponza.obj is absent from the reference checkout,
@@ -32,6 +32,12 @@ per step.  A step = one frame = one launch of the persistent ray kernel per GPU.
 
 --impl reference times the reference's own CPU implementation on the same workload
 (bounded sample per step) and prints the same JSON shape with "impl": "reference".
+
+--dump-outputs DIR writes what the last timed step computed, for comparing two builds output for
+output: the film and the 16-byte hit records of a fixed, seeded sample of the frame's pixels
+(DUMP_PIXELS of them, every sample ray of each), as DIR/<name>.npy in float32 / float64.
+The orbit workloads move the camera every step (the last timed step shows camera (steps - 1) % 64),
+so their dumps depend on --steps; the fixed-camera workloads dump the same frame for any --steps.
 """
 from __future__ import annotations
 
@@ -290,6 +296,24 @@ def make_cams(capi, wl, cam10, nx, ny, spp):
     return cams
 
 
+DUMP_PIXELS = 1 << 18  # pixels of the --dump-outputs sample: about 34 MB at 4 spp
+DUMP_SEED = 20190722
+
+
+def sample_outputs(torch, film, hit_rows, ny, nx, spp):
+    """--dump-outputs: the film values and the hit records (vrt_hit16: leaf, tri, t, hit) of every sample ray of a
+    fixed, seeded set of pixels.  film: [ny, nx, 3] float32 on the device; hit_rows: film-ordered [>= ny, nx*spp*4]
+    int32 on the device.  Integer fields are widened to float64 (exact), so every array is float32 or float64."""
+    n = min(DUMP_PIXELS, ny * nx)
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(ny * nx, n, replace=False))
+    sel = torch.from_numpy(idx).to(film.device)
+    px = film.reshape(ny * nx, 3).index_select(0, sel).cpu().numpy()
+    rec = hit_rows[:ny].reshape(ny * nx, spp, 4).index_select(0, sel).cpu().numpy().view(np.uint32)
+    return {"pixel_index": idx.astype(np.float64), "film": px.astype(np.float32),
+            "hit_leaf": rec[..., 0].astype(np.float64), "hit_tri": rec[..., 1].astype(np.float64),
+            "hit_t": rec[..., 2].view(np.float32).copy(), "hit_flag": rec[..., 3].astype(np.float64)}
+
+
 def config5_block(args, capi, vdist, torch, world, rank, dev, tri, nrm):
     """BASELINE.json configs[4] inside the default run (every rank calls this): the same triangles voxelized at 2048^3,
     7680x4320 x 4 spp, camera orbit, primary rays + one shadow ray per hit, bands over all GPUs, frames assembled on
@@ -509,6 +533,17 @@ def run_ours(args):
     # timed region is the CUDA-event time of the region / launches
     kern_ms = ms_per_step
     value = rays_per_step / (ms_per_step * 1e-3) / 1e6
+
+    # ---- --dump-outputs: the last timed step's frame and hit records, before anything below overwrites them ----
+    if args.dump_outputs:
+        k_last = (args.steps - 1) & 1
+        hit_rows = hits[k_last] if world == 1 else vdist.gather_rows(hits[k_last], ny)  # collective
+        if rank == 0:
+            film = fg.frame if use_gather else pf.frame(k_last)
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in sample_outputs(torch, film, hit_rows, ny, nx, spp).items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
+        del hit_rows
 
     # ---- the dominant kernel alone: one stream, CUDA events around every launch (no overlap with a neighbour) ----
     tree.set_stream(stream.cuda_stream)
@@ -859,7 +894,14 @@ def main():
     ap.add_argument("--no-gi", action="store_true", help="skip the GI rows (splat/filter/cone-trace film)")
     ap.add_argument("--no-build-soup", action="store_true", help="skip the 2 M-triangle soup build (BASELINE config 4)")
     ap.add_argument("--no-config5", action="store_true", help="skip the BASELINE config 5 block (2048^3, 8K orbit + shadow rays)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the film and hit records of a seeded sample of the last step's "
+                         "pixels to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
