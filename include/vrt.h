@@ -225,7 +225,8 @@ int vrt_render_camera_async(const vrt_tree* tree, const vrt_camera* cam,
                             const vrt_shade* sh, int x0, int y0, int x1, int y1,
                             float* film_rgb);
 /* Film export encodings, fused into the store of a finished pixel (every film-writing entry point of the handle:
- * vrt_render_camera*, vrt_render_bands*, vrt_frame_bands*, vrt_gi_render_camera*, vrt_mgpu_render*).  The reference
+ * vrt_render_camera*, vrt_render_bands*, vrt_frame_bands*, vrt_gi_render_camera*, vrt_gi_render_bands_async,
+ * vrt_mgpu_render*, vrt_mgpu_gi_render*).  The reference
  * keeps a float film and converts it after the render loop; on a multi-GPU node the float film is what saturates
  * the host's device->host ingest, so the conversion runs in the ray kernel and the encoded film crosses PCIe:
  *   VRT_FILM_F32   [ny][nx][3] float            Film::to_float_array, camera.cc:50-63 (default)
@@ -273,7 +274,8 @@ int vrt_render_bands_async(const vrt_tree* tree, const vrt_camera* cam, const vr
  * the blob), then per frame deal the film's 8-row bands round-robin to the devices.  Every device runs the
  * vrt_render_bands_async pipeline and DMA-copies its bands to their final rows of film_rgb_full (pinned host
  * memory, e.g. vrt_host_register'ed); vrt_mgpu_sync (or the synchronous vrt_mgpu_render) completes the frame.
- * The source tree stays the caller's and may be freed after vrt_mgpu_create. */
+ * The source tree stays the caller's and may be freed after vrt_mgpu_create.  vrt_mgpu_create copies the
+ * geometry only; materials and the GI state of the replicas are set through the vrt_mgpu_* GI calls below. */
 typedef struct vrt_mgpu vrt_mgpu;
 int vrt_mgpu_create(const vrt_tree* tree, int num_devices, const int* devices, vrt_mgpu** out);
 int vrt_mgpu_num_devices(const vrt_mgpu* m);
@@ -357,6 +359,38 @@ int vrt_gi_render_camera(const vrt_tree* tree, const vrt_camera* cam, const floa
                          int y0, int x1, int y1, float* film_rgb);
 int vrt_gi_render_camera_dev(const vrt_tree* tree, const vrt_camera* cam, const float kd[3], float res,
                              int x0, int y0, int x1, int y1, float* d_film_rgb);
+/* The GI film of vrt_gi_render_camera in the banded, pipelined form of vrt_render_bands_async: this handle's
+ * bands of the film are cone-traced into one of two device band buffers (kernels alternating between two
+ * streams) and DMA-copied to their final rows of film_rgb_full, the FULL [ny][nx][...] host frame in the
+ * handle's film format (pinned; on a multi-process node a shared mapping every rank has registered).  kd is a
+ * host pointer.  Returns once the frame is ENQUEUED; the frame is complete after vrt_tree_sync() (and, with
+ * several ranks, a process barrier).  Requires vrt_gi_init (VRT_ERR_ARG otherwise).  bands = {ny, 0, 1} is the
+ * single-GPU pipelined GI loop (main.cc:117-123 frame after frame): alternate between two host frames.
+ * vrt_set_materials, vrt_gi_init, vrt_gi_splat_camera and vrt_gi_filter may be called between enqueued frames
+ * without a vrt_tree_sync: they run after every frame enqueued before them and before every frame after. */
+int vrt_gi_render_bands_async(const vrt_tree* tree, const vrt_camera* cam, const float kd[3], float res,
+                              const vrt_bands* bands, float* film_rgb_full);
+/* The GI rows on the replicas of a vrt_mgpu (main.cc:75-126 over N devices).  vrt_mgpu_create copies the
+ * geometry only: materials and the GI state are set through these calls, each of which runs the single-device
+ * call on every replica (host pointers, like the single-device calls).  The light pass runs on every replica --
+ * the splat is deterministic, so every replica holds the same bits -- and the replicas work concurrently.
+ *   vrt_mgpu_set_materials    vrt_set_materials on every replica
+ *   vrt_mgpu_gi_init          vrt_gi_init                  (main.cc:75)
+ *   vrt_mgpu_gi_splat_camera  vrt_gi_splat_camera          (main.cc:81-96, the light-map render_mt loop)
+ *   vrt_mgpu_gi_filter        vrt_gi_filter                (gi::cone_trace_init_filter, main.cc:97)
+ *   vrt_mgpu_gi_render_async  the GI film (main.cc:117-123): the 8-row bands dealt round-robin, each replica's
+ *                             through vrt_gi_render_bands_async into film_rgb_full (pinned host memory); the
+ *                             frame is complete after vrt_mgpu_sync.  Alternate between two host frames.
+ *   vrt_mgpu_gi_render        vrt_mgpu_gi_render_async + vrt_mgpu_sync */
+int vrt_mgpu_set_materials(vrt_mgpu* m, const float* tri_uv, const uint32_t* tri_mtl, uint32_t num_mtl,
+                           const float* kd, const int32_t* mtl_tex, uint32_t num_tex, const vrt_texture* tex);
+int vrt_mgpu_gi_init(vrt_mgpu* m);
+int vrt_mgpu_gi_splat_camera(vrt_mgpu* m, const vrt_camera* light_cam, const float kd[3]);
+int vrt_mgpu_gi_filter(vrt_mgpu* m);
+int vrt_mgpu_gi_render_async(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_rgb_full);
+int vrt_mgpu_gi_render(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_rgb_full);
+/* vrt_mean_kernel_ms of replica `index` (0 for a bad index): the per-device balance of a multi-GPU frame loop */
+double vrt_mgpu_mean_kernel_ms(vrt_mgpu* m, int index, int last_n);
 
 /* out = {node expansions cross-checked against the slab expansion, mismatches}; counts only in
  * a library built with -DVRT_PARAM_CHECK (tests), {0,0} otherwise. */

@@ -72,6 +72,8 @@ SYMBOLS = [
     "vrt_film_pixel_bytes", "vrt_hdr_file", "vrt_mgpu_set_film_format", "vrt_film_encode", "vrt_set_materials", "vrt_albedo", "vrt_gi_init", "vrt_gi_splat_camera", "vrt_gi_filter",
     "vrt_gi_get_level", "vrt_gi_cone_trace", "vrt_gi_render_camera", "vrt_gi_render_camera_dev", "vrt_tribox_batch",
     "vrt_tri_overlap_aabb_batch", "vrt_raytri_batch", "vrt_aabb_isect_batch",
+    "vrt_gi_render_bands_async", "vrt_mgpu_set_materials", "vrt_mgpu_gi_init", "vrt_mgpu_gi_splat_camera",
+    "vrt_mgpu_gi_filter", "vrt_mgpu_gi_render_async", "vrt_mgpu_gi_render", "vrt_mgpu_mean_kernel_ms",
 ]
 
 _lib = None
@@ -164,6 +166,15 @@ def load(build_if_missing: bool = True):
     L.vrt_gi_cone_trace.argtypes = [vp, vp, vp, u64, f32, vp]
     L.vrt_gi_render_camera.argtypes = [vp, C.POINTER(vrt_camera), vp, f32, i32, i32, i32, i32, vp]
     L.vrt_gi_render_camera_dev.argtypes = L.vrt_gi_render_camera.argtypes
+    L.vrt_gi_render_bands_async.argtypes = [vp, C.POINTER(vrt_camera), vp, f32, C.POINTER(vrt_bands), vp]
+    L.vrt_mgpu_set_materials.argtypes = [vp, vp, vp, C.c_uint32, vp, vp, C.c_uint32, vp]
+    L.vrt_mgpu_gi_init.argtypes = [vp]
+    L.vrt_mgpu_gi_splat_camera.argtypes = [vp, C.POINTER(vrt_camera), vp]
+    L.vrt_mgpu_gi_filter.argtypes = [vp]
+    L.vrt_mgpu_gi_render_async.argtypes = [vp, C.POINTER(vrt_camera), vp, f32, vp]
+    L.vrt_mgpu_gi_render.argtypes = L.vrt_mgpu_gi_render_async.argtypes
+    L.vrt_mgpu_mean_kernel_ms.restype = C.c_double
+    L.vrt_mgpu_mean_kernel_ms.argtypes = [vp, i32, i32]
     L.vrt_tree_sync.argtypes = [vp]
     L.vrt_mean_kernel_ms.restype = C.c_double
     L.vrt_mean_kernel_ms.argtypes = [vp, i32]
@@ -459,16 +470,7 @@ class Octree:
     # ---- materials / textures (SURVEY.md 8f row 3) -------------------------------
     def set_materials(self, tri_uv, tri_mtl, kd, mtl_tex, textures):
         """textures: list of uint8 arrays [h, w, channels] (as stbi_load returns them)."""
-        tri_uv = np.ascontiguousarray(tri_uv, np.float32).reshape(-1, 6)
-        tri_mtl = np.ascontiguousarray(tri_mtl, np.uint32)
-        kd = np.ascontiguousarray(kd, np.float32).reshape(-1, 3)
-        mtl_tex = np.ascontiguousarray(mtl_tex, np.int32)
-        texs = [np.ascontiguousarray(t, np.uint8) for t in textures]
-        arr = (vrt_texture * max(len(texs), 1))()
-        for i, t in enumerate(texs):
-            arr[i] = vrt_texture(t.shape[1], t.shape[0], t.shape[2], t.ctypes.data)
-        _check(load().vrt_set_materials(self._h, _ptr(tri_uv), _ptr(tri_mtl), len(kd), _ptr(kd), _ptr(mtl_tex), len(texs),
-                                        C.cast(arr, C.c_void_p)))
+        _set_materials(load().vrt_set_materials, self._h, tri_uv, tri_mtl, kd, mtl_tex, textures)
 
     def albedo(self, tri, pos, kd_default=(0.8, 0.8, 0.8)):
         tri = np.ascontiguousarray(tri, np.uint32)
@@ -512,6 +514,15 @@ class Octree:
         _check(load().vrt_gi_render_camera(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)), x0, y0, x1, y1,
                                            _ptr(out)))
         return out
+
+    def gi_render_bands_async(self, cam: Camera, kd, res, host_frame_ptr, band_h, band_first, band_stride):
+        """The GI film's bands `band_first`, `band_first + band_stride`, ... DMA-copied to their final rows of the
+        full (pinned, possibly shared between the ranks) host frame in the handle's film format; asynchronous, see
+        sync().  (band_h = ny, 0, 1: the whole film as one pipelined frame.)"""
+        kd = np.ascontiguousarray(kd, np.float32)
+        b = vrt_bands(int(band_h), int(band_first), int(band_stride))
+        _check(load().vrt_gi_render_bands_async(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)), C.byref(b),
+                                                C.c_void_p(int(host_frame_ptr))))
 
     def gi_render_dev(self, cam: Camera, kd, res, d_film_ptr, rect=None):
         x0, y0, x1, y1 = rect if rect else (0, 0, cam.nx, cam.ny)
@@ -589,10 +600,55 @@ class MultiGpu:
     def set_film_format(self, fmt):
         _check(load().vrt_mgpu_set_film_format(self._h, FILM_FORMATS[fmt] if isinstance(fmt, str) else int(fmt)))
 
+    # ---- GI film on the replicas (the replicas hold geometry only until these calls) ----------------------------
+    def set_materials(self, tri_uv, tri_mtl, kd, mtl_tex, textures):
+        """Octree.set_materials on every replica."""
+        _set_materials(load().vrt_mgpu_set_materials, self._h, tri_uv, tri_mtl, kd, mtl_tex, textures)
+
+    def gi_init(self):
+        _check(load().vrt_mgpu_gi_init(self._h))
+
+    def gi_splat(self, light_cam: Camera, kd):
+        """The light pass on every replica (deterministic: every replica holds the same bits)."""
+        kd = np.ascontiguousarray(kd, np.float32)
+        _check(load().vrt_mgpu_gi_splat_camera(self._h, C.byref(light_cam.c), _ptr(kd)))
+
+    def gi_filter(self):
+        _check(load().vrt_mgpu_gi_filter(self._h))
+
+    def gi_render_async(self, cam: Camera, kd, res, host_frame_ptr):
+        """Enqueue one GI film: 8-row bands round-robin over the replicas, each DMA-copied to its final rows of the
+        (pinned) host frame in the replicas' film format; call sync() before reading."""
+        kd = np.ascontiguousarray(kd, np.float32)
+        _check(load().vrt_mgpu_gi_render_async(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)),
+                                               C.c_void_p(int(host_frame_ptr))))
+
+    def gi_render(self, cam: Camera, kd, res, host_frame_ptr):
+        kd = np.ascontiguousarray(kd, np.float32)
+        _check(load().vrt_mgpu_gi_render(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)),
+                                         C.c_void_p(int(host_frame_ptr))))
+
+    def mean_kernel_ms(self, index, last_n):
+        """Mean device time of the last `last_n` kernels of replica `index` (waits for them)."""
+        return float(load().vrt_mgpu_mean_kernel_ms(self._h, int(index), int(last_n)))
+
     def close(self):
         if self._h:
             load().vrt_mgpu_free(self._h)
             self._h = None
+
+
+def _set_materials(fn, h, tri_uv, tri_mtl, kd, mtl_tex, textures):
+    """vrt_set_materials / vrt_mgpu_set_materials on handle `h` (textures: uint8 arrays [h, w, channels])."""
+    tri_uv = np.ascontiguousarray(tri_uv, np.float32).reshape(-1, 6)
+    tri_mtl = np.ascontiguousarray(tri_mtl, np.uint32)
+    kd = np.ascontiguousarray(kd, np.float32).reshape(-1, 3)
+    mtl_tex = np.ascontiguousarray(mtl_tex, np.int32)
+    texs = [np.ascontiguousarray(t, np.uint8) for t in textures]
+    arr = (vrt_texture * max(len(texs), 1))()
+    for i, t in enumerate(texs):
+        arr[i] = vrt_texture(t.shape[1], t.shape[0], t.shape[2], t.ctypes.data)
+    _check(fn(h, _ptr(tri_uv), _ptr(tri_mtl), len(kd), _ptr(kd), _ptr(mtl_tex), len(texs), C.cast(arr, C.c_void_p)))
 
 
 def debug_hull_stats():

@@ -5,6 +5,8 @@
 // checkout), or "v/vn/f" triangles from an OBJ given on the command line.
 //   demo_main [out.bmp] [max_depth] [nx] [ny] [scene.obj]
 // With --dump <file> it also writes (hit,tri,cell,pos,nrm) per ray for the parity test.
+// With --gi <file> it also writes main.cc's cone-traced GI film (float, plus <file>.hdr); with --gi-devices 0,0,...
+// as well, the same film rendered through gi::MultiGpu on those devices goes to <file>.mgpu.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -121,11 +123,21 @@ int main(int argc, char** argv)
         const char* out = "demo.bmp";
         const char* dump = nullptr;
         const char* gi_dump = nullptr;  // --gi <file>: also run main.cc's light map + filter + cone-traced film
+        std::vector<int> gi_devices;    // --gi-devices 0,0,...: the GI film again on these replicas -> <file>.mgpu
         const char* obj = nullptr;
         int depth = 6, nx = 1024, ny = 1024, pos = 0;  // main.cc:34-35,67
         for (int i = 1; i < argc; ++i) {
                 if (!std::strcmp(argv[i], "--dump") && i + 1 < argc) { dump = argv[++i]; continue; }
                 if (!std::strcmp(argv[i], "--gi") && i + 1 < argc) { gi_dump = argv[++i]; continue; }
+                if (!std::strcmp(argv[i], "--gi-devices") && i + 1 < argc) {
+                        for (const char* p = argv[++i]; *p;) {
+                                char* end = nullptr;
+                                gi_devices.push_back((int)std::strtol(p, &end, 10));
+                                p = (*end == ',') ? end + 1 : end;
+                                if (end == p && *p) { std::fprintf(stderr, "bad --gi-devices list\n"); return 1; }
+                        }
+                        continue;
+                }
                 switch (pos++) {
                 case 0: out = argv[i]; break;
                 case 1: depth = std::atoi(argv[i]); break;
@@ -189,6 +201,19 @@ int main(int argc, char** argv)
                         FILE* f = std::fopen(gi_dump, "wb");
                         std::fwrite(d.data(), sizeof(float), d.size(), f);
                         std::fclose(f);
+                        if (!gi_devices.empty()) {
+                                // the same three GI statements on the replicas of gi::MultiGpu
+                                std::printf("GI film on %zu replicas...\n", gi_devices.size());
+                                gi::MultiGpu replicas(&root, gi_devices);
+                                light_map_gpu(sfilm, scam, replicas, 4, kd);
+                                gi::cone_trace_init_filter(replicas);
+                                Film mfilm(1.f, 1.f, nx, ny);
+                                render_gi_gpu(&mfilm, cam, replicas, 4, kd, res);
+                                const auto md = mfilm.to_float_array();
+                                FILE* mf = std::fopen((std::string(gi_dump) + ".mgpu").c_str(), "wb");
+                                std::fwrite(md.data(), sizeof(float), md.size(), mf);
+                                std::fclose(mf);
+                        }
                 }
                 std::printf("success.\n");
         } catch (const std::exception& e) {

@@ -333,6 +333,18 @@ Vec3 cone_trace(const VoxelOctree& root, const ISect& isect, float min_voxel_siz
         cone_trace_batch(root, { isect }, min_voxel_size, &out);
         return out[0];
 }
+
+MultiGpu::MultiGpu(const VoxelOctree* root, const std::vector<int>& devices)
+{
+        check(vrt_mgpu_create(gi_tree(root, "gi::MultiGpu"), (int)devices.size(), devices.data(), &m_), "gi::MultiGpu");
+}
+
+MultiGpu::~MultiGpu() { vrt_mgpu_free(m_); }
+
+void cone_trace_init_filter(MultiGpu& replicas)
+{
+        check(vrt_mgpu_gi_filter(replicas.native()), "cone_trace_init_filter");
+}
 }  // namespace gi
 
 void light_map_gpu(const Film& sfilm, Camera& scam, gi::VoxelOctree* root, int spp, const jql::Vec3& kd)
@@ -352,10 +364,34 @@ void render_gi_gpu(Film* film, Camera& cam, gi::VoxelOctree* root, int spp, cons
         check(vrt_gi_render_camera(t, &c, k, res, 0, 0, film->nx, film->ny, &film->data()->x), "render_gi_gpu");
 }
 
-void set_materials_gpu(gi::VoxelOctree* root, const std::vector<jql::Vec2>& uv, const std::vector<std::uint32_t>& tri_material,
-                       const std::vector<GpuMaterial>& materials, const std::vector<GpuTexture>& textures)
+void light_map_gpu(const Film& sfilm, Camera& scam, gi::MultiGpu& replicas, int spp, const jql::Vec3& kd)
 {
-        vrt_tree* t = gi::gi_tree(root, "set_materials_gpu");
+        const vrt_camera c = scam.native(sfilm, spp);
+        const float k[3] = { kd.x, kd.y, kd.z };
+        check(vrt_mgpu_gi_init(replicas.native()), "light_map_gpu");
+        check(vrt_mgpu_gi_splat_camera(replicas.native(), &c, k), "light_map_gpu");
+}
+
+void render_gi_gpu(Film* film, Camera& cam, gi::MultiGpu& replicas, int spp, const jql::Vec3& kd, float res)
+{
+        const vrt_camera c = cam.native(*film, spp);
+        const float k[3] = { kd.x, kd.y, kd.z };
+        // the devices DMA their bands into the film; page-locked for the call, they copy in parallel (if the range
+        // cannot be locked, e.g. because the caller already did, the copies still land, staged by the driver)
+        float* dst = &film->data()->x;
+        const uint64_t bytes = (uint64_t)film->nx * film->ny * 3 * sizeof(float);
+        const bool locked = vrt_host_register(dst, bytes) == VRT_OK;
+        const int rc = vrt_mgpu_gi_render(replicas.native(), &c, k, res, dst);
+        if (locked)
+                vrt_host_unregister(dst);
+        check(rc, "render_gi_gpu");
+}
+
+// vrt_set_materials / vrt_mgpu_set_materials with the mirror's material records
+template <class H, class Fn>
+static void set_materials_native(Fn fn, H* h, const std::vector<jql::Vec2>& uv, const std::vector<std::uint32_t>& tri_material,
+                                 const std::vector<GpuMaterial>& materials, const std::vector<GpuTexture>& textures)
+{
         std::vector<float> kd(3 * materials.size());
         std::vector<int32_t> mt(materials.size());
         for (size_t m = 0; m < materials.size(); ++m) {
@@ -367,9 +403,21 @@ void set_materials_gpu(gi::VoxelOctree* root, const std::vector<jql::Vec2>& uv, 
         std::vector<vrt_texture> tx(textures.size());
         for (size_t i = 0; i < textures.size(); ++i)
                 tx[i] = vrt_texture{ textures[i].width, textures[i].height, textures[i].channels, textures[i].data };
-        check(vrt_set_materials(t, uv.empty() ? nullptr : &uv[0].x, tri_material.data(), (uint32_t)materials.size(), kd.data(),
-                                mt.data(), (uint32_t)tx.size(), tx.data()),
+        check(fn(h, uv.empty() ? nullptr : &uv[0].x, tri_material.data(), (uint32_t)materials.size(), kd.data(), mt.data(),
+                 (uint32_t)tx.size(), tx.data()),
               "set_materials_gpu");
+}
+
+void set_materials_gpu(gi::VoxelOctree* root, const std::vector<jql::Vec2>& uv, const std::vector<std::uint32_t>& tri_material,
+                       const std::vector<GpuMaterial>& materials, const std::vector<GpuTexture>& textures)
+{
+        set_materials_native(vrt_set_materials, gi::gi_tree(root, "set_materials_gpu"), uv, tri_material, materials, textures);
+}
+
+void set_materials_gpu(gi::MultiGpu& replicas, const std::vector<jql::Vec2>& uv, const std::vector<std::uint32_t>& tri_material,
+                       const std::vector<GpuMaterial>& materials, const std::vector<GpuTexture>& textures)
+{
+        set_materials_native(vrt_mgpu_set_materials, replicas.native(), uv, tri_material, materials, textures);
 }
 
 // ---- predicates ----------------------------------------------------------------------------

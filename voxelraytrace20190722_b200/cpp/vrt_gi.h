@@ -110,6 +110,23 @@ void cone_trace_init_filter(VoxelOctree* root);
 Vec3 cone_trace(const VoxelOctree& root, const ISect& isect, float min_voxel_size);
 void cone_trace_batch(const VoxelOctree& root, const std::vector<ISect>& isects, float min_voxel_size,
                       std::vector<Vec3>* out);
+
+// Replicas of a built octree on several devices (vrt_mgpu_*; a device may be listed more than once), for main.cc's
+// GI statements on N GPUs: light_map_gpu / cone_trace_init_filter / render_gi_gpu below take one in place of the
+// root.  The replicas hold the geometry only; the light pass runs on each of them.  Owns the vrt_mgpu*.
+class MultiGpu {
+public:
+        MultiGpu(const VoxelOctree* root, const std::vector<int>& devices);
+        ~MultiGpu();
+        MultiGpu(const MultiGpu&) = delete;
+        MultiGpu& operator=(const MultiGpu&) = delete;
+        vrt_mgpu* native() const { return m_; }
+        int num_devices() const { return vrt_mgpu_num_devices(m_); }
+
+private:
+        vrt_mgpu* m_ = nullptr;
+};
+void cone_trace_init_filter(MultiGpu& replicas);
 }  // namespace gi
 
 class Film {  // camera.h:24-39 -- storage is y*nx+x (the reference's y*ny+x is only right for nx==ny)
@@ -156,6 +173,11 @@ void render_gpu(Film* film, Camera& cam, gi::VoxelOctree* root, int spp, const j
 void light_map_gpu(const Film& sfilm, Camera& scam, gi::VoxelOctree* root, int spp, const jql::Vec3& kd);
 // Replacement of the final render_mt loop of main.cc:117-123 (trace() per sample, film += c / spp).
 void render_gi_gpu(Film* film, Camera& cam, gi::VoxelOctree* root, int spp, const jql::Vec3& kd, float res);
+// The same two statements on the replicas of a gi::MultiGpu: the light map is splatted on every replica, and the
+// film's 8-row bands are dealt round-robin to the devices, each copying its bands straight into film->data().
+// Both return when the work is done; the film equals the single-device one bytewise.
+void light_map_gpu(const Film& sfilm, Camera& scam, gi::MultiGpu& replicas, int spp, const jql::Vec3& kd);
+void render_gi_gpu(Film* film, Camera& cam, gi::MultiGpu& replicas, int spp, const jql::Vec3& kd, float res);
 
 // Materials for the GI passes (the half of gi::Triangle the geometry mirror leaves out: t_[3] and
 // tinyobj::material_t::diffuse / diffuse_texname, voxel_octree.h:110-111).  uv holds three texture
@@ -170,6 +192,9 @@ struct GpuTexture {
         const std::uint8_t* data;
 };
 void set_materials_gpu(gi::VoxelOctree* root, const std::vector<jql::Vec2>& uv, const std::vector<std::uint32_t>& tri_material,
+                       const std::vector<GpuMaterial>& materials, const std::vector<GpuTexture>& textures);
+// the same materials on every replica
+void set_materials_gpu(gi::MultiGpu& replicas, const std::vector<jql::Vec2>& uv, const std::vector<std::uint32_t>& tri_material,
                        const std::vector<GpuMaterial>& materials, const std::vector<GpuTexture>& textures);
 
 // tribox2.h:15 and raytri.h:5-7 -- same signatures, evaluated on the GPU.

@@ -579,7 +579,8 @@ void vrt_tree_free(vrt_tree* t)
         t->hull_buf.release();
         t->tri64_buf.release();
         t->gi_recs.release();
-        t->gi_steps.release();
+        t->gi_steps[0].release();
+        t->gi_steps[1].release();
         t->tabrel_buf.release();
         for (auto& rs : t->tabrel_slot)
                 if (rs.ev) {
@@ -600,6 +601,8 @@ void vrt_tree_free(vrt_tree* t)
                 if (t->film_copied[i])
                         cudaEventDestroy(t->film_copied[i]);
         }
+        if (t->gi_written)
+                cudaEventDestroy(t->gi_written);
         for (unsigned l = 0; l <= VRT_MAX_DEPTH; ++l) {
                 t->level_morton[l].release();
                 t->level_first[l].release();
@@ -1155,6 +1158,7 @@ static int async_pipeline_prepare(vrt_tree* t)
                         VRT_CUDA(cudaEventCreateWithFlags(&t->film_ready[i], cudaEventDisableTiming));
                         VRT_CUDA(cudaEventCreateWithFlags(&t->film_copied[i], cudaEventDisableTiming));
                 }
+                VRT_CUDA(cudaEventCreateWithFlags(&t->gi_written, cudaEventDisableTiming));
         }
         if (t->n_async_frames == 0)  // the alternate stream starts behind everything enqueued so far
                 VRT_CUDA(cudaStreamSynchronize(t->stream));
@@ -1162,6 +1166,26 @@ static int async_pipeline_prepare(vrt_tree* t)
 }
 // kernel stream of async frame k: even frames on the handle's stream, odd frames on the alternate one
 static cudaStream_t async_kernel_stream(const vrt_tree* t) { return (t->n_async_frames & 1) ? t->alt_stream : t->stream; }
+
+// The writers of the state a GI frame reads (vrt_gi_init, vrt_gi_splat_camera, vrt_gi_filter, vrt_set_materials) work
+// on `stream`, while the odd frames of a pipelined sequence run on `alt_stream`.  Between the two calls of this pair
+// the writer is ordered after every frame enqueued so far (the even ones are on `stream` already, the last odd one
+// recorded film_ready[1]), and every later frame is ordered after the writer (the even ones by stream order, the odd
+// ones by the wait of alt_stream).  The frame path itself gains nothing: consecutive frames still overlap.
+static int gi_writer_begin(vrt_tree* t)
+{
+        if (t->n_async_frames >= 2)  // an odd frame of the current sequence exists
+                VRT_CUDA(cudaStreamWaitEvent(t->stream, t->film_ready[1], 0));
+        return VRT_OK;
+}
+static int gi_writer_end(vrt_tree* t, int rc)
+{
+        if (t->alt_stream) {  // (no pipelined frame yet: the first one synchronises with `stream` anyway)
+                VRT_CUDA(cudaEventRecord(t->gi_written, t->stream));
+                VRT_CUDA(cudaStreamWaitEvent(t->alt_stream, t->gi_written, 0));
+        }
+        return rc;
+}
 
 // Pipelined frame loop: the kernel of frame k+1 runs while frame k's film crosses PCIe.
 int vrt_render_camera_async(const vrt_tree* tc, const vrt_camera* cam, const vrt_shade* sh, int x0, int y0, int x1,
@@ -1302,9 +1326,11 @@ int vrt_render_bands_dev(const vrt_tree* t, const vrt_camera* cam, const vrt_sha
 // band buffers and copied by one strided DMA (cudaMemcpy2DAsync: one row per band) straight to
 // their final rows of the full host frame, which every rank of the node maps (shared + pinned),
 // so the N ranks use their N PCIe links in parallel and the copy of frame k overlaps the kernel
-// of frame k+1 -- the N-GPU counterpart of vrt_render_camera_async.
-int vrt_render_bands_async(const vrt_tree* tc, const vrt_camera* cam, const vrt_shade* sh, const vrt_bands* b,
-                           float* film_rgb_full)
+// of frame k+1 -- the N-GPU counterpart of vrt_render_camera_async.  mode OUT_FILM: the harness
+// film (sh); OUT_GI_FILM: the cone-traced GI film (gi->kd, gi->res; the step table is filled on
+// the frame's kernel stream).
+static int bands_async_common(const vrt_tree* tc, const vrt_camera* cam, const vrt_shade* sh, const GiArgs* gi,
+                              const vrt_bands* b, float* film_rgb_full, OutMode mode)
 {
         int rc = check_tree(tc);
         if (rc)
@@ -1317,8 +1343,12 @@ int vrt_render_bands_async(const vrt_tree* tc, const vrt_camera* cam, const vrt_
                 return rows;
         if (rows == 0)
                 return VRT_OK;
-        if (!film_rgb_full || !sh) {
+        if (!film_rgb_full || (mode == OUT_FILM ? !sh : !gi)) {
                 set_error("null out/shade pointer");
+                return VRT_ERR_ARG;
+        }
+        if (mode == OUT_GI_FILM && !tc->dev.gi) {
+                set_error("vrt_gi_init has not been called on this tree");
                 return VRT_ERR_ARG;
         }
         vrt_tree* t = const_cast<vrt_tree*>(tc);
@@ -1338,8 +1368,14 @@ int vrt_render_bands_async(const vrt_tree* tc, const vrt_camera* cam, const vrt_
                 VRT_CUDA(cudaStreamWaitEvent(ks, t->film_copied[k], 0));
         const int y0 = b->band_first * b->band_h;
         t->launch_stream = ks;
-        rc = launch_trace_camera(t, cam, sh, 0, y0, cam->nx, y0 + rows, t->film_dev[k].p, OUT_FILM, b->band_h,
-                                 b->band_stride * b->band_h);
+        GiArgs ga{};
+        if (mode == OUT_GI_FILM) {
+                ga = *gi;
+                rc = gi_step_table(t, ga.res, &ga.steps);
+        }
+        if (!rc)
+                rc = launch_trace_camera(t, cam, sh, 0, y0, cam->nx, y0 + rows, t->film_dev[k].p, mode, b->band_h,
+                                         b->band_stride * b->band_h, nullptr, 0, mode == OUT_GI_FILM ? &ga : nullptr);
         t->launch_stream = nullptr;
         if (rc)
                 return rc;
@@ -1365,6 +1401,24 @@ int vrt_render_bands_async(const vrt_tree* tc, const vrt_camera* cam, const vrt_
         VRT_CUDA(cudaEventRecord(t->film_copied[k], t->copy_stream));
         t->n_async_frames++;
         return VRT_OK;
+}
+
+int vrt_render_bands_async(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, const vrt_bands* b,
+                           float* film_rgb_full)
+{
+        return bands_async_common(t, cam, sh, nullptr, b, film_rgb_full, OUT_FILM);
+}
+
+// The cone-traced GI film (vrt_gi_render_camera) through the same banded, pipelined path.
+int vrt_gi_render_bands_async(const vrt_tree* t, const vrt_camera* cam, const float kd[3], float res,
+                              const vrt_bands* b, float* film_rgb_full)
+{
+        if (!kd) {
+                set_error("null argument");
+                return VRT_ERR_ARG;
+        }
+        const GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
+        return bands_async_common(t, cam, nullptr, &ga, b, film_rgb_full, OUT_GI_FILM);
 }
 
 // ---- single-process multi-GPU render (SURVEY.md 8e; replaces render_mt camera.h:41-68 over N devices) -------
@@ -1480,7 +1534,11 @@ int vrt_mgpu_create(const vrt_tree* tree, int num_devices, const int* devices, v
 
 int vrt_mgpu_num_devices(const vrt_mgpu* m) { return m ? (int)m->trees.size() : 0; }
 
-int vrt_mgpu_render_async(vrt_mgpu* m, const vrt_camera* cam, const vrt_shade* sh, float* film_rgb_full)
+// f(i, replica i) for every replica with its device current, up to the first failure; the caller's device is restored
+extern "C++" {
+namespace {
+template <class F>
+int mgpu_each(vrt_mgpu* m, F&& f)
 {
         if (!m || m->trees.empty()) {
                 set_error("null multi-GPU handle");
@@ -1489,18 +1547,33 @@ int vrt_mgpu_render_async(vrt_mgpu* m, const vrt_camera* cam, const vrt_shade* s
         int cur = 0;
         VRT_CUDA(cudaGetDevice(&cur));
         int rc = VRT_OK;
-        const int n = (int)m->trees.size();
-        for (int i = 0; i < n && !rc; ++i) {
+        for (int i = 0; i < (int)m->trees.size() && !rc; ++i) {
                 rc = set_device_checked(m->devices[i]);
-                if (rc)
-                        break;
-                const vrt_bands b = { m->band_h, i, n };
-                if (cam && (long)i * m->band_h >= cam->ny)
-                        continue;  // more devices than bands
-                rc = vrt_render_bands_async(m->trees[i], cam, sh, &b, film_rgb_full);
+                if (!rc)
+                        rc = f(i, m->trees[i]);
         }
         cudaSetDevice(cur);
         return rc;
+}
+}  // namespace
+}  // extern "C++"
+
+// one frame: the 8-row bands dealt round-robin, each replica through its bands_async_common pipeline
+static int mgpu_bands_async(vrt_mgpu* m, const vrt_camera* cam, const vrt_shade* sh, const GiArgs* gi,
+                            float* film_rgb_full, OutMode mode)
+{
+        const int n = m ? (int)m->trees.size() : 0;
+        return mgpu_each(m, [&](int i, vrt_tree* t) {
+                if (cam && (long)i * m->band_h >= cam->ny)
+                        return (int)VRT_OK;  // more devices than bands
+                const vrt_bands b = { m->band_h, i, n };
+                return bands_async_common(t, cam, sh, gi, &b, film_rgb_full, mode);
+        });
+}
+
+int vrt_mgpu_render_async(vrt_mgpu* m, const vrt_camera* cam, const vrt_shade* sh, float* film_rgb_full)
+{
+        return mgpu_bands_async(m, cam, sh, nullptr, film_rgb_full, OUT_FILM);
 }
 
 int vrt_mgpu_sync(vrt_mgpu* m)
@@ -1530,6 +1603,65 @@ int vrt_mgpu_render(vrt_mgpu* m, const vrt_camera* cam, const vrt_shade* sh, flo
         return rc ? rc : rs;
 }
 
+// ---- GI film on the replicas.  vrt_mgpu_create copies the geometry blob only; materials and the per-node GI state
+// are set per replica.  The light pass runs on every replica (the splat accumulates in the sequential loop order, so
+// every replica holds the same bits) -- concurrently, since none of the passes waits on the host.
+int vrt_mgpu_set_materials(vrt_mgpu* m, const float* tri_uv, const uint32_t* tri_mtl, uint32_t num_mtl,
+                           const float* kd, const int32_t* mtl_tex, uint32_t num_tex, const vrt_texture* tex)
+{
+        return mgpu_each(m, [&](int, vrt_tree* t) {
+                return vrt_set_materials(t, tri_uv, tri_mtl, num_mtl, kd, mtl_tex, num_tex, tex);
+        });
+}
+
+int vrt_mgpu_gi_init(vrt_mgpu* m)
+{
+        return mgpu_each(m, [](int, vrt_tree* t) { return vrt_gi_init(t); });
+}
+
+int vrt_mgpu_gi_splat_camera(vrt_mgpu* m, const vrt_camera* light_cam, const float kd[3])
+{
+        return mgpu_each(m, [&](int, vrt_tree* t) { return vrt_gi_splat_camera(t, light_cam, kd); });
+}
+
+int vrt_mgpu_gi_filter(vrt_mgpu* m)
+{
+        return mgpu_each(m, [](int, vrt_tree* t) { return vrt_gi_filter(t); });
+}
+
+int vrt_mgpu_gi_render_async(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_rgb_full)
+{
+        if (!kd) {
+                set_error("null argument");
+                return VRT_ERR_ARG;
+        }
+        const GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
+        return mgpu_bands_async(m, cam, nullptr, &ga, film_rgb_full, OUT_GI_FILM);
+}
+
+int vrt_mgpu_gi_render(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_rgb_full)
+{
+        int rc = vrt_mgpu_gi_render_async(m, cam, kd, res, film_rgb_full);
+        const int rs = vrt_mgpu_sync(m);
+        return rc ? rc : rs;
+}
+
+double vrt_mgpu_mean_kernel_ms(vrt_mgpu* m, int index, int last_n)
+{
+        if (!m || index < 0 || index >= (int)m->trees.size())
+                return 0;
+        double ms = 0;
+        int cur = 0;
+        if (cudaGetDevice(&cur) != cudaSuccess) {
+                cudaGetLastError();
+                return 0;
+        }
+        if (!set_device_checked(m->devices[index]))
+                ms = vrt_mean_kernel_ms(m->trees[index], last_n);
+        cudaSetDevice(cur);
+        return ms;
+}
+
 int vrt_trace_bands16_dev(const vrt_tree* t, const vrt_camera* cam, const vrt_bands* b, vrt_hit16* d_out)
 {
         return bands_common(t, cam, nullptr, b, d_out, OUT_HIT16);
@@ -1555,7 +1687,9 @@ double vrt_mean_kernel_ms(const vrt_tree* t, int last_n)
 int vrt_gi_init(vrt_tree* t)
 {
         int rc = check_tree(t);
-        return rc ? rc : gi_init(t);
+        if (rc || (rc = gi_writer_begin(t)))
+                return rc;
+        return gi_writer_end(t, gi_init(t));
 }
 
 int vrt_gi_splat_camera(vrt_tree* t, const vrt_camera* light_cam, const float kd[3])
@@ -1568,13 +1702,17 @@ int vrt_gi_splat_camera(vrt_tree* t, const vrt_camera* light_cam, const float kd
                 return VRT_ERR_ARG;
         }
         rc = check_camera(light_cam, 0, 0, light_cam->nx, light_cam->ny);
-        return rc ? rc : gi_splat_camera(t, light_cam, kd);
+        if (rc || (rc = gi_writer_begin(t)))
+                return rc;
+        return gi_writer_end(t, gi_splat_camera(t, light_cam, kd));
 }
 
 int vrt_gi_filter(vrt_tree* t)
 {
         int rc = check_tree(t);
-        return rc ? rc : gi_filter(t);
+        if (rc || (rc = gi_writer_begin(t)))
+                return rc;
+        return gi_writer_end(t, gi_filter(t));
 }
 
 int vrt_gi_get_level(const vrt_tree* t, int level, float* coverage, float* illum18)
@@ -1679,19 +1817,28 @@ int vrt_set_materials(vrt_tree* t, const float* tri_uv, const uint32_t* tri_mtl,
         const uint64_t o_uv = 0, o_tri = align256(o_uv + std::max<uint64_t>(T, 1) * 24);
         const uint64_t o_kd = align256(o_tri + std::max<uint64_t>(T, 1) * 4), o_tex = align256(o_kd + (uint64_t)num_mtl * 16);
         const uint64_t o_px = align256(o_tex + (uint64_t)std::max<uint32_t>(num_tex, 1) * 16);
+        rc = gi_writer_begin(t);
+        if (rc)
+                return rc;
         if (t->mat_buf.reserve(o_px + std::max<uint64_t>(texel_bytes, 256)))
-                return VRT_ERR_NOMEM;
+                return gi_writer_end(t, VRT_ERR_NOMEM);
         char* base = static_cast<char*>(t->mat_buf.p);
-        VRT_CUDA(cudaStreamSynchronize(t->stream));
+        // the copies are ordered on the handle's stream (behind every frame that may still read the old materials,
+        // gi_writer_begin) and complete before the call returns: the host arrays are borrowed for the call only
         if (T) {
-                VRT_CUDA(cudaMemcpy(base + o_uv, tri_uv, T * 24, cudaMemcpyHostToDevice));
-                VRT_CUDA(cudaMemcpy(base + o_tri, tri_mtl, T * 4, cudaMemcpyHostToDevice));
+                VRT_CUDA(cudaMemcpyAsync(base + o_uv, tri_uv, T * 24, cudaMemcpyHostToDevice, t->stream));
+                VRT_CUDA(cudaMemcpyAsync(base + o_tri, tri_mtl, T * 4, cudaMemcpyHostToDevice, t->stream));
         }
-        VRT_CUDA(cudaMemcpy(base + o_kd, hkd.data(), (size_t)num_mtl * 16, cudaMemcpyHostToDevice));
-        VRT_CUDA(cudaMemcpy(base + o_tex, htex.data(), htex.size() * 4, cudaMemcpyHostToDevice));
+        VRT_CUDA(cudaMemcpyAsync(base + o_kd, hkd.data(), (size_t)num_mtl * 16, cudaMemcpyHostToDevice, t->stream));
+        VRT_CUDA(cudaMemcpyAsync(base + o_tex, htex.data(), htex.size() * 4, cudaMemcpyHostToDevice, t->stream));
         for (uint32_t i = 0; i < num_tex; ++i)
-                VRT_CUDA(cudaMemcpy(base + o_px + (uint32_t)htex[4 * i], tex[i].data,
-                                    (size_t)tex[i].width * tex[i].height * tex[i].channels, cudaMemcpyHostToDevice));
+                VRT_CUDA(cudaMemcpyAsync(base + o_px + (uint32_t)htex[4 * i], tex[i].data,
+                                         (size_t)tex[i].width * tex[i].height * tex[i].channels, cudaMemcpyHostToDevice,
+                                         t->stream));
+        VRT_CUDA(cudaStreamSynchronize(t->stream));
+        rc = gi_writer_end(t, VRT_OK);
+        if (rc)
+                return rc;
         t->dev.mat_uv = reinterpret_cast<const float2*>(base + o_uv);
         t->dev.mat_tri = reinterpret_cast<const uint32_t*>(base + o_tri);
         t->dev.mat_kd = reinterpret_cast<const float4*>(base + o_kd);

@@ -208,16 +208,17 @@ int gi_step_table(const vrt_tree* t, float res, const float4** d_steps)
         }
         if (!on)
                 return VRT_OK;
-        if (t->gi_steps.reserve((size_t)(kGiMaxSteps + 2) * sizeof(float4)))  // (+1: the cone loop reads one entry ahead)
+        cudaStream_t s = t->launch_stream ? t->launch_stream : t->stream;
+        Scratch& tab = t->gi_steps[(t->alt_stream && s == t->alt_stream) ? 1 : 0];
+        if (tab.reserve((size_t)(kGiMaxSteps + 2) * sizeof(float4)))  // (+1: the cone loop reads one entry ahead)
                 return VRT_ERR_NOMEM;
         GiRoot6 r;
         for (int k = 0; k < 6; ++k)
                 r.v[k] = t->hdr.root_aabb[k];
-        cudaStream_t s = t->launch_stream ? t->launch_stream : t->stream;
-        k_gi_step_table<<<1, 1, 0, s>>>(r, res, t->gi_steps.as<float4>());
+        k_gi_step_table<<<1, 1, 0, s>>>(r, res, tab.as<float4>());
         count_launch();
         VRT_CUDA(cudaGetLastError());
-        *d_steps = t->gi_steps.as<float4>();
+        *d_steps = tab.as<float4>();
         return VRT_OK;
 }
 

@@ -156,7 +156,9 @@ struct vrt_tree {
         vrt::Scratch io_in, io_out;
         // GI rows (SURVEY.md 8f): per-node coverage + illum[6], see vrt_gi.cuh
         vrt::Scratch gi_buf, gi_recs, mat_buf;
-        mutable vrt::Scratch gi_steps;  // step table of the last cone trace launch
+        // step table of the last cone trace launch, one per kernel stream ([0] `stream`, [1] `alt_stream`): a GI frame
+        // on one stream never overwrites the table a frame on the other stream may still read
+        mutable vrt::Scratch gi_steps[2];
         vrt::Scratch hull_buf;  // TreeDev::hull
         vrt::Scratch tri64_buf;  // TreeDev::tri64
         // pipelined host-film path (vrt_render_camera_async): two device films, a copy stream
@@ -168,6 +170,8 @@ struct vrt_tree {
         cudaStream_t alt_stream = nullptr;
         mutable cudaStream_t launch_stream = nullptr;
         cudaEvent_t film_ready[2] = {}, film_copied[2] = {};
+        // recorded on `stream` when a GI / material writer returns; alt_stream waits on it (vrt_api.cu gi_writer_end)
+        cudaEvent_t gi_written = nullptr;
         mutable uint64_t n_async_frames = 0;
         cudaEvent_t ev0 = nullptr, ev1 = nullptr;  // build timing
         // trace launches are asynchronous: each one records a (start, stop) pair in this ring
@@ -235,7 +239,8 @@ int hull_stats(unsigned long long* out80);
 int gi_init(vrt_tree* t);
 int gi_splat_camera(vrt_tree* t, const vrt_camera* cam, const float kd[3]);
 int gi_filter(vrt_tree* t);
-// fills the tree's step table for `res` on its stream (vrt_gi.cuh) and returns the device pointer
+// fills the tree's step table for `res` on its launch stream (vrt_gi.cuh) -- the table of that kernel stream --
+// and returns the device pointer
 int gi_step_table(const vrt_tree* t, float res, const float4** d_steps);
 int gi_cone_points(const vrt_tree* t, const float* d_pos, const float* d_nrm, uint64_t n, float res, float* d_out);
 int gi_albedo_points(const vrt_tree* t, const uint32_t* d_tri, const float* d_pos, uint64_t n, const float kd[3], float* d_out);
