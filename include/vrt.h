@@ -370,6 +370,35 @@ int vrt_gi_render_camera_dev(const vrt_tree* tree, const vrt_camera* cam, const 
  * without a vrt_tree_sync: they run after every frame enqueued before them and before every frame after. */
 int vrt_gi_render_bands_async(const vrt_tree* tree, const vrt_camera* cam, const float kd[3], float res,
                               const vrt_bands* bands, float* film_rgb_full);
+/* What the GI film is made of: the per-pixel planes of one vrt_gi_render_camera launch (for a denoiser's albedo and
+ * normal guides, a compositor, or tuning octree depth, light-film resolution and textures).  For a sample that hits,
+ * with d the ray direction, the library computes exactly the terms the film is built from:
+ *   A  albedo    Triangle::get_albedo at the hit, kd the untextured colour (what vrt_albedo returns);
+ *   I  indirect  gi::cone_trace(root, isect, res), six cones (what vrt_gi_cone_trace returns);
+ *   D  direct    the hit leaf's VoxelOctree::compute_illum(-d) (voxel_octree.h:71-81);
+ *   N  normal    the ISect normal the cone basis is built from;
+ * and the film sample is A * (I + D).  A miss adds +0 to every plane; the sky goes into the film only.
+ * Every float plane is [(y1-y0)][(x1-x0)][3] float32 whatever the film format, accumulated like the film
+ * (main.cc:119-122): acc = +0, then acc += v_s * (1/spp) in sample order, so the normal plane is the sample mean and
+ * is not renormalised.  hits is [(y1-y0)][(x1-x0)][spp] vrt_hit16, bytewise the records of the 16-byte camera
+ * trace for the same camera and rectangle.  Every member is optional (NULL: not written). */
+typedef struct vrt_gi_aov {
+        float* albedo;    /* [rows][cols][3] */
+        float* direct;    /* [rows][cols][3] */
+        float* indirect;  /* [rows][cols][3] */
+        float* normal;    /* [rows][cols][3] */
+        vrt_hit16* hits;  /* [rows][cols][spp] */
+} vrt_gi_aov;
+/* The GI film of the camera-film GI call plus any of the planes above, in one launch.  The film (in the handle's
+ * film format, bytewise that call's film) may be NULL; a request with every plane NULL is VRT_ERR_ARG (the film
+ * alone is that call).  Otherwise requirements and errors are those of the camera-film GI call: vrt_gi_init first,
+ * and a rectangle outside the film is VRT_ERR_ARG.  The first form takes host pointers and returns when they are
+ * filled; the _dev form takes device pointers and is enqueued on the handle's stream (with that stream's cone-trace
+ * step table, like the _dev camera-film GI call). */
+int vrt_gi_render_aov(const vrt_tree* tree, const vrt_camera* cam, const float kd[3], float res, int x0, int y0,
+                      int x1, int y1, float* film_or_null, const vrt_gi_aov* aov);
+int vrt_gi_render_aov_dev(const vrt_tree* tree, const vrt_camera* cam, const float kd[3], float res, int x0, int y0,
+                          int x1, int y1, float* d_film_or_null, const vrt_gi_aov* d_aov);
 /* The GI rows on the replicas of a vrt_mgpu (main.cc:75-126 over N devices).  vrt_mgpu_create copies the
  * geometry only: materials and the GI state are set through these calls, each of which runs the single-device
  * call on every replica (host pointers, like the single-device calls).  The light pass runs on every replica --

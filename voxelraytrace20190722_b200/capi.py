@@ -39,6 +39,15 @@ class vrt_texture(C.Structure):
     _fields_ = [("width", C.c_int32), ("height", C.c_int32), ("channels", C.c_int32), ("data", C.c_void_p)]
 
 
+class vrt_gi_aov(C.Structure):
+    """The per-pixel planes of vrt_gi_render_aov(_dev); a null member is not written."""
+    _fields_ = [("albedo", C.c_void_p), ("direct", C.c_void_p), ("indirect", C.c_void_p), ("normal", C.c_void_p),
+                ("hits", C.c_void_p)]
+
+
+GI_AOV_PLANES = ("albedo", "direct", "indirect", "normal", "hits")
+
+
 class vrt_tree_info(C.Structure):
     _fields_ = [("num_tris", C.c_uint32), ("max_depth", C.c_int32), ("root_aabb", C.c_float * 6),
                 ("num_nodes", C.c_uint64), ("num_leaves", C.c_uint64), ("num_refs", C.c_uint64),
@@ -74,6 +83,7 @@ SYMBOLS = [
     "vrt_tri_overlap_aabb_batch", "vrt_raytri_batch", "vrt_aabb_isect_batch",
     "vrt_gi_render_bands_async", "vrt_mgpu_set_materials", "vrt_mgpu_gi_init", "vrt_mgpu_gi_splat_camera",
     "vrt_mgpu_gi_filter", "vrt_mgpu_gi_render_async", "vrt_mgpu_gi_render", "vrt_mgpu_mean_kernel_ms",
+    "vrt_gi_render_aov", "vrt_gi_render_aov_dev",
 ]
 
 _lib = None
@@ -167,6 +177,8 @@ def load(build_if_missing: bool = True):
     L.vrt_gi_render_camera.argtypes = [vp, C.POINTER(vrt_camera), vp, f32, i32, i32, i32, i32, vp]
     L.vrt_gi_render_camera_dev.argtypes = L.vrt_gi_render_camera.argtypes
     L.vrt_gi_render_bands_async.argtypes = [vp, C.POINTER(vrt_camera), vp, f32, C.POINTER(vrt_bands), vp]
+    L.vrt_gi_render_aov.argtypes = [vp, C.POINTER(vrt_camera), vp, f32, i32, i32, i32, i32, vp, C.POINTER(vrt_gi_aov)]
+    L.vrt_gi_render_aov_dev.argtypes = L.vrt_gi_render_aov.argtypes
     L.vrt_mgpu_set_materials.argtypes = [vp, vp, vp, C.c_uint32, vp, vp, C.c_uint32, vp]
     L.vrt_mgpu_gi_init.argtypes = [vp]
     L.vrt_mgpu_gi_splat_camera.argtypes = [vp, C.POINTER(vrt_camera), vp]
@@ -529,6 +541,36 @@ class Octree:
         kd = np.ascontiguousarray(kd, np.float32)
         _check(load().vrt_gi_render_camera_dev(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)), x0, y0, x1,
                                                y1, C.c_void_p(d_film_ptr)))
+
+    def gi_render_aov(self, cam: Camera, kd, res, rect=None, planes=GI_AOV_PLANES, film=True):
+        """The GI film (gi_render's, in the handle's film format; None with film=False) and what it is made of, from
+        one launch: {name: array} for the requested planes -- 'albedo', 'direct', 'indirect', 'normal' as float32
+        [h, w, 3] sample means, 'hits' as HIT16_DTYPE [h, w, spp] (include/vrt.h vrt_gi_aov)."""
+        x0, y0, x1, y1 = rect if rect else (0, 0, cam.nx, cam.ny)
+        h, w = y1 - y0, x1 - x0
+        unknown = set(planes) - set(GI_AOV_PLANES)
+        if unknown:
+            raise ValueError(f"unknown GI planes {sorted(unknown)}")
+        out = {n: (np.zeros((h, w, cam.spp), HIT16_DTYPE) if n == "hits" else np.zeros((h, w, 3), np.float32))
+               for n in planes}
+        f = self._film_array(h, w) if film else None
+        aov = vrt_gi_aov(**{n: a.ctypes.data for n, a in out.items()})
+        kd = np.ascontiguousarray(kd, np.float32)
+        _check(load().vrt_gi_render_aov(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)), x0, y0, x1, y1,
+                                        _ptr(f), C.byref(aov)))
+        return f, out
+
+    def gi_render_aov_dev(self, cam: Camera, kd, res, d_film_or_0, d_planes: dict, rect=None):
+        """gi_render_aov into device memory, enqueued on the handle's stream: d_planes maps plane names to device
+        pointers (float32 [h, w, 3], hits vrt_hit16 [h, w, spp]); d_film_or_0 = 0 writes no film."""
+        x0, y0, x1, y1 = rect if rect else (0, 0, cam.nx, cam.ny)
+        unknown = set(d_planes) - set(GI_AOV_PLANES)
+        if unknown:
+            raise ValueError(f"unknown GI planes {sorted(unknown)}")
+        aov = vrt_gi_aov(**{n: int(p) for n, p in d_planes.items() if p})
+        kd = np.ascontiguousarray(kd, np.float32)
+        _check(load().vrt_gi_render_aov_dev(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)), x0, y0, x1,
+                                            y1, C.c_void_p(int(d_film_or_0) or None), C.byref(aov)))
 
     def render_async(self, cam: Camera, out, light=None, kd=0.8, rect=None, shadow_eps=None):
         """Pipelined frame loop: enqueue one frame whose film lands in the (pinned) host array

@@ -6,7 +6,8 @@
 //   demo_main [out.bmp] [max_depth] [nx] [ny] [scene.obj]
 // With --dump <file> it also writes (hit,tri,cell,pos,nrm) per ray for the parity test.
 // With --gi <file> it also writes main.cc's cone-traced GI film (float, plus <file>.hdr); with --gi-devices 0,0,...
-// as well, the same film rendered through gi::MultiGpu on those devices goes to <file>.mgpu.
+// as well, the same film rendered through gi::MultiGpu on those devices goes to <file>.mgpu; with --gi-aov <prefix> as
+// well, what that film is made of goes to <prefix>.{albedo,direct,indirect,normal}.hdr.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -124,11 +125,13 @@ int main(int argc, char** argv)
         const char* dump = nullptr;
         const char* gi_dump = nullptr;  // --gi <file>: also run main.cc's light map + filter + cone-traced film
         std::vector<int> gi_devices;    // --gi-devices 0,0,...: the GI film again on these replicas -> <file>.mgpu
+        const char* gi_aov = nullptr;   // --gi-aov <prefix>: the GI film's planes -> <prefix>.<plane>.hdr
         const char* obj = nullptr;
         int depth = 6, nx = 1024, ny = 1024, pos = 0;  // main.cc:34-35,67
         for (int i = 1; i < argc; ++i) {
                 if (!std::strcmp(argv[i], "--dump") && i + 1 < argc) { dump = argv[++i]; continue; }
                 if (!std::strcmp(argv[i], "--gi") && i + 1 < argc) { gi_dump = argv[++i]; continue; }
+                if (!std::strcmp(argv[i], "--gi-aov") && i + 1 < argc) { gi_aov = argv[++i]; continue; }
                 if (!std::strcmp(argv[i], "--gi-devices") && i + 1 < argc) {
                         for (const char* p = argv[++i]; *p;) {
                                 char* end = nullptr;
@@ -201,6 +204,23 @@ int main(int argc, char** argv)
                         FILE* f = std::fopen(gi_dump, "wb");
                         std::fwrite(d.data(), sizeof(float), d.size(), f);
                         std::fclose(f);
+                        if (gi_aov) {
+                                // the film's factors (a denoiser's albedo and normal guides, the light terms)
+                                Film albedo(1.f, 1.f, nx, ny), direct(1.f, 1.f, nx, ny), indirect(1.f, 1.f, nx, ny),
+                                        normal(1.f, 1.f, nx, ny);
+                                gi::GiAov aov;
+                                aov.albedo = &albedo;
+                                aov.direct = &direct;
+                                aov.indirect = &indirect;
+                                aov.normal = &normal;
+                                render_gi_aov_gpu(nullptr, cam, &root, 4, kd, res, aov);
+                                const std::pair<const char*, const Film*> planes[4] = {
+                                        { "albedo", &albedo }, { "direct", &direct }, { "indirect", &indirect }, { "normal", &normal }
+                                };
+                                for (const auto& pl : planes)
+                                        write_hdr((std::string(gi_aov) + "." + pl.first + ".hdr").c_str(), *pl.second);
+                                std::printf("GI planes written\n");
+                        }
                         if (!gi_devices.empty()) {
                                 // the same three GI statements on the replicas of gi::MultiGpu
                                 std::printf("GI film on %zu replicas...\n", gi_devices.size());

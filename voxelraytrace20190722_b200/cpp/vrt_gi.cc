@@ -364,6 +364,33 @@ void render_gi_gpu(Film* film, Camera& cam, gi::VoxelOctree* root, int spp, cons
         check(vrt_gi_render_camera(t, &c, k, res, 0, 0, film->nx, film->ny, &film->data()->x), "render_gi_gpu");
 }
 
+void render_gi_aov_gpu(Film* film_or_null, Camera& cam, gi::VoxelOctree* root, int spp, const jql::Vec3& kd, float res,
+                       gi::GiAov& aov)
+{
+        vrt_tree* t = gi::gi_tree(root, "render_gi_aov_gpu");
+        Film* const planes[4] = { aov.albedo, aov.direct, aov.indirect, aov.normal };
+        const Film* geo = film_or_null;
+        for (Film* p : planes)
+                if (!geo)
+                        geo = p;
+        if (!geo)
+                throw std::runtime_error("render_gi_aov_gpu: neither a film nor a float plane gives the film size");
+        for (Film* p : planes)
+                if (p && (p->nx != geo->nx || p->ny != geo->ny))
+                        throw std::runtime_error("render_gi_aov_gpu: the planes and the film differ in size");
+        const vrt_camera c = cam.native(*geo, spp);
+        const float k[3] = { kd.x, kd.y, kd.z };
+        if (aov.hits)
+                aov.hits->resize((size_t)geo->nx * geo->ny * spp);
+        float* dst[4];
+        for (int i = 0; i < 4; ++i)
+                dst[i] = planes[i] ? &planes[i]->data()->x : nullptr;
+        const vrt_gi_aov a = { dst[0], dst[1], dst[2], dst[3], aov.hits ? aov.hits->data() : nullptr };
+        check(vrt_gi_render_aov(t, &c, k, res, 0, 0, geo->nx, geo->ny, film_or_null ? &film_or_null->data()->x : nullptr,
+                                &a),
+              "render_gi_aov_gpu");
+}
+
 void light_map_gpu(const Film& sfilm, Camera& scam, gi::MultiGpu& replicas, int spp, const jql::Vec3& kd)
 {
         const vrt_camera c = scam.native(sfilm, spp);

@@ -179,6 +179,24 @@ void render_gi_gpu(Film* film, Camera& cam, gi::VoxelOctree* root, int spp, cons
 void light_map_gpu(const Film& sfilm, Camera& scam, gi::MultiGpu& replicas, int spp, const jql::Vec3& kd);
 void render_gi_gpu(Film* film, Camera& cam, gi::MultiGpu& replicas, int spp, const jql::Vec3& kd, float res);
 
+namespace gi {
+// What main.cc's GI film is made of, per pixel (vrt_gi_aov in include/vrt.h): the sample means of the albedo, the
+// leaf's direct light, the cone-traced indirect light and the ISect normal (a miss adds 0), and the 16-byte hit
+// record of every sample.  Every member is optional (nullptr: not written).
+struct GiAov {
+        Film* albedo = nullptr;
+        Film* direct = nullptr;
+        Film* indirect = nullptr;
+        Film* normal = nullptr;
+        std::vector<vrt_hit16>* hits = nullptr;  // resized to nx * ny * spp (pixel row-major, then sample)
+};
+}  // namespace gi
+// render_gi_gpu plus the planes of `aov`, from one launch.  film_or_null (when given) receives the same film as
+// render_gi_gpu; the film and the float planes must have one size, and at least one of them gives the camera's film
+// geometry.
+void render_gi_aov_gpu(Film* film_or_null, Camera& cam, gi::VoxelOctree* root, int spp, const jql::Vec3& kd, float res,
+                       gi::GiAov& aov);
+
 // Materials for the GI passes (the half of gi::Triangle the geometry mirror leaves out: t_[3] and
 // tinyobj::material_t::diffuse / diffuse_texname, voxel_octree.h:110-111).  uv holds three texture
 // coordinates per triangle in the order of the voxels given to ray_march_init; a material with

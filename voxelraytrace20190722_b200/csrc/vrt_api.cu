@@ -1914,6 +1914,86 @@ int vrt_gi_render_camera_dev(const vrt_tree* t, const vrt_camera* cam, const flo
         return gi_render_common(t, cam, kd, res, x0, y0, x1, y1, d_film_rgb, true);
 }
 
+// The GI film plus its planes (vrt_gi_aov) in one OUT_GI_AOV launch; host pointers go through one device buffer.
+static int gi_render_aov_common(const vrt_tree* tc, const vrt_camera* cam, const float kd[3], float res, int x0,
+                                int y0, int x1, int y1, float* film, const vrt_gi_aov* aov, bool dev)
+{
+        int rc = check_tree(tc);
+        if (rc)
+                return rc;
+        if (!cam || !kd || !aov) {
+                set_error("null argument");
+                return VRT_ERR_ARG;
+        }
+        float* const planes[4] = { aov->albedo, aov->direct, aov->indirect, aov->normal };
+        if (!planes[0] && !planes[1] && !planes[2] && !planes[3] && !aov->hits) {
+                set_error("vrt_gi_render_aov: every plane is NULL (the film alone is vrt_gi_render_camera)");
+                return VRT_ERR_ARG;
+        }
+        if (!tc->dev.gi) {
+                set_error("vrt_gi_init has not been called on this tree");
+                return VRT_ERR_ARG;
+        }
+        rc = check_camera(cam, x0, y0, x1, y1);
+        if (rc)
+                return rc;
+        const uint64_t npix = (uint64_t)(x1 - x0) * (y1 - y0);
+        if (!npix)
+                return VRT_OK;
+        GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
+        rc = gi_step_table(tc, res, &ga.steps);
+        if (rc)
+                return rc;
+        if (dev)
+                return launch_trace_camera(tc, cam, nullptr, x0, y0, x1, y1, film, OUT_GI_AOV, 0, 0, nullptr, 0, &ga, aov);
+        // one device buffer: film, the four float planes, the hit records (each part 256-byte aligned)
+        auto up = [](uint64_t b) { return (b + 255) & ~255ull; };
+        const uint64_t film_bytes = npix * (uint64_t)vrt_film_pixel_bytes(tc->film_fmt), plane_bytes = npix * 12,
+                       hit_bytes = npix * cam->spp * sizeof(vrt_hit16);
+        uint64_t off[6] = { 0 };
+        off[1] = off[0] + (film ? up(film_bytes) : 0);
+        for (int i = 0; i < 4; ++i)
+                off[i + 2] = off[i + 1] + (planes[i] ? up(plane_bytes) : 0);
+        const uint64_t total = off[5] + (aov->hits ? hit_bytes : 0);
+        vrt_tree* t = const_cast<vrt_tree*>(tc);
+        if (t->io_out.reserve(total))
+                return VRT_ERR_NOMEM;
+        char* const base = static_cast<char*>(t->io_out.p);
+        vrt_gi_aov d_aov = {};
+        float** const d_planes[4] = { &d_aov.albedo, &d_aov.direct, &d_aov.indirect, &d_aov.normal };
+        for (int i = 0; i < 4; ++i)
+                if (planes[i])
+                        *d_planes[i] = reinterpret_cast<float*>(base + off[i + 1]);
+        if (aov->hits)
+                d_aov.hits = reinterpret_cast<vrt_hit16*>(base + off[5]);
+        rc = launch_trace_camera(t, cam, nullptr, x0, y0, x1, y1, film ? base : nullptr, OUT_GI_AOV, 0, 0, nullptr, 0,
+                                 &ga, &d_aov);
+        if (rc)
+                return rc;
+        if (film)
+                VRT_CUDA(cudaMemcpyAsync(film, base, film_bytes, cudaMemcpyDeviceToHost, t->stream));
+        for (int i = 0; i < 4; ++i)
+                if (planes[i])
+                        VRT_CUDA(cudaMemcpyAsync(planes[i], base + off[i + 1], plane_bytes, cudaMemcpyDeviceToHost,
+                                                 t->stream));
+        if (aov->hits)
+                VRT_CUDA(cudaMemcpyAsync(aov->hits, base + off[5], hit_bytes, cudaMemcpyDeviceToHost, t->stream));
+        VRT_CUDA(cudaStreamSynchronize(t->stream));
+        return VRT_OK;
+}
+
+int vrt_gi_render_aov(const vrt_tree* t, const vrt_camera* cam, const float kd[3], float res, int x0, int y0, int x1,
+                      int y1, float* film_or_null, const vrt_gi_aov* aov)
+{
+        return gi_render_aov_common(t, cam, kd, res, x0, y0, x1, y1, film_or_null, aov, false);
+}
+
+int vrt_gi_render_aov_dev(const vrt_tree* t, const vrt_camera* cam, const float kd[3], float res, int x0, int y0,
+                          int x1, int y1, float* d_film_or_null, const vrt_gi_aov* d_aov)
+{
+        return gi_render_aov_common(t, cam, kd, res, x0, y0, x1, y1, d_film_or_null, d_aov, true);
+}
+
 int vrt_debug_param_check(uint64_t out[2])
 {
         if (!out) {

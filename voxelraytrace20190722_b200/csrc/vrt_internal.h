@@ -217,11 +217,12 @@ int import_leaves(vrt_tree* t, int max_depth, const float root_aabb[6], uint64_t
                   const uint32_t* leaf_cell, const uint32_t* leaf_count,
                   const uint32_t* leaf_refs);
 // trace (vrt_trace.cu)
-enum OutMode { OUT_HIT48 = 0, OUT_HIT16 = 1, OUT_FILM = 2, OUT_COUNT = 3, OUT_HIT16_FILM = 4, OUT_SPLAT = 5, OUT_GI_FILM = 6 };
+enum OutMode { OUT_HIT48 = 0, OUT_HIT16 = 1, OUT_FILM = 2, OUT_COUNT = 3, OUT_HIT16_FILM = 4, OUT_SPLAT = 5, OUT_GI_FILM = 6,
+              OUT_GI_AOV = 7 };
 int launch_trace_rays(const vrt_tree* t, const vrt_ray* d_rays, uint64_t n, vrt_hit* d_out);
 // band_h > 0: rows [y0,y1) are LOCAL rows of a banded shard; local row r maps to film row
 // y0_film + (r / band_h) * band_pitch + r % band_h (y0 then carries y0_film, y1 = y0 + local rows).
-struct GiArgs {  // OUT_SPLAT / OUT_GI_FILM: default material colour, cone-trace min_voxel_size
+struct GiArgs {  // OUT_SPLAT / OUT_GI_FILM / OUT_GI_AOV: default material colour, cone-trace min_voxel_size
         float kd[3];
         float res;
         const float4* steps = nullptr;  // step table of the cone trace for (res, root box), see gi_step_table
@@ -229,7 +230,7 @@ struct GiArgs {  // OUT_SPLAT / OUT_GI_FILM: default material colour, cone-trace
 int launch_trace_camera(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, int x0,
                         int y0, int x1, int y1, void* d_out, OutMode mode, int band_h = 0,
                         int band_pitch = 0, void* d_out2 = nullptr, int film_full = 0,
-                        const GiArgs* gi = nullptr);
+                        const GiArgs* gi = nullptr, const vrt_gi_aov* aov = nullptr);
 int launch_film_encode(const vrt_tree* t, const float* d_film, uint64_t npix, int fmt, uint8_t* d_out);
 // mean device time (ms) of the last n trace launches (waits for them)
 int trace_ms_mean(const vrt_tree* t, int last_n, double* ms);

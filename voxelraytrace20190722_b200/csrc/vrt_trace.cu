@@ -78,6 +78,7 @@ struct TraceParams {
         // (k_tab_rel: the reference's (plane - o) of every slab test, evaluated once per table entry instead of once
         // per ray and node); null: the expansion subtracts itself
         const float4* tabrel[3];
+        vrt_gi_aov aov;  // OUT_GI_AOV: the per-pixel planes (include/vrt.h); a null member is not written
 };
 
 struct HitState {
@@ -1157,10 +1158,25 @@ __device__ __forceinline__ void shade(const TraceParams& p, const HitState& hs, 
         rgb[0] = rgb[1] = rgb[2] = c;
 }
 
+// The per-ray records, the film and the GI planes are written once and never read by the kernel: streaming stores
+// (st.global.cs) keep them from displacing octree lines in L2 (-DVRT_PLAIN_STORES: ordinary stores).
+#ifdef VRT_PLAIN_STORES
+#define VRT_STORE_OUT(ptr, val) (*(ptr) = (val))
+#else
+#define VRT_STORE_OUT(ptr, val) __stcs((ptr), (val))
+#endif
+
+// The factors of one trace() sample that hits (main.cc:10-30): the ISect normal the cone basis is built from, the
+// albedo, the cone-traced indirect light and the hit leaf's direct light toward the eye.  A miss leaves them +0.
+struct GiTerms {
+        float nrm[3], albedo[3], ind[3], dir[3];
+};
+
 // trace() of main.cc:10-30: sky on a miss, else albedo * (cone-traced indirect light + the leaf's
 // direct light toward the eye); Triangle::is_visible() is true, albedo = material diffuse.
+// g receives the factors (OUT_GI_AOV); the film mode discards them.
 __device__ __forceinline__ void shade_gi(const TraceParams& p, const HitState& hs, const float o[3], const float d[3],
-                                         uint32_t* s_col, float rgb[3])
+                                         uint32_t* s_col, float rgb[3], GiTerms& g)
 {
         if (!hs.hit) {
                 const float t = __double2float_rn(dmul(0.5, dadd((double)d[1], 1.0)));
@@ -1170,17 +1186,36 @@ __device__ __forceinline__ void shade_gi(const TraceParams& p, const HitState& h
                         rgb[k] = fadd(1.0f, fmul(fsub(v1[k], 1.0f), t));
                 return;
         }
-        float pos[3], nrm[3], ind[3], dir[3], albedo[3];
-        finish_isect(p.tree, hs, o, d, pos, nrm);
-        gi_albedo(p.tree, hs.tri, pos, p.kd3, albedo);
+        float pos[3];
+        finish_isect(p.tree, hs, o, d, pos, g.nrm);
+        gi_albedo(p.tree, hs.tri, pos, p.kd3, g.albedo);
         // the traversal is over: this thread's stack column doubles as the cone trace's path cache
-        gi_cone_trace_point(p.tree, p.root, reinterpret_cast<float*>(s_col), kTraceThreads, pos, nrm, p.gi_res, p.gi_steps,
-                            ind);
+        gi_cone_trace_point(p.tree, p.root, reinterpret_cast<float*>(s_col), kTraceThreads, pos, g.nrm, p.gi_res,
+                            p.gi_steps, g.ind);
         const float nd[3] = { -d[0], -d[1], -d[2] };
-        gi_compute_illum(p.tree.gi + (size_t)kGiStride * hs.leaf, nd, dir);
+        gi_compute_illum(p.tree.gi + (size_t)kGiStride * hs.leaf, nd, g.dir);
 #pragma unroll
         for (int k = 0; k < 3; ++k)
-                rgb[k] = fmul(albedo[k], fadd(ind[k], dir[k]));
+                rgb[k] = fmul(g.albedo[k], fadd(g.ind[k], g.dir[k]));
+}
+
+// film->add(px,py, v * (1/spp)) in sample order (main.cc:119-122), acc = +0 first: the pixel's sum, in the lane
+// of sample 0.  Every lane of the warp takes part (shuffles).
+__device__ __forceinline__ void accumulate_samples(const float v[3], int spp, float acc[3])
+{
+        const float wgt = (spp == 4) ? .25f : 1.f;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+                const float c = fmul(v[k], wgt);
+                if (spp == 4) {
+                        const float c1 = __shfl_down_sync(0xffffffffu, c, 1);
+                        const float c2 = __shfl_down_sync(0xffffffffu, c, 2);
+                        const float c3 = __shfl_down_sync(0xffffffffu, c, 3);
+                        acc[k] = fadd(fadd(fadd(fadd(0.f, c), c1), c2), c3);
+                } else {
+                        acc[k] = fadd(0.f, c);
+                }
+        }
 }
 
 // ---------------------------------------------------------------------------
@@ -1221,13 +1256,6 @@ k_trace_rays(const __grid_constant__ TraceParams p)
 // since the tiles of an SM are neighbours on the film (per-SM queues below: L1 hit rate 73 -> 87 %) the warps wait
 // less on memory, and the 1/d values that 64 registers push into local memory (re-read in every expansion and hull
 // test) cost more than the eighth CTA hides: hit16 5.92 -> 5.72 ms per headline frame.
-// The per-ray records and the film are written once and never read by the kernel: streaming stores
-// (st.global.cs) keep them from displacing octree lines in L2 (-DVRT_PLAIN_STORES: ordinary stores).
-#ifdef VRT_PLAIN_STORES
-#define VRT_STORE_OUT(ptr, val) (*(ptr) = (val))
-#else
-#define VRT_STORE_OUT(ptr, val) __stcs((ptr), (val))
-#endif
 template <int MODE, bool WS>
 #ifndef VRT_FILM_MIN_BLOCKS
 #define VRT_FILM_MIN_BLOCKS 7
@@ -1239,7 +1267,7 @@ template <int MODE, bool WS>
 #define VRT_GI_MIN_BLOCKS 5
 #endif
 __global__ void __launch_bounds__(kTraceThreads, (MODE == OUT_HIT16 || MODE == OUT_COUNT) ? VRT_HIT16_MIN_BLOCKS
-                                                 : (MODE == OUT_GI_FILM)                  ? VRT_GI_MIN_BLOCKS
+                                                 : (MODE == OUT_GI_FILM || MODE == OUT_GI_AOV) ? VRT_GI_MIN_BLOCKS
                                                                                           : VRT_FILM_MIN_BLOCKS)
 k_trace_camera(const __grid_constant__ TraceParams p)
 {
@@ -1456,38 +1484,30 @@ k_trace_camera(const __grid_constant__ TraceParams p)
                                 VRT_STORE_OUT(reinterpret_cast<uint4*>(p.out) + (pix * spp + s), q);
                         }
                 } else {
-                        if (MODE == OUT_HIT16_FILM && active) {
+                        // the hit records of OUT_HIT16_FILM and OUT_GI_AOV, stored before shading (hs is then dead
+                        // during the cone trace)
+                        if ((MODE == OUT_HIT16_FILM || (MODE == OUT_GI_AOV && p.aov.hits)) && active) {
                                 uint4 q;
                                 q.x = hs.hit ? (hs.leaf - p.tree.num_nodes + p.tree.num_leaves) : VRT_NO_TRI;
                                 q.y = hs.tri;
                                 q.z = __float_as_uint(hs.hit ? hs.t : 0.f);
                                 q.w = hs.hit ? 1u : 0u;
-                                VRT_STORE_OUT(reinterpret_cast<uint4*>(p.out) + (pix * spp + s), q);
+                                VRT_STORE_OUT(reinterpret_cast<uint4*>(MODE == OUT_GI_AOV ? (void*)p.aov.hits : p.out) +
+                                                      (pix * spp + s),
+                                              q);
                         }
                         float rgb[3] = { 0, 0, 0 };
+                        GiTerms g = {};
                         if (active) {
-                                if (MODE == OUT_GI_FILM)
-                                        shade_gi(p, hs, o, d, s_first, rgb);
+                                if (MODE == OUT_GI_FILM || MODE == OUT_GI_AOV)
+                                        shade_gi(p, hs, o, d, s_first, rgb, g);
                                 else
                                         shade<MODE == OUT_COUNT, WS>(p, hs, o, d, s_first, s_meta, s_list, wc, rgb);
                         }
-                        // film->add(px,py, c * (1/spp)) in sample order (main.cc:119-122)
-                        const float wgt = (spp == 4) ? .25f : 1.f;
                         float acc[3];
-#pragma unroll
-                        for (int k = 0; k < 3; ++k) {
-                                const float c = fmul(rgb[k], wgt);
-                                if (spp == 4) {
-                                        const float c1 = __shfl_down_sync(0xffffffffu, c, 1);
-                                        const float c2 = __shfl_down_sync(0xffffffffu, c, 2);
-                                        const float c3 = __shfl_down_sync(0xffffffffu, c, 3);
-                                        acc[k] = fadd(fadd(fadd(fadd(0.f, c), c1), c2), c3);
-                                } else {
-                                        acc[k] = fadd(0.f, c);
-                                }
-                        }
-                        if (active && s == 0) {
-                                void* const film = (MODE == OUT_HIT16_FILM) ? p.out2 : p.out;
+                        accumulate_samples(rgb, spp, acc);
+                        void* const film = (MODE == OUT_HIT16_FILM) ? p.out2 : p.out;
+                        if (active && s == 0 && (MODE != OUT_GI_AOV || film)) {
                                 const unsigned long long fpix = (MODE == OUT_HIT16_FILM && p.film_full)
                                                                     ? (unsigned long long)py * p.cam.nx + px
                                                                     : pix;
@@ -1504,6 +1524,24 @@ k_trace_camera(const __grid_constant__ TraceParams p)
                                         f[0] = (uint8_t)v;
                                         f[1] = (uint8_t)(v >> 8);
                                         f[2] = (uint8_t)(v >> 16);
+                                }
+                        }
+                        if (MODE == OUT_GI_AOV) {
+                                // the planes accumulate exactly as the film does (f32 whatever the film format); the
+                                // null tests are uniform
+                                float* const planes[4] = { p.aov.albedo, p.aov.direct, p.aov.indirect, p.aov.normal };
+                                const float* const terms[4] = { g.albedo, g.dir, g.ind, g.nrm };
+#pragma unroll
+                                for (int i = 0; i < 4; ++i) {
+                                        if (!planes[i])
+                                                continue;
+                                        accumulate_samples(terms[i], spp, acc);
+                                        if (active && s == 0) {
+                                                float* f = planes[i] + pix * 3ull;
+                                                VRT_STORE_OUT(f + 0, acc[0]);
+                                                VRT_STORE_OUT(f + 1, acc[1]);
+                                                VRT_STORE_OUT(f + 2, acc[2]);
+                                        }
                                 }
                         }
                 }
@@ -1641,7 +1679,7 @@ static size_t stack_bytes(const vrt_tree* t, OutMode mode = OUT_HIT48)
 {
         const int L = std::max(t->dev.L, 1);
         size_t words = (size_t)3 * (size_t)(L + 1);
-        if (mode == OUT_GI_FILM)  // the same column then holds the cone trace's path cache (vrt_gi.cuh)
+        if (mode == OUT_GI_FILM || mode == OUT_GI_AOV)  // the same column then holds the cone trace's path cache (vrt_gi.cuh)
                 words = std::max(words, (size_t)kGiPathWords * (size_t)L);
         return words * kTraceThreads * sizeof(uint32_t);
 }
@@ -1766,7 +1804,7 @@ static void camera_eye_host(const vrt_camera* cam, float eye[3])
 
 int launch_trace_camera(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, int x0, int y0,
                         int x1, int y1, void* d_out, OutMode mode, int band_h, int band_pitch, void* d_out2, int film_full,
-                        const GiArgs* gi)
+                        const GiArgs* gi, const vrt_gi_aov* aov)
 {
         if (x1 <= x0 || y1 <= y0)
                 return VRT_OK;
@@ -1800,6 +1838,8 @@ int launch_trace_camera(const vrt_tree* t, const vrt_camera* cam, const vrt_shad
                 p.gi_res = gi->res;
                 p.gi_steps = gi->steps;
         }
+        if (aov)
+                p.aov = *aov;
         if (sh) {
                 p.light[0] = sh->light_dir[0];
                 p.light[1] = sh->light_dir[1];
@@ -1852,6 +1892,7 @@ int launch_trace_camera(const vrt_tree* t, const vrt_camera* cam, const vrt_shad
         case OUT_HIT16_FILM: VRT_PICK(OUT_HIT16_FILM); break;
         case OUT_SPLAT: VRT_PICK(OUT_SPLAT); break;
         case OUT_GI_FILM: VRT_PICK(OUT_GI_FILM); break;
+        case OUT_GI_AOV: VRT_PICK(OUT_GI_AOV); break;
         default: VRT_PICK(OUT_FILM); break;
         }
 #undef VRT_PICK
