@@ -399,6 +399,22 @@ int vrt_gi_render_aov(const vrt_tree* tree, const vrt_camera* cam, const float k
                       int x1, int y1, float* film_or_null, const vrt_gi_aov* aov);
 int vrt_gi_render_aov_dev(const vrt_tree* tree, const vrt_camera* cam, const float kd[3], float res, int x0, int y0,
                           int x1, int y1, float* d_film_or_null, const vrt_gi_aov* d_aov);
+/* The GI film and its planes (vrt_gi_render_aov) in the banded, pipelined form of vrt_gi_render_bands_async, for a
+ * denoiser or compositor that reads the planes in host memory every frame.  aov_full holds HOST pointers to FULL
+ * frames: each float plane [ny][nx][3] float32, hits [ny][nx][spp] vrt_hit16, and film_full_or_null (NULL: no film)
+ * [ny][nx][...] in the handle's film format.  This handle's bands of every non-NULL output are rendered by one launch
+ * into one of two device buffers and DMA-copied to their final rows; every other byte of those frames, and every
+ * NULL member, is left untouched.  Every byte written equals vrt_gi_render_aov for the same camera, kd, res, film
+ * format and GI state; the film is bytewise vrt_gi_render_bands_async's.  The frames should be pinned (on a
+ * multi-process node: shared mappings every rank has registered) and stay valid until vrt_tree_sync; the
+ * vrt_gi_aov struct, cam and kd are read during the call only.  A request with every plane NULL is VRT_ERR_ARG
+ * (the film alone is vrt_gi_render_bands_async); so are a missing vrt_gi_init, bad bands and a NULL cam, kd or
+ * aov_full.  A handle with no rows in `bands` returns VRT_OK and enqueues nothing, and a rejected call enqueues
+ * nothing.  The frames share the pipeline (two kernel streams, one copy stream) of vrt_render_camera_async,
+ * vrt_render_bands_async and vrt_gi_render_bands_async, so the four calls may be interleaved on one handle, and
+ * the light-map calls may be issued between enqueued frames without a sync, as for vrt_gi_render_bands_async. */
+int vrt_gi_render_aov_bands_async(const vrt_tree* tree, const vrt_camera* cam, const float kd[3], float res,
+                                  const vrt_bands* bands, float* film_full_or_null, const vrt_gi_aov* aov_full);
 /* The GI rows on the replicas of a vrt_mgpu (main.cc:75-126 over N devices).  vrt_mgpu_create copies the
  * geometry only: materials and the GI state are set through these calls, each of which runs the single-device
  * call on every replica (host pointers, like the single-device calls).  The light pass runs on every replica --
@@ -410,7 +426,11 @@ int vrt_gi_render_aov_dev(const vrt_tree* tree, const vrt_camera* cam, const flo
  *   vrt_mgpu_gi_render_async  the GI film (main.cc:117-123): the 8-row bands dealt round-robin, each replica's
  *                             through vrt_gi_render_bands_async into film_rgb_full (pinned host memory); the
  *                             frame is complete after vrt_mgpu_sync.  Alternate between two host frames.
- *   vrt_mgpu_gi_render        vrt_mgpu_gi_render_async + vrt_mgpu_sync */
+ *   vrt_mgpu_gi_render        vrt_mgpu_gi_render_async + vrt_mgpu_sync
+ *   vrt_mgpu_gi_render_aov_async  the GI film (optional) and its planes: the same 8-row bands, each replica's
+ *                             through vrt_gi_render_aov_bands_async into the full host frames of film_full_or_null
+ *                             and aov_full (pinned); complete after vrt_mgpu_sync.  Alternate between two sets.
+ *   vrt_mgpu_gi_render_aov    vrt_mgpu_gi_render_aov_async + vrt_mgpu_sync */
 int vrt_mgpu_set_materials(vrt_mgpu* m, const float* tri_uv, const uint32_t* tri_mtl, uint32_t num_mtl,
                            const float* kd, const int32_t* mtl_tex, uint32_t num_tex, const vrt_texture* tex);
 int vrt_mgpu_gi_init(vrt_mgpu* m);
@@ -418,6 +438,10 @@ int vrt_mgpu_gi_splat_camera(vrt_mgpu* m, const vrt_camera* light_cam, const flo
 int vrt_mgpu_gi_filter(vrt_mgpu* m);
 int vrt_mgpu_gi_render_async(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_rgb_full);
 int vrt_mgpu_gi_render(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_rgb_full);
+int vrt_mgpu_gi_render_aov_async(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res,
+                                 float* film_full_or_null, const vrt_gi_aov* aov_full);
+int vrt_mgpu_gi_render_aov(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_full_or_null,
+                           const vrt_gi_aov* aov_full);
 /* vrt_mean_kernel_ms of replica `index` (0 for a bad index): the per-device balance of a multi-GPU frame loop */
 double vrt_mgpu_mean_kernel_ms(vrt_mgpu* m, int index, int last_n);
 

@@ -84,6 +84,7 @@ SYMBOLS = [
     "vrt_gi_render_bands_async", "vrt_mgpu_set_materials", "vrt_mgpu_gi_init", "vrt_mgpu_gi_splat_camera",
     "vrt_mgpu_gi_filter", "vrt_mgpu_gi_render_async", "vrt_mgpu_gi_render", "vrt_mgpu_mean_kernel_ms",
     "vrt_gi_render_aov", "vrt_gi_render_aov_dev",
+    "vrt_gi_render_aov_bands_async", "vrt_mgpu_gi_render_aov_async", "vrt_mgpu_gi_render_aov",
 ]
 
 _lib = None
@@ -179,6 +180,10 @@ def load(build_if_missing: bool = True):
     L.vrt_gi_render_bands_async.argtypes = [vp, C.POINTER(vrt_camera), vp, f32, C.POINTER(vrt_bands), vp]
     L.vrt_gi_render_aov.argtypes = [vp, C.POINTER(vrt_camera), vp, f32, i32, i32, i32, i32, vp, C.POINTER(vrt_gi_aov)]
     L.vrt_gi_render_aov_dev.argtypes = L.vrt_gi_render_aov.argtypes
+    L.vrt_gi_render_aov_bands_async.argtypes = [vp, C.POINTER(vrt_camera), vp, f32, C.POINTER(vrt_bands), vp,
+                                                C.POINTER(vrt_gi_aov)]
+    L.vrt_mgpu_gi_render_aov_async.argtypes = [vp, C.POINTER(vrt_camera), vp, f32, vp, C.POINTER(vrt_gi_aov)]
+    L.vrt_mgpu_gi_render_aov.argtypes = L.vrt_mgpu_gi_render_aov_async.argtypes
     L.vrt_mgpu_set_materials.argtypes = [vp, vp, vp, C.c_uint32, vp, vp, C.c_uint32, vp]
     L.vrt_mgpu_gi_init.argtypes = [vp]
     L.vrt_mgpu_gi_splat_camera.argtypes = [vp, C.POINTER(vrt_camera), vp]
@@ -564,13 +569,22 @@ class Octree:
         """gi_render_aov into device memory, enqueued on the handle's stream: d_planes maps plane names to device
         pointers (float32 [h, w, 3], hits vrt_hit16 [h, w, spp]); d_film_or_0 = 0 writes no film."""
         x0, y0, x1, y1 = rect if rect else (0, 0, cam.nx, cam.ny)
-        unknown = set(d_planes) - set(GI_AOV_PLANES)
-        if unknown:
-            raise ValueError(f"unknown GI planes {sorted(unknown)}")
-        aov = vrt_gi_aov(**{n: int(p) for n, p in d_planes.items() if p})
+        aov = _gi_aov(d_planes)
         kd = np.ascontiguousarray(kd, np.float32)
         _check(load().vrt_gi_render_aov_dev(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)), x0, y0, x1,
                                             y1, C.c_void_p(int(d_film_or_0) or None), C.byref(aov)))
+
+    def gi_render_aov_bands_async(self, cam: Camera, kd, res, host_film_ptr_or_0, host_planes: dict, band_h,
+                                  band_first, band_stride):
+        """gi_render_aov in the banded, pipelined form of gi_render_bands_async: host_planes maps plane names to
+        (pinned) FULL host frames (float32 [ny, nx, 3], hits vrt_hit16 [ny, nx, spp]), of which only this handle's
+        band rows are written, like the film's (host_film_ptr_or_0 = 0: no film); asynchronous, see sync()."""
+        aov = _gi_aov(host_planes)
+        kd = np.ascontiguousarray(kd, np.float32)
+        b = vrt_bands(int(band_h), int(band_first), int(band_stride))
+        _check(load().vrt_gi_render_aov_bands_async(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)),
+                                                    C.byref(b), C.c_void_p(int(host_film_ptr_or_0) or None),
+                                                    C.byref(aov)))
 
     def render_async(self, cam: Camera, out, light=None, kd=0.8, rect=None, shadow_eps=None):
         """Pipelined frame loop: enqueue one frame whose film lands in the (pinned) host array
@@ -670,6 +684,20 @@ class MultiGpu:
         _check(load().vrt_mgpu_gi_render(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)),
                                          C.c_void_p(int(host_frame_ptr))))
 
+    def gi_render_aov_async(self, cam: Camera, kd, res, host_film_ptr_or_0, host_planes: dict):
+        """Enqueue one GI film (host_film_ptr_or_0 = 0: none) and its planes (Octree.gi_render_aov_bands_async's
+        host_planes) over the replicas, 8-row bands round-robin; call sync() before reading."""
+        aov = _gi_aov(host_planes)
+        kd = np.ascontiguousarray(kd, np.float32)
+        _check(load().vrt_mgpu_gi_render_aov_async(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)),
+                                                   C.c_void_p(int(host_film_ptr_or_0) or None), C.byref(aov)))
+
+    def gi_render_aov(self, cam: Camera, kd, res, host_film_ptr_or_0, host_planes: dict):
+        aov = _gi_aov(host_planes)
+        kd = np.ascontiguousarray(kd, np.float32)
+        _check(load().vrt_mgpu_gi_render_aov(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)),
+                                             C.c_void_p(int(host_film_ptr_or_0) or None), C.byref(aov)))
+
     def mean_kernel_ms(self, index, last_n):
         """Mean device time of the last `last_n` kernels of replica `index` (waits for them)."""
         return float(load().vrt_mgpu_mean_kernel_ms(self._h, int(index), int(last_n)))
@@ -678,6 +706,14 @@ class MultiGpu:
         if self._h:
             load().vrt_mgpu_free(self._h)
             self._h = None
+
+
+def _gi_aov(planes: dict) -> vrt_gi_aov:
+    """A vrt_gi_aov of the pointers in `planes` (names of GI_AOV_PLANES; 0 / None: not written)."""
+    unknown = set(planes) - set(GI_AOV_PLANES)
+    if unknown:
+        raise ValueError(f"unknown GI planes {sorted(unknown)}")
+    return vrt_gi_aov(**{n: int(p) for n, p in planes.items() if p})
 
 
 def _set_materials(fn, h, tri_uv, tri_mtl, kd, mtl_tex, textures):

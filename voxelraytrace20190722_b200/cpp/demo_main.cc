@@ -7,7 +7,8 @@
 // With --dump <file> it also writes (hit,tri,cell,pos,nrm) per ray for the parity test.
 // With --gi <file> it also writes main.cc's cone-traced GI film (float, plus <file>.hdr); with --gi-devices 0,0,...
 // as well, the same film rendered through gi::MultiGpu on those devices goes to <file>.mgpu; with --gi-aov <prefix> as
-// well, what that film is made of goes to <prefix>.{albedo,direct,indirect,normal}.hdr.
+// well, what that film is made of goes to <prefix>.{albedo,direct,indirect,normal}.hdr (and, with --gi-devices, the
+// same planes rendered through the replicas to <prefix>.mgpu.{albedo,direct,indirect,normal}.hdr).
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -204,8 +205,9 @@ int main(int argc, char** argv)
                         FILE* f = std::fopen(gi_dump, "wb");
                         std::fwrite(d.data(), sizeof(float), d.size(), f);
                         std::fclose(f);
-                        if (gi_aov) {
-                                // the film's factors (a denoiser's albedo and normal guides, the light terms)
+                        // the film's factors (a denoiser's albedo and normal guides, the light terms), rendered by
+                        // `render` and written to <prefix><infix>.<plane>.hdr
+                        auto write_planes = [&](const char* infix, auto&& render) {
                                 Film albedo(1.f, 1.f, nx, ny), direct(1.f, 1.f, nx, ny), indirect(1.f, 1.f, nx, ny),
                                         normal(1.f, 1.f, nx, ny);
                                 gi::GiAov aov;
@@ -213,12 +215,15 @@ int main(int argc, char** argv)
                                 aov.direct = &direct;
                                 aov.indirect = &indirect;
                                 aov.normal = &normal;
-                                render_gi_aov_gpu(nullptr, cam, &root, 4, kd, res, aov);
+                                render(aov);
                                 const std::pair<const char*, const Film*> planes[4] = {
                                         { "albedo", &albedo }, { "direct", &direct }, { "indirect", &indirect }, { "normal", &normal }
                                 };
                                 for (const auto& pl : planes)
-                                        write_hdr((std::string(gi_aov) + "." + pl.first + ".hdr").c_str(), *pl.second);
+                                        write_hdr((std::string(gi_aov) + infix + "." + pl.first + ".hdr").c_str(), *pl.second);
+                        };
+                        if (gi_aov) {
+                                write_planes("", [&](gi::GiAov& aov) { render_gi_aov_gpu(nullptr, cam, &root, 4, kd, res, aov); });
                                 std::printf("GI planes written\n");
                         }
                         if (!gi_devices.empty()) {
@@ -233,6 +238,12 @@ int main(int argc, char** argv)
                                 FILE* mf = std::fopen((std::string(gi_dump) + ".mgpu").c_str(), "wb");
                                 std::fwrite(md.data(), sizeof(float), md.size(), mf);
                                 std::fclose(mf);
+                                if (gi_aov) {
+                                        write_planes(".mgpu", [&](gi::GiAov& aov) {
+                                                render_gi_aov_gpu(nullptr, cam, replicas, 4, kd, res, aov);
+                                        });
+                                        std::printf("GI planes on %zu replicas written\n", gi_devices.size());
+                                }
                         }
                 }
                 std::printf("success.\n");

@@ -364,10 +364,10 @@ void render_gi_gpu(Film* film, Camera& cam, gi::VoxelOctree* root, int spp, cons
         check(vrt_gi_render_camera(t, &c, k, res, 0, 0, film->nx, film->ny, &film->data()->x), "render_gi_gpu");
 }
 
-void render_gi_aov_gpu(Film* film_or_null, Camera& cam, gi::VoxelOctree* root, int spp, const jql::Vec3& kd, float res,
-                       gi::GiAov& aov)
+// The film geometry of a render_gi_aov_gpu call (the film, else the first float plane; all of one size), with
+// aov.hits resized for it; returns the vrt_gi_aov of aov's buffers.
+static vrt_gi_aov gi_aov_native(const Film* film_or_null, int spp, gi::GiAov& aov, const Film** geometry)
 {
-        vrt_tree* t = gi::gi_tree(root, "render_gi_aov_gpu");
         Film* const planes[4] = { aov.albedo, aov.direct, aov.indirect, aov.normal };
         const Film* geo = film_or_null;
         for (Film* p : planes)
@@ -378,14 +378,23 @@ void render_gi_aov_gpu(Film* film_or_null, Camera& cam, gi::VoxelOctree* root, i
         for (Film* p : planes)
                 if (p && (p->nx != geo->nx || p->ny != geo->ny))
                         throw std::runtime_error("render_gi_aov_gpu: the planes and the film differ in size");
-        const vrt_camera c = cam.native(*geo, spp);
-        const float k[3] = { kd.x, kd.y, kd.z };
         if (aov.hits)
                 aov.hits->resize((size_t)geo->nx * geo->ny * spp);
         float* dst[4];
         for (int i = 0; i < 4; ++i)
                 dst[i] = planes[i] ? &planes[i]->data()->x : nullptr;
-        const vrt_gi_aov a = { dst[0], dst[1], dst[2], dst[3], aov.hits ? aov.hits->data() : nullptr };
+        *geometry = geo;
+        return vrt_gi_aov{ dst[0], dst[1], dst[2], dst[3], aov.hits ? aov.hits->data() : nullptr };
+}
+
+void render_gi_aov_gpu(Film* film_or_null, Camera& cam, gi::VoxelOctree* root, int spp, const jql::Vec3& kd, float res,
+                       gi::GiAov& aov)
+{
+        vrt_tree* t = gi::gi_tree(root, "render_gi_aov_gpu");
+        const Film* geo = nullptr;
+        const vrt_gi_aov a = gi_aov_native(film_or_null, spp, aov, &geo);
+        const vrt_camera c = cam.native(*geo, spp);
+        const float k[3] = { kd.x, kd.y, kd.z };
         check(vrt_gi_render_aov(t, &c, k, res, 0, 0, geo->nx, geo->ny, film_or_null ? &film_or_null->data()->x : nullptr,
                                 &a),
               "render_gi_aov_gpu");
@@ -412,6 +421,30 @@ void render_gi_gpu(Film* film, Camera& cam, gi::MultiGpu& replicas, int spp, con
         if (locked)
                 vrt_host_unregister(dst);
         check(rc, "render_gi_gpu");
+}
+
+void render_gi_aov_gpu(Film* film_or_null, Camera& cam, gi::MultiGpu& replicas, int spp, const jql::Vec3& kd, float res,
+                       gi::GiAov& aov)
+{
+        const Film* geo = nullptr;
+        const vrt_gi_aov a = gi_aov_native(film_or_null, spp, aov, &geo);
+        const vrt_camera c = cam.native(*geo, spp);
+        const float k[3] = { kd.x, kd.y, kd.z };
+        float* const film = film_or_null ? &film_or_null->data()->x : nullptr;
+        // every output page-locked for the call, as in render_gi_gpu (a range that cannot be locked still receives
+        // its bands, staged by the driver)
+        const uint64_t plane_bytes = (uint64_t)geo->nx * geo->ny * 3 * sizeof(float);
+        void* const dst[6] = { film, a.albedo, a.direct, a.indirect, a.normal, a.hits };
+        const uint64_t bytes[6] = { plane_bytes, plane_bytes, plane_bytes, plane_bytes, plane_bytes,
+                                    (uint64_t)geo->nx * geo->ny * spp * sizeof(vrt_hit16) };
+        bool locked[6] = {};
+        for (int i = 0; i < 6; ++i)
+                locked[i] = dst[i] && vrt_host_register(dst[i], bytes[i]) == VRT_OK;
+        const int rc = vrt_mgpu_gi_render_aov(replicas.native(), &c, k, res, film, &a);
+        for (int i = 0; i < 6; ++i)
+                if (locked[i])
+                        vrt_host_unregister(dst[i]);
+        check(rc, "render_gi_aov_gpu");
 }
 
 // vrt_set_materials / vrt_mgpu_set_materials with the mirror's material records

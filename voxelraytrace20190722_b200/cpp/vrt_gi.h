@@ -196,6 +196,11 @@ struct GiAov {
 // geometry.
 void render_gi_aov_gpu(Film* film_or_null, Camera& cam, gi::VoxelOctree* root, int spp, const jql::Vec3& kd, float res,
                        gi::GiAov& aov);
+// The same on the replicas of a gi::MultiGpu: 8-row bands dealt round-robin, each device copying its bands straight
+// into the film and the planes (page-locked for the call).  Returns when the work is done; every output equals the
+// single-device one bytewise.
+void render_gi_aov_gpu(Film* film_or_null, Camera& cam, gi::MultiGpu& replicas, int spp, const jql::Vec3& kd, float res,
+                       gi::GiAov& aov);
 
 // Materials for the GI passes (the half of gi::Triangle the geometry mirror leaves out: t_[3] and
 // tinyobj::material_t::diffuse / diffuse_texname, voxel_octree.h:110-111).  uv holds three texture

@@ -1322,15 +1322,39 @@ int vrt_render_bands_dev(const vrt_tree* t, const vrt_camera* cam, const vrt_sha
         return bands_common(t, cam, sh, b, d_film_rgb, OUT_FILM);
 }
 
+// One output's compact band rows (src: this rank's rows, band after band) to their final rows of the full host
+// frame dst_full: the full bands by one 2-D copy ("row" = one band of band_h frame rows), then the last, shorter band.
+static int copy_bands_to_host(char* dst_full, const char* src, size_t row_bytes, const vrt_bands* b, int rows,
+                              cudaStream_t s)
+{
+        const size_t band_bytes = (size_t)b->band_h * row_bytes;
+        const int full_bands = rows / b->band_h, tail_rows = rows % b->band_h;
+        char* dst = dst_full + (size_t)b->band_first * band_bytes;
+        static int dbg_no_copy = -1;  // VRT_DEBUG_NO_COPY=1: diagnostic only (frames never reach the host)
+        if (dbg_no_copy < 0) {
+                const char* e = getenv("VRT_DEBUG_NO_COPY");
+                dbg_no_copy = (e && e[0] == '1') ? 1 : 0;
+        }
+        if (full_bands && !dbg_no_copy)
+                VRT_CUDA(cudaMemcpy2DAsync(dst, (size_t)b->band_stride * band_bytes, src, band_bytes, band_bytes,
+                                           (size_t)full_bands, cudaMemcpyDeviceToHost, s));
+        if (tail_rows)
+                VRT_CUDA(cudaMemcpyAsync(dst + (size_t)full_bands * b->band_stride * band_bytes,
+                                         src + (size_t)full_bands * band_bytes, (size_t)tail_rows * row_bytes,
+                                         cudaMemcpyDeviceToHost, s));
+        return VRT_OK;
+}
+
 // Multi-GPU frame loop to HOST memory: this rank's bands are rendered into one of two device
 // band buffers and copied by one strided DMA (cudaMemcpy2DAsync: one row per band) straight to
 // their final rows of the full host frame, which every rank of the node maps (shared + pinned),
 // so the N ranks use their N PCIe links in parallel and the copy of frame k overlaps the kernel
 // of frame k+1 -- the N-GPU counterpart of vrt_render_camera_async.  mode OUT_FILM: the harness
 // film (sh); OUT_GI_FILM: the cone-traced GI film (gi->kd, gi->res; the step table is filled on
-// the frame's kernel stream).
+// the frame's kernel stream); OUT_GI_AOV: the GI film (film_rgb_full may be NULL) plus the planes
+// of aov_full (host frames), whose compact band rows share the frame slot's one device buffer.
 static int bands_async_common(const vrt_tree* tc, const vrt_camera* cam, const vrt_shade* sh, const GiArgs* gi,
-                              const vrt_bands* b, float* film_rgb_full, OutMode mode)
+                              const vrt_gi_aov* aov_full, const vrt_bands* b, float* film_rgb_full, OutMode mode)
 {
         int rc = check_tree(tc);
         if (rc)
@@ -1343,22 +1367,36 @@ static int bands_async_common(const vrt_tree* tc, const vrt_camera* cam, const v
                 return rows;
         if (rows == 0)
                 return VRT_OK;
-        if (!film_rgb_full || (mode == OUT_FILM ? !sh : !gi)) {
+        if ((mode == OUT_GI_AOV ? !aov_full : !film_rgb_full) || (mode == OUT_FILM ? !sh : !gi)) {
                 set_error("null out/shade pointer");
                 return VRT_ERR_ARG;
         }
-        if (mode == OUT_GI_FILM && !tc->dev.gi) {
+        if (mode != OUT_FILM && !tc->dev.gi) {
                 set_error("vrt_gi_init has not been called on this tree");
                 return VRT_ERR_ARG;
         }
+        // the outputs (film, albedo, direct, indirect, normal, hits): full host frames, and the bytes of one row
+        const vrt_gi_aov none = {};
+        const vrt_gi_aov& a = mode == OUT_GI_AOV ? *aov_full : none;
+        char* const dst[6] = { reinterpret_cast<char*>(film_rgb_full), reinterpret_cast<char*>(a.albedo),
+                               reinterpret_cast<char*>(a.direct), reinterpret_cast<char*>(a.indirect),
+                               reinterpret_cast<char*>(a.normal), reinterpret_cast<char*>(a.hits) };
+        const size_t plane_row = (size_t)cam->nx * 12;
+        const size_t row_bytes[6] = { (size_t)cam->nx * (size_t)vrt_film_pixel_bytes(tc->film_fmt), plane_row,
+                                      plane_row, plane_row, plane_row, (size_t)cam->nx * cam->spp * sizeof(vrt_hit16) };
+        // their compact band rows in the frame slot's one device buffer, each part 256-byte aligned
+        uint64_t off[6] = {}, bytes = 0;
+        for (int i = 0; i < 6; ++i)
+                if (dst[i]) {
+                        off[i] = (bytes + 255) & ~255ull;
+                        bytes = off[i] + (uint64_t)rows * row_bytes[i];
+                }
         vrt_tree* t = const_cast<vrt_tree*>(tc);
         rc = async_pipeline_prepare(t);
         if (rc)
                 return rc;
         cudaStream_t ks = async_kernel_stream(t);
         const int k = (int)(t->n_async_frames & 1);
-        const size_t row_bytes = (size_t)cam->nx * (size_t)vrt_film_pixel_bytes(t->film_fmt);
-        const uint64_t bytes = (uint64_t)rows * row_bytes;
         if (t->film_dev[k].cap < bytes) {
                 VRT_CUDA(cudaStreamSynchronize(t->copy_stream));  // nothing may still read the old buffer
                 if (t->film_dev[k].reserve(bytes))
@@ -1366,38 +1404,35 @@ static int bands_async_common(const vrt_tree* tc, const vrt_camera* cam, const v
         }
         if (t->n_async_frames >= 2)  // the copy that last read this device buffer must be done
                 VRT_CUDA(cudaStreamWaitEvent(ks, t->film_copied[k], 0));
+        char* const base = static_cast<char*>(t->film_dev[k].p);
+        vrt_gi_aov d_aov = {};
+        float** const d_planes[4] = { &d_aov.albedo, &d_aov.direct, &d_aov.indirect, &d_aov.normal };
+        for (int i = 0; i < 4; ++i)
+                if (dst[i + 1])
+                        *d_planes[i] = reinterpret_cast<float*>(base + off[i + 1]);
+        if (dst[5])
+                d_aov.hits = reinterpret_cast<vrt_hit16*>(base + off[5]);
         const int y0 = b->band_first * b->band_h;
         t->launch_stream = ks;
         GiArgs ga{};
-        if (mode == OUT_GI_FILM) {
+        if (mode != OUT_FILM) {
                 ga = *gi;
                 rc = gi_step_table(t, ga.res, &ga.steps);
         }
         if (!rc)
-                rc = launch_trace_camera(t, cam, sh, 0, y0, cam->nx, y0 + rows, t->film_dev[k].p, mode, b->band_h,
-                                         b->band_stride * b->band_h, nullptr, 0, mode == OUT_GI_FILM ? &ga : nullptr);
+                rc = launch_trace_camera(t, cam, sh, 0, y0, cam->nx, y0 + rows, dst[0] ? base + off[0] : nullptr, mode,
+                                         b->band_h, b->band_stride * b->band_h, nullptr, 0,
+                                         mode == OUT_FILM ? nullptr : &ga, mode == OUT_GI_AOV ? &d_aov : nullptr);
         t->launch_stream = nullptr;
         if (rc)
                 return rc;
         VRT_CUDA(cudaEventRecord(t->film_ready[k], ks));
         VRT_CUDA(cudaStreamWaitEvent(t->copy_stream, t->film_ready[k], 0));
-        // full bands: one 2-D copy, "row" = one band of band_h film rows; then the last, shorter band
-        const size_t band_bytes = (size_t)b->band_h * row_bytes;
-        const int full_bands = rows / b->band_h, tail_rows = rows % b->band_h;
-        char* dst = reinterpret_cast<char*>(film_rgb_full) + (size_t)y0 * row_bytes;
-        const char* src = static_cast<const char*>(t->film_dev[k].p);
-        static int dbg_no_copy = -1;  // VRT_DEBUG_NO_COPY=1: diagnostic only (frames never reach the host)
-        if (dbg_no_copy < 0) {
-                const char* e = getenv("VRT_DEBUG_NO_COPY");
-                dbg_no_copy = (e && e[0] == '1') ? 1 : 0;
-        }
-        if (full_bands && !dbg_no_copy)
-                VRT_CUDA(cudaMemcpy2DAsync(dst, (size_t)b->band_stride * band_bytes, src, band_bytes, band_bytes,
-                                           (size_t)full_bands, cudaMemcpyDeviceToHost, t->copy_stream));
-        if (tail_rows)
-                VRT_CUDA(cudaMemcpyAsync(dst + (size_t)full_bands * b->band_stride * band_bytes,
-                                         src + (size_t)full_bands * band_bytes, (size_t)tail_rows * row_bytes,
-                                         cudaMemcpyDeviceToHost, t->copy_stream));
+        for (int i = 0; i < 6 && !rc; ++i)
+                if (dst[i])
+                        rc = copy_bands_to_host(dst[i], base + off[i], row_bytes[i], b, rows, t->copy_stream);
+        if (rc)
+                return rc;
         VRT_CUDA(cudaEventRecord(t->film_copied[k], t->copy_stream));
         t->n_async_frames++;
         return VRT_OK;
@@ -1406,7 +1441,7 @@ static int bands_async_common(const vrt_tree* tc, const vrt_camera* cam, const v
 int vrt_render_bands_async(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, const vrt_bands* b,
                            float* film_rgb_full)
 {
-        return bands_async_common(t, cam, sh, nullptr, b, film_rgb_full, OUT_FILM);
+        return bands_async_common(t, cam, sh, nullptr, nullptr, b, film_rgb_full, OUT_FILM);
 }
 
 // The cone-traced GI film (vrt_gi_render_camera) through the same banded, pipelined path.
@@ -1418,7 +1453,32 @@ int vrt_gi_render_bands_async(const vrt_tree* t, const vrt_camera* cam, const fl
                 return VRT_ERR_ARG;
         }
         const GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
-        return bands_async_common(t, cam, nullptr, &ga, b, film_rgb_full, OUT_GI_FILM);
+        return bands_async_common(t, cam, nullptr, &ga, nullptr, b, film_rgb_full, OUT_GI_FILM);
+}
+
+// kd and the planes of a banded plane request: VRT_ERR_ARG for a null pointer or a request without any plane
+static int check_gi_aov_request(const float kd[3], const vrt_gi_aov* aov)
+{
+        if (!kd || !aov) {
+                set_error("null argument");
+                return VRT_ERR_ARG;
+        }
+        if (!aov->albedo && !aov->direct && !aov->indirect && !aov->normal && !aov->hits) {
+                set_error("every GI plane is NULL (the film alone is the banded GI film call)");
+                return VRT_ERR_ARG;
+        }
+        return VRT_OK;
+}
+
+// The GI film and its planes (vrt_gi_render_aov) through the same banded, pipelined path.
+int vrt_gi_render_aov_bands_async(const vrt_tree* t, const vrt_camera* cam, const float kd[3], float res,
+                                  const vrt_bands* b, float* film_full_or_null, const vrt_gi_aov* aov_full)
+{
+        const int rc = check_gi_aov_request(kd, aov_full);
+        if (rc)
+                return rc;
+        const GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
+        return bands_async_common(t, cam, nullptr, &ga, aov_full, b, film_full_or_null, OUT_GI_AOV);
 }
 
 // ---- single-process multi-GPU render (SURVEY.md 8e; replaces render_mt camera.h:41-68 over N devices) -------
@@ -1560,20 +1620,20 @@ int mgpu_each(vrt_mgpu* m, F&& f)
 
 // one frame: the 8-row bands dealt round-robin, each replica through its bands_async_common pipeline
 static int mgpu_bands_async(vrt_mgpu* m, const vrt_camera* cam, const vrt_shade* sh, const GiArgs* gi,
-                            float* film_rgb_full, OutMode mode)
+                            const vrt_gi_aov* aov_full, float* film_rgb_full, OutMode mode)
 {
         const int n = m ? (int)m->trees.size() : 0;
         return mgpu_each(m, [&](int i, vrt_tree* t) {
                 if (cam && (long)i * m->band_h >= cam->ny)
                         return (int)VRT_OK;  // more devices than bands
                 const vrt_bands b = { m->band_h, i, n };
-                return bands_async_common(t, cam, sh, gi, &b, film_rgb_full, mode);
+                return bands_async_common(t, cam, sh, gi, aov_full, &b, film_rgb_full, mode);
         });
 }
 
 int vrt_mgpu_render_async(vrt_mgpu* m, const vrt_camera* cam, const vrt_shade* sh, float* film_rgb_full)
 {
-        return mgpu_bands_async(m, cam, sh, nullptr, film_rgb_full, OUT_FILM);
+        return mgpu_bands_async(m, cam, sh, nullptr, nullptr, film_rgb_full, OUT_FILM);
 }
 
 int vrt_mgpu_sync(vrt_mgpu* m)
@@ -1636,12 +1696,30 @@ int vrt_mgpu_gi_render_async(vrt_mgpu* m, const vrt_camera* cam, const float kd[
                 return VRT_ERR_ARG;
         }
         const GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
-        return mgpu_bands_async(m, cam, nullptr, &ga, film_rgb_full, OUT_GI_FILM);
+        return mgpu_bands_async(m, cam, nullptr, &ga, nullptr, film_rgb_full, OUT_GI_FILM);
 }
 
 int vrt_mgpu_gi_render(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_rgb_full)
 {
         int rc = vrt_mgpu_gi_render_async(m, cam, kd, res, film_rgb_full);
+        const int rs = vrt_mgpu_sync(m);
+        return rc ? rc : rs;
+}
+
+int vrt_mgpu_gi_render_aov_async(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res,
+                                 float* film_full_or_null, const vrt_gi_aov* aov_full)
+{
+        const int rc = check_gi_aov_request(kd, aov_full);
+        if (rc)
+                return rc;
+        const GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
+        return mgpu_bands_async(m, cam, nullptr, &ga, aov_full, film_full_or_null, OUT_GI_AOV);
+}
+
+int vrt_mgpu_gi_render_aov(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_full_or_null,
+                           const vrt_gi_aov* aov_full)
+{
+        int rc = vrt_mgpu_gi_render_aov_async(m, cam, kd, res, film_full_or_null, aov_full);
         const int rs = vrt_mgpu_sync(m);
         return rc ? rc : rs;
 }
