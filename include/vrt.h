@@ -322,7 +322,8 @@ uint64_t vrt_debug_general_order_calls(void);
  *      and cone_trace (voxel_octree.cc:190-303), the final trace() pixel (main.cc:10-30).
  *      One untextured material: kd = tinyobj material_t::diffuse (voxel_octree.cc:474-476).
  *      Per-node state (coverage, illum[6]) lives beside the node array; it belongs to one
- *      build: call vrt_gi_init again after vrt_rebuild. ------------------------------------ */
+ *      build: call vrt_gi_init again after vrt_rebuild, vrt_update_triangles(_dev) or
+ *      vrt_update_xform (and their vrt_mgpu_* forms). ------------------------------------- */
 /* Materials (Triangle::get_albedo, voxel_octree.cc:471-484): tri_uv[T][3][2] per-vertex texture
  * coordinates, tri_mtl[T] material ids, per material kd[m][3] (tinyobj material_t::diffuse) and
  * mtl_tex[m] = index into tex[] or -1 (empty diffuse_texname).  Textures are the bytes stbi_load
@@ -444,6 +445,55 @@ int vrt_mgpu_gi_render_aov(vrt_mgpu* m, const vrt_camera* cam, const float kd[3]
                            const vrt_gi_aov* aov_full);
 /* vrt_mean_kernel_ms of replica `index` (0 for a bad index): the per-device balance of a multi-GPU frame loop */
 double vrt_mgpu_mean_kernel_ms(vrt_mgpu* m, int index, int last_n);
+
+/* ---- animated geometry: new triangles for a built handle, then the build of vrt_rebuild at max_depth ----------
+ * Full update: vrt_update_triangles(_dev) replaces the handle's triangles (its REST pose) and rebuilds.  num_tris must
+ *   equal the handle's count (the per-triangle materials stay valid), tri_nrm must be given exactly when the handle
+ *   was built with normals, and the handle's VRT_BUILD_UNIT_NORMALS flag is kept.  The _dev form copies from the
+ *   caller's device arrays on the handle's stream; like every build both forms return when the build is done, so the
+ *   arrays may be reused at once.
+ * Transform update: vrt_update_xform sets the current pose to the rest pose with each range moved by its transform,
+ *     p' = M[:, :3] p + M[:, 3]   for the three vertices   (m: row-major 3x4)
+ *     n' = N n                    for the three normals    (n: row-major 3x3, normally the inverse transpose of
+ *                                                           M[:, :3]; ignored when the handle has no normals)
+ *   each coordinate evaluated as ((m0*x + m1*y) + m2*z) + m3 in float32 without fused multiply-add (and the same
+ *   for n), and rebuilds.  Triangles outside every range keep their rest pose.  Ranges are non-empty, lie inside
+ *   [0, num_tris) and do not overlap; transforms are absolute (the same table twice gives the same tree).  The rest
+ *   pose is the triangles of the last build or full update; vrt_rebuild after a transform update rebuilds the
+ *   current pose.
+ * After either call the handle is bytewise the one vrt_build_ex with the same flags makes from the current pose (the
+ * blob up to its size, vrt_tree_export, vrt_tree_get_info but build_ms and device_bytes).  Materials, film format,
+ * stream and the pipelined-frame state are kept; the GI state is dropped as after every build (vrt_gi_init again).
+ * Each update runs after every frame already enqueued on the handle (both kernel streams of the pipelined loops)
+ * and before every frame enqueued later, as the GI writers do: frames enqueued before it render the old geometry,
+ * frames after it the new, with no vrt_tree_sync in between.
+ * Errors: VRT_ERR_ARG for a NULL handle or array, a wrong count, normals given or missing against the handle,
+ * max_depth out of range, num_xf == 0, an empty, out-of-range or overlapping range, and a non-finite m or n entry;
+ * VRT_ERR_STATE for a handle without input triangles (vrt_tree_load, vrt_tree_from_blob_dev) or on another
+ * device.  A rejected call changes nothing and enqueues nothing.  A build failure (VRT_ERR_NOMEM, VRT_ERR_CAPACITY)
+ * leaves what a failed vrt_rebuild leaves: the new pose is the handle's input and vrt_rebuild builds it, while the
+ * octree is whatever the failed build left (the previous blob when it failed before assembly, none when the blob
+ * could not be allocated: then every other call returns VRT_ERR_STATE); render nothing from it before a
+ * successful update or vrt_rebuild. */
+typedef struct vrt_xform {
+        uint32_t first_tri, num_tris;
+        float m[12]; /* row-major 3x4 */
+        float n[9];  /* row-major 3x3 */
+} vrt_xform;
+int vrt_update_triangles(vrt_tree* tree, const float* tri_xyz, const float* tri_nrm, uint32_t num_tris,
+                         int max_depth);
+int vrt_update_triangles_dev(vrt_tree* tree, const float* d_tri_xyz, const float* d_tri_nrm, uint32_t num_tris,
+                             int max_depth);
+int vrt_update_xform(vrt_tree* tree, const vrt_xform* xf, uint32_t num_xf, int max_depth);
+/* The same on the replicas of a vrt_mgpu: the first replica rebuilds, every other one then takes a copy of its blob
+ * after its own enqueued frames, so every replica is bytewise the fresh build.  vrt_mgpu_create copies the source
+ * tree's input triangles (about 72 bytes per triangle) as the rest pose; a replica set made from a tree without
+ * them returns VRT_ERR_STATE from vrt_mgpu_update_xform until vrt_mgpu_update_triangles has given it triangles
+ * (with or without normals; without VRT_BUILD_UNIT_NORMALS).  Host pointers.  On a failure the other replicas keep
+ * their previous octree. */
+int vrt_mgpu_update_triangles(vrt_mgpu* m, const float* tri_xyz, const float* tri_nrm, uint32_t num_tris,
+                              int max_depth);
+int vrt_mgpu_update_xform(vrt_mgpu* m, const vrt_xform* xf, uint32_t num_xf, int max_depth);
 
 /* out = {node expansions cross-checked against the slab expansion, mismatches}; counts only in
  * a library built with -DVRT_PARAM_CHECK (tests), {0,0} otherwise. */

@@ -48,6 +48,11 @@ class vrt_gi_aov(C.Structure):
 GI_AOV_PLANES = ("albedo", "direct", "indirect", "normal", "hits")
 
 
+class vrt_xform(C.Structure):
+    """One range of vrt_update_xform: p' = M[:, :3] p + M[:, 3], n' = N n for triangles [first_tri, +num_tris)."""
+    _fields_ = [("first_tri", C.c_uint32), ("num_tris", C.c_uint32), ("m", C.c_float * 12), ("n", C.c_float * 9)]
+
+
 class vrt_tree_info(C.Structure):
     _fields_ = [("num_tris", C.c_uint32), ("max_depth", C.c_int32), ("root_aabb", C.c_float * 6),
                 ("num_nodes", C.c_uint64), ("num_leaves", C.c_uint64), ("num_refs", C.c_uint64),
@@ -85,6 +90,8 @@ SYMBOLS = [
     "vrt_mgpu_gi_filter", "vrt_mgpu_gi_render_async", "vrt_mgpu_gi_render", "vrt_mgpu_mean_kernel_ms",
     "vrt_gi_render_aov", "vrt_gi_render_aov_dev",
     "vrt_gi_render_aov_bands_async", "vrt_mgpu_gi_render_aov_async", "vrt_mgpu_gi_render_aov",
+    "vrt_update_triangles", "vrt_update_triangles_dev", "vrt_update_xform", "vrt_mgpu_update_triangles",
+    "vrt_mgpu_update_xform",
 ]
 
 _lib = None
@@ -193,6 +200,11 @@ def load(build_if_missing: bool = True):
     L.vrt_mgpu_mean_kernel_ms.restype = C.c_double
     L.vrt_mgpu_mean_kernel_ms.argtypes = [vp, i32, i32]
     L.vrt_tree_sync.argtypes = [vp]
+    L.vrt_update_triangles.argtypes = [vp, vp, vp, u32, i32]
+    L.vrt_update_triangles_dev.argtypes = [vp, vp, vp, u32, i32]
+    L.vrt_update_xform.argtypes = [vp, vp, u32, i32]
+    L.vrt_mgpu_update_triangles.argtypes = [vp, vp, vp, u32, i32]
+    L.vrt_mgpu_update_xform.argtypes = [vp, vp, u32, i32]
     L.vrt_mean_kernel_ms.restype = C.c_double
     L.vrt_mean_kernel_ms.argtypes = [vp, i32]
     L.vrt_last_kernel_ms.restype = C.c_double
@@ -340,6 +352,34 @@ class Octree:
 
     def rebuild(self, max_depth):
         _check(load().vrt_rebuild(self._h, int(max_depth)))
+
+    # ---- animated geometry (include/vrt.h vrt_update_*) ------------------------------------------------------------
+    def _update_args(self, num_tris, max_depth):
+        """max_depth None -> the handle's current depth; a triangle count other than the handle's raises."""
+        i = self.info()
+        if num_tris is not None and num_tris != i["num_tris"]:
+            raise ValueError(f"update needs {i['num_tris']} triangles (the handle's count), got {num_tris}")
+        return i["max_depth"] if max_depth is None else int(max_depth)
+
+    def update(self, tri_xyz, tri_nrm=None, max_depth=None):
+        """Replace the handle's triangles (same count; normals exactly when it was built with them) and rebuild at
+        max_depth (None: the current depth).  Materials and film format stay; call gi_init again."""
+        tri, nrm = _update_arrays(tri_xyz, tri_nrm)
+        depth = self._update_args(tri.shape[0], max_depth)
+        _check(load().vrt_update_triangles(self._h, _ptr(tri), _ptr(nrm), tri.shape[0], depth))
+
+    def update_dev(self, d_tri_ptr, d_nrm_ptr, num_tris, max_depth=None):
+        """update() from device arrays [num_tris, 9] float32 (d_nrm_ptr 0 / None: no normals)."""
+        depth = self._update_args(int(num_tris), max_depth)
+        _check(load().vrt_update_triangles_dev(self._h, C.c_void_p(int(d_tri_ptr or 0) or None),
+                                               C.c_void_p(int(d_nrm_ptr or 0) or None), int(num_tris), depth))
+
+    def update_xform(self, xforms, max_depth=None):
+        """Set the pose to the rest pose (the triangles of the last build or update()) with ranges moved: xforms is a
+        list of (first, count, M 3x4[, N 3x3]); N defaults to the float64 inverse transpose of M[:, :3]."""
+        arr = _xform_table(xforms)
+        depth = self._update_args(None, max_depth)
+        _check(load().vrt_update_xform(self._h, C.cast(arr, C.c_void_p), len(arr), depth))
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
@@ -637,6 +677,8 @@ class MultiGpu:
         h = C.c_void_p()
         _check(load().vrt_mgpu_create(tree._h, len(dv), _ptr(dv), C.byref(h)))
         self._h = h
+        i = tree.info()
+        self.max_depth, self.num_tris = i["max_depth"], i["num_tris"]
 
     @property
     def num_devices(self):
@@ -698,6 +740,23 @@ class MultiGpu:
         _check(load().vrt_mgpu_gi_render_aov(self._h, C.byref(cam.c), _ptr(kd), float(np.float32(res)),
                                              C.c_void_p(int(host_film_ptr_or_0) or None), C.byref(aov)))
 
+    def update(self, tri_xyz, tri_nrm=None, max_depth=None):
+        """Octree.update on the replicas: the first one rebuilds, the others copy its blob (max_depth None: the
+        replicas' current depth)."""
+        tri, nrm = _update_arrays(tri_xyz, tri_nrm)
+        if tri.shape[0] != self.num_tris:
+            raise ValueError(f"update needs {self.num_tris} triangles (the replicas' count), got {tri.shape[0]}")
+        depth = self.max_depth if max_depth is None else int(max_depth)
+        _check(load().vrt_mgpu_update_triangles(self._h, _ptr(tri), _ptr(nrm), tri.shape[0], depth))
+        self.max_depth = depth
+
+    def update_xform(self, xforms, max_depth=None):
+        """Octree.update_xform on the replicas (rest pose: the source tree's triangles, or the last update())."""
+        arr = _xform_table(xforms)
+        depth = self.max_depth if max_depth is None else int(max_depth)
+        _check(load().vrt_mgpu_update_xform(self._h, C.cast(arr, C.c_void_p), len(arr), depth))
+        self.max_depth = depth
+
     def mean_kernel_ms(self, index, last_n):
         """Mean device time of the last `last_n` kernels of replica `index` (waits for them)."""
         return float(load().vrt_mgpu_mean_kernel_ms(self._h, int(index), int(last_n)))
@@ -706,6 +765,47 @@ class MultiGpu:
         if self._h:
             load().vrt_mgpu_free(self._h)
             self._h = None
+
+
+def _update_arrays(tri_xyz, tri_nrm):
+    """float32 [T, 9] triangles (and normals of the same shape) for the update calls; shape errors raise here."""
+    tri = np.ascontiguousarray(tri_xyz, np.float32)
+    if tri.size % 9 or tri.size == 0:
+        raise ValueError(f"tri_xyz must hold [T, 9] floats, got shape {tri.shape}")
+    tri = tri.reshape(-1, 9)
+    if tri_nrm is None:
+        return tri, None
+    nrm = np.ascontiguousarray(tri_nrm, np.float32)
+    if nrm.size != tri.size:
+        raise ValueError(f"tri_nrm must have the shape of tri_xyz {tri.shape}, got {nrm.shape}")
+    return tri, nrm.reshape(-1, 9)
+
+
+def xform_normal_matrix(m):
+    """The default normal matrix of a 3x4 transform: the float64 inverse transpose of M[:, :3], as float32."""
+    return np.linalg.inv(np.asarray(m, np.float64).reshape(3, 4)[:, :3]).T.astype(np.float32)
+
+
+def _xform_table(xforms):
+    """vrt_xform array from (first, count, M 3x4[, N 3x3]) tuples; malformed tuples raise ValueError."""
+    xforms = list(xforms)
+    if not xforms:
+        raise ValueError("update_xform needs at least one transform")
+    arr = (vrt_xform * len(xforms))()
+    for k, x in enumerate(xforms):
+        if not isinstance(x, (tuple, list)) or len(x) not in (3, 4):
+            raise ValueError(f"transform {k}: expected (first, count, M[, N]), got {x!r}")
+        first, count = int(x[0]), int(x[1])
+        if first < 0 or count < 0 or first >= 2 ** 32 or count >= 2 ** 32:
+            raise ValueError(f"transform {k}: bad range ({first}, {count})")
+        m = np.asarray(x[2], np.float32)
+        if m.shape != (3, 4):
+            raise ValueError(f"transform {k}: M must be 3x4, got shape {m.shape}")
+        n = np.asarray(x[3], np.float32) if len(x) == 4 and x[3] is not None else xform_normal_matrix(x[2])
+        if n.shape != (3, 3):
+            raise ValueError(f"transform {k}: N must be 3x3, got shape {n.shape}")
+        arr[k] = vrt_xform(first, count, (C.c_float * 12)(*m.reshape(-1)), (C.c_float * 9)(*n.reshape(-1)))
+    return arr
 
 
 def _gi_aov(planes: dict) -> vrt_gi_aov:

@@ -9,6 +9,9 @@
 // as well, the same film rendered through gi::MultiGpu on those devices goes to <file>.mgpu; with --gi-aov <prefix> as
 // well, what that film is made of goes to <prefix>.{albedo,direct,indirect,normal}.hdr (and, with --gi-devices, the
 // same planes rendered through the replicas to <prefix>.mgpu.{albedo,direct,indirect,normal}.hdr).
+// With --animate <prefix> it renders four GI frames, the scene turned by one more quarter turn about the vertical
+// axis through the centre of its root box before each (gi::transform_gpu, then the light map and filter again), and
+// writes frame k to <prefix>.<k>.hdr.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -127,12 +130,14 @@ int main(int argc, char** argv)
         const char* gi_dump = nullptr;  // --gi <file>: also run main.cc's light map + filter + cone-traced film
         std::vector<int> gi_devices;    // --gi-devices 0,0,...: the GI film again on these replicas -> <file>.mgpu
         const char* gi_aov = nullptr;   // --gi-aov <prefix>: the GI film's planes -> <prefix>.<plane>.hdr
+        const char* animate = nullptr;  // --animate <prefix>: four GI frames of the turning scene -> <prefix>.<k>.hdr
         const char* obj = nullptr;
         int depth = 6, nx = 1024, ny = 1024, pos = 0;  // main.cc:34-35,67
         for (int i = 1; i < argc; ++i) {
                 if (!std::strcmp(argv[i], "--dump") && i + 1 < argc) { dump = argv[++i]; continue; }
                 if (!std::strcmp(argv[i], "--gi") && i + 1 < argc) { gi_dump = argv[++i]; continue; }
                 if (!std::strcmp(argv[i], "--gi-aov") && i + 1 < argc) { gi_aov = argv[++i]; continue; }
+                if (!std::strcmp(argv[i], "--animate") && i + 1 < argc) { animate = argv[++i]; continue; }
                 if (!std::strcmp(argv[i], "--gi-devices") && i + 1 < argc) {
                         for (const char* p = argv[++i]; *p;) {
                                 char* end = nullptr;
@@ -245,6 +250,47 @@ int main(int argc, char** argv)
                                         std::printf("GI planes on %zu replicas written\n", gi_devices.size());
                                 }
                         }
+                }
+                if (animate) {
+                        // a moving scene: per frame one transform update (the pose is absolute: a turn of (k+1)
+                        // quarters from the rest pose), the light map and filter again, the GI film
+                        const Vec3 kd{ 0.7f, 0.6f, 0.5f };
+                        Film sfilm(1.f, 1.f, nx, ny);
+                        Camera scam{ 60.f * 3.1415926535897932384626f / 180.f, { 1, 10, 1 }, { 0, 0, 0 }, { 0, 1, 0 } };
+                        const float cx = (root.aabb.min.x + root.aabb.max.x) * 0.5f;
+                        const float cz = (root.aabb.min.z + root.aabb.max.z) * 0.5f;
+                        const float cs[4][2] = { { 0, 1 }, { -1, 0 }, { 0, -1 }, { 1, 0 } };  // cos, sin of (k+1) * 90 deg
+                        for (int k = 0; k < 4; ++k) {
+                                const float c = cs[k][0], s = cs[k][1];
+                                // p' = R (p - centre) + centre about the y axis: R = [[c,0,s],[0,1,0],[-s,0,c]]
+                                vrt_xform xf{};
+                                xf.first_tri = 0;
+                                xf.num_tris = (uint32_t)voxels.size();
+                                const float m[12] = { c, 0, s, cx - (c * cx + s * cz), 0, 1, 0, 0, -s, 0, c, cz - (-s * cx + c * cz) };
+                                const float n[9] = { c, 0, s, 0, 1, 0, -s, 0, c };
+                                std::memcpy(xf.m, m, sizeof m);
+                                std::memcpy(xf.n, n, sizeof n);
+                                gi::transform_gpu(&root, { xf });
+                                light_map_gpu(sfilm, scam, &root, 4, kd);
+                                gi::cone_trace_init_filter(&root);
+                                float res = 3.4e38f;
+                                for (int a = 0; a < 3; ++a)
+                                        res = std::min(res, (root.aabb.max[a] - root.aabb.min[a]) / std::pow(2.f, (float)depth));
+                                Film afilm(1.f, 1.f, nx, ny);
+                                render_gi_gpu(&afilm, cam, &root, 4, kd, res);
+                                write_hdr((std::string(animate) + "." + std::to_string(k) + ".hdr").c_str(), afilm);
+                                // the per-ray mirror sees the new leaves: the centre ray's leaf and triangle
+                                gi::VoxelOctree* aleaf = nullptr;
+                                gi::VoxelBase* avox = nullptr;
+                                jql::ISect ais{};
+                                if (gi::ray_march(&root, rays[0], &aleaf, &avox, &ais))
+                                        std::printf("frame %d centre ray: leaf cell (%u,%u,%u) with %zu triangles, triangle %td\n", k,
+                                                    aleaf->cell[0], aleaf->cell[1], aleaf->cell[2], aleaf->voxels.size(),
+                                                    static_cast<gi::Triangle*>(avox) - voxels.data());
+                                else
+                                        std::printf("frame %d centre ray: miss\n", k);
+                        }
+                        std::printf("animation written\n");
                 }
                 std::printf("success.\n");
         } catch (const std::exception& e) {

@@ -141,6 +141,34 @@ bool Triangle::isect(const Ray& ray, ISect* isect) const
         return true;
 }
 
+static GpuTree* gpu_tree(VoxelOctree* root, const char* what)
+{
+        if (!root || !root->gpu)
+                throw std::runtime_error(std::string(what) + ": octree not initialised (call ray_march_init)");
+        return root->gpu.get();
+}
+
+// the root box, depth and exported leaf set of the handle's current octree; the leaves materialised from an earlier
+// one are dropped (after an update their cells and triangle lists no longer hold)
+static void load_leaf_set(VoxelOctree* root)
+{
+        GpuTree* g = root->gpu.get();
+        vrt_tree_info info;
+        check(vrt_tree_get_info(g->tree, &info), "vrt_tree_get_info");
+        root->aabb.min = Vec3{ info.root_aabb[0], info.root_aabb[1], info.root_aabb[2] };
+        root->aabb.max = Vec3{ info.root_aabb[3], info.root_aabb[4], info.root_aabb[5] };
+        std::lock_guard<std::mutex> lock(g->mu);
+        g->max_depth = info.max_depth;
+        g->leaf_cell.assign(3 * info.num_leaves, 0);
+        g->leaf_count.assign(info.num_leaves, 0);
+        g->leaf_refs.assign(info.num_refs, 0);
+        g->leaf_start.clear();
+        g->leaf_index.clear();
+        g->leaves.clear();
+        vrt_tree_view view{ g->leaf_cell.data(), g->leaf_count.data(), g->leaf_refs.data(), nullptr };
+        check(vrt_tree_export(g->tree, &view), "vrt_tree_export");
+}
+
 void ray_march_init(VoxelOctree* root, std::vector<VoxelBase*>& voxels, int max_depth)
 {
         auto g = std::make_shared<GpuTree>();
@@ -153,17 +181,44 @@ void ray_march_init(VoxelOctree* root, std::vector<VoxelBase*>& voxels, int max_
         }
         check(vrt_build_ex(tri.data(), nrm.data(), (uint32_t)voxels.size(), max_depth, VRT_BUILD_UNIT_NORMALS, &g->tree),
               "gi::ray_march_init");
-        vrt_tree_info info;
-        check(vrt_tree_get_info(g->tree, &info), "vrt_tree_get_info");
-        root->aabb.min = Vec3{ info.root_aabb[0], info.root_aabb[1], info.root_aabb[2] };
-        root->aabb.max = Vec3{ info.root_aabb[3], info.root_aabb[4], info.root_aabb[5] };
         root->depth = 1;
-        g->leaf_cell.resize(3 * info.num_leaves);
-        g->leaf_count.resize(info.num_leaves);
-        g->leaf_refs.resize(info.num_refs);
-        vrt_tree_view view{ g->leaf_cell.data(), g->leaf_count.data(), g->leaf_refs.data(), nullptr };
-        check(vrt_tree_export(g->tree, &view), "vrt_tree_export");
         root->gpu = std::move(g);
+        load_leaf_set(root);
+}
+
+void update_triangles_gpu(VoxelOctree* root, const std::vector<float>& tri_xyz, const std::vector<float>& tri_nrm,
+                          int max_depth)
+{
+        GpuTree* g = gpu_tree(root, "gi::update_triangles_gpu");
+        if (tri_xyz.size() != 9 * g->voxels.size() || (!tri_nrm.empty() && tri_nrm.size() != tri_xyz.size()))
+                throw std::runtime_error("gi::update_triangles_gpu: expected 9 floats per triangle of the octree");
+        check(vrt_update_triangles(g->tree, tri_xyz.data(), tri_nrm.empty() ? nullptr : tri_nrm.data(),
+                                   (uint32_t)g->voxels.size(), max_depth ? max_depth : g->max_depth),
+              "gi::update_triangles_gpu");
+        load_leaf_set(root);
+}
+
+void transform_gpu(VoxelOctree* root, const std::vector<vrt_xform>& xf, int max_depth)
+{
+        GpuTree* g = gpu_tree(root, "gi::transform_gpu");
+        check(vrt_update_xform(g->tree, xf.data(), (uint32_t)xf.size(), max_depth ? max_depth : g->max_depth),
+              "gi::transform_gpu");
+        load_leaf_set(root);
+}
+
+void update_triangles_gpu(MultiGpu& replicas, const std::vector<float>& tri_xyz, const std::vector<float>& tri_nrm,
+                          int max_depth)
+{
+        if (tri_xyz.empty() || tri_xyz.size() % 9 || (!tri_nrm.empty() && tri_nrm.size() != tri_xyz.size()))
+                throw std::runtime_error("gi::update_triangles_gpu: expected 9 floats per triangle");
+        check(vrt_mgpu_update_triangles(replicas.native(), tri_xyz.data(), tri_nrm.empty() ? nullptr : tri_nrm.data(),
+                                        (uint32_t)(tri_xyz.size() / 9), max_depth),
+              "gi::update_triangles_gpu");
+}
+
+void transform_gpu(MultiGpu& replicas, const std::vector<vrt_xform>& xf, int max_depth)
+{
+        check(vrt_mgpu_update_xform(replicas.native(), xf.data(), (uint32_t)xf.size(), max_depth), "gi::transform_gpu");
 }
 
 const vrt_tree* native_handle(const VoxelOctree* root)

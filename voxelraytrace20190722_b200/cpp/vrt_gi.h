@@ -127,6 +127,20 @@ private:
         vrt_mgpu* m_ = nullptr;
 };
 void cone_trace_init_filter(MultiGpu& replicas);
+
+// Animated geometry (vrt_update_triangles / vrt_update_xform): move the triangles of a built octree and revoxelise.
+// tri_xyz and tri_nrm hold 9 floats per triangle in the order of the voxels given to ray_march_init (tri_nrm: the
+// normals as Triangle stores them, or empty exactly when the octree has no input normals); xf ranges index that
+// order too.  The VoxelBase objects stay the caller's and are not changed.  max_depth 0: the current depth.  The
+// root box and the leaf set ray_march reads follow the new octree; leaf pointers from earlier calls are invalid.
+// The GI state is dropped: light the scene again (light_map_gpu, cone_trace_init_filter).
+void update_triangles_gpu(VoxelOctree* root, const std::vector<float>& tri_xyz, const std::vector<float>& tri_nrm,
+                          int max_depth = 0);
+void transform_gpu(VoxelOctree* root, const std::vector<vrt_xform>& xf, int max_depth = 0);
+// the same on the replicas (every replica ends up with the first one's octree); max_depth is required
+void update_triangles_gpu(MultiGpu& replicas, const std::vector<float>& tri_xyz, const std::vector<float>& tri_nrm,
+                          int max_depth);
+void transform_gpu(MultiGpu& replicas, const std::vector<vrt_xform>& xf, int max_depth);
 }  // namespace gi
 
 class Film {  // camera.h:24-39 -- storage is y*nx+x (the reference's y*ny+x is only right for nx==ny)

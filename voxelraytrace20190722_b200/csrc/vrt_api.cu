@@ -290,6 +290,60 @@ __global__ void k_gather_indexed(const float* __restrict__ vertices, const float
         }
 }
 
+// row r of a row-major 3x4 (w = 4, translation m[3]) or 3x3 (w = 3, no translation) matrix times p, as
+// ((m0*x + m1*y) + m2*z) [+ m3] with scalar __fmul_rn / __fadd_rn: these are never contracted, not even into the
+// packed FFMA2 that ptxas forms from -fmad=false multiply-add chains (vrt_trace.cu), so a float32 evaluation in this
+// order on the host reproduces every coordinate
+template <int W>
+__device__ __forceinline__ float xf_row(const float* __restrict__ m, float x, float y, float z)
+{
+        float s = __fadd_rn(__fadd_rn(__fmul_rn(m[0], x), __fmul_rn(m[1], y)), __fmul_rn(m[2], z));
+        if (W == 4)
+                s = __fadd_rn(s, m[3]);
+        return s;
+}
+
+// vrt_update_xform: the current pose of triangle i (what the build reads) from its rest pose -- moved by the
+// transform whose range holds i, copied when no range does.  xf is sorted by first_tri, its ranges disjoint and
+// non-empty (validated on the host), so the range of i is the last one starting at or before i.
+__global__ void k_apply_xforms(const float* __restrict__ rest_tri, const float* __restrict__ rest_nrm,
+                               const vrt_xform* __restrict__ xf, uint32_t num_xf, uint32_t T, float* __restrict__ tri,
+                               float* __restrict__ nrm)
+{
+        const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;  // one triangle
+        if (i >= T)
+                return;
+        uint32_t lo = 0, hi = num_xf;  // lo = number of ranges starting at or before i
+        while (lo < hi) {
+                const uint32_t mid = (lo + hi) >> 1;
+                if (xf[mid].first_tri <= i)
+                        lo = mid + 1;
+                else
+                        hi = mid;
+        }
+        const vrt_xform* x = (lo && i - xf[lo - 1].first_tri < xf[lo - 1].num_tris) ? &xf[lo - 1] : nullptr;
+        const float* p = rest_tri + 9ull * i;
+        float* q = tri + 9ull * i;
+#pragma unroll
+        for (int v = 0; v < 3; ++v) {
+                const float px = p[3 * v], py = p[3 * v + 1], pz = p[3 * v + 2];
+#pragma unroll
+                for (int r = 0; r < 3; ++r)
+                        q[3 * v + r] = x ? xf_row<4>(x->m + 4 * r, px, py, pz) : p[3 * v + r];
+        }
+        if (!nrm)
+                return;
+        p = rest_nrm + 9ull * i;
+        q = nrm + 9ull * i;
+#pragma unroll
+        for (int v = 0; v < 3; ++v) {
+                const float nx = p[3 * v], ny = p[3 * v + 1], nz = p[3 * v + 2];
+#pragma unroll
+                for (int r = 0; r < 3; ++r)
+                        q[3 * v + r] = x ? xf_row<3>(x->n + 3 * r, nx, ny, nz) : p[3 * v + r];
+        }
+}
+
 static int build_indexed_impl(const float* vertices, uint64_t num_vertices, const float* normals, uint64_t num_normals,
                               const int32_t* index3, uint32_t num_tris, int max_depth, vrt_tree** out)
 {
@@ -566,6 +620,11 @@ void vrt_tree_free(vrt_tree* t)
                 cudaFree(t->d_tri_in);
         if (t->d_nrm_in)
                 cudaFree(t->d_nrm_in);
+        if (t->d_tri_rest)
+                cudaFree(t->d_tri_rest);
+        if (t->d_nrm_rest)
+                cudaFree(t->d_nrm_rest);
+        t->xf_buf.release();
         t->keys_a.release();
         t->keys_b.release();
         t->tmp_a.release();
@@ -647,7 +706,9 @@ int vrt_tree_get_info(const vrt_tree* t, vrt_tree_info* out)
         out->num_refs = t->hdr.num_refs;
         memcpy(out->level_offset, t->hdr.level_offset, sizeof out->level_offset);
         out->device_bytes = t->blob_bytes + t->scratch_bytes() + (t->d_tri_in ? (uint64_t)t->hdr.num_tris * 36 : 0) +
-                            (t->d_nrm_in ? (uint64_t)t->hdr.num_tris * 36 : 0);
+                            (t->d_nrm_in ? (uint64_t)t->hdr.num_tris * 36 : 0) +
+                            (t->d_tri_rest ? (uint64_t)t->hdr.num_tris * 36 : 0) +
+                            (t->d_nrm_rest ? (uint64_t)t->hdr.num_tris * 36 : 0);
         out->build_ms = t->build_ms;
         return VRT_OK;
 }
@@ -1481,6 +1542,162 @@ int vrt_gi_render_aov_bands_async(const vrt_tree* t, const vrt_camera* cam, cons
         return bands_async_common(t, cam, nullptr, &ga, aov_full, b, film_full_or_null, OUT_GI_AOV);
 }
 
+// ---- animated geometry: new input triangles, then the build of vrt_rebuild ---------------------------------------
+// An update writes the pose the build reads (d_tri_in / d_nrm_in) on `stream` and runs build_tree, which rewrites the
+// blob, the hulls and tri64 in place.  Frames of the pipelined loops may still read them, on both kernel streams, so
+// the update runs between the GI writer pair: after every frame enqueued before it, before every frame after it.
+static int check_update(const vrt_tree* t, const char* fn, int max_depth)
+{
+        if (!t) {
+                set_error("%s: null tree handle", fn);
+                return VRT_ERR_ARG;
+        }
+        if (!t->d_tri_in) {
+                set_error("%s: handle holds no input triangles (loaded, or made from a blob)", fn);
+                return VRT_ERR_STATE;
+        }
+        int dev = -1;
+        if (cudaGetDevice(&dev) != cudaSuccess || dev != t->device) {
+                cudaGetLastError();
+                set_error("%s: tree lives on device %d but the current device is %d", fn, t->device, dev);
+                return VRT_ERR_STATE;
+        }
+        if (max_depth < 1 || max_depth > (int)VRT_MAX_DEPTH) {
+                set_error("%s: max_depth %d out of range [1,%u]", fn, max_depth, VRT_MAX_DEPTH);
+                return VRT_ERR_ARG;
+        }
+        return VRT_OK;
+}
+
+static int check_update_triangles(const vrt_tree* t, const char* fn, const float* tri, bool has_nrm, bool nrm_known,
+                                  uint32_t num_tris)
+{
+        if (num_tris != t->hdr.num_tris) {
+                set_error("%s: num_tris %u differs from the handle's %u", fn, num_tris, t->hdr.num_tris);
+                return VRT_ERR_ARG;
+        }
+        if (!tri) {
+                set_error("%s: null tri_xyz", fn);
+                return VRT_ERR_ARG;
+        }
+        if (nrm_known && has_nrm != (t->d_nrm_in != nullptr)) {
+                set_error("%s: tri_nrm must be given exactly when the handle was built with normals", fn);
+                return VRT_ERR_ARG;
+        }
+        return VRT_OK;
+}
+
+static int update_triangles(vrt_tree* t, const float* tri, const float* nrm, uint32_t num_tris, int max_depth,
+                            bool from_device, const char* fn)
+{
+        int rc = check_update(t, fn, max_depth);
+        if (!rc)
+                rc = check_update_triangles(t, fn, tri, nrm != nullptr, true, num_tris);
+        if (rc)
+                return rc;
+        const cudaMemcpyKind kind = from_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+        const size_t bytes = (size_t)num_tris * 36;
+        rc = gi_writer_begin(t);
+        if (!rc && bytes && !cuda_ok(cudaMemcpyAsync(t->d_tri_in, tri, bytes, kind, t->stream), "copy triangles"))
+                rc = VRT_ERR_CUDA;
+        if (!rc && bytes && nrm && !cuda_ok(cudaMemcpyAsync(t->d_nrm_in, nrm, bytes, kind, t->stream), "copy normals"))
+                rc = VRT_ERR_CUDA;
+        if (!rc) {
+                t->rest_valid = false;  // the new triangles are the rest pose of later transform updates
+                rc = build_tree(t, max_depth);  // (synchronises: the caller's arrays are free again on return)
+        }
+        return gi_writer_end(t, rc);
+}
+
+// the table sorted by first_tri; every range non-empty, inside [0, T), disjoint from the others; m and n finite
+static int sort_xforms(const vrt_xform* xf, uint32_t num_xf, uint32_t T, const char* fn, std::vector<vrt_xform>* out)
+{
+        if (!xf || num_xf == 0) {
+                set_error("%s: no transforms", fn);
+                return VRT_ERR_ARG;
+        }
+        out->assign(xf, xf + num_xf);
+        for (const vrt_xform& x : *out) {
+                for (float v : x.m)
+                        if (!std::isfinite(v)) {
+                                set_error("%s: non-finite matrix entry", fn);
+                                return VRT_ERR_ARG;
+                        }
+                for (float v : x.n)
+                        if (!std::isfinite(v)) {
+                                set_error("%s: non-finite normal matrix entry", fn);
+                                return VRT_ERR_ARG;
+                        }
+                if (x.num_tris == 0 || (uint64_t)x.first_tri + x.num_tris > T) {
+                        set_error("%s: range [%u, +%u) is empty or outside [0, %u)", fn, x.first_tri, x.num_tris, T);
+                        return VRT_ERR_ARG;
+                }
+        }
+        std::stable_sort(out->begin(), out->end(),
+                         [](const vrt_xform& a, const vrt_xform& b) { return a.first_tri < b.first_tri; });
+        for (size_t k = 1; k < out->size(); ++k)
+                if ((*out)[k].first_tri < (uint64_t)(*out)[k - 1].first_tri + (*out)[k - 1].num_tris) {
+                        set_error("%s: ranges starting at %u and %u overlap", fn, (*out)[k - 1].first_tri,
+                                  (*out)[k].first_tri);
+                        return VRT_ERR_ARG;
+                }
+        return VRT_OK;
+}
+
+// current pose = rest pose moved by the sorted table, on `stream`; the rest pose is saved from the current one first
+// when the inputs were last replaced by a build or a full update
+static int apply_xforms(vrt_tree* t, const std::vector<vrt_xform>& xf)
+{
+        const uint32_t T = t->hdr.num_tris;
+        const size_t bytes = (size_t)T * 36;
+        if ((!t->d_tri_rest && !cuda_ok(cudaMalloc(&t->d_tri_rest, bytes), "cudaMalloc(rest pose)")) ||
+            (t->d_nrm_in && !t->d_nrm_rest && !cuda_ok(cudaMalloc(&t->d_nrm_rest, bytes), "cudaMalloc(rest normals)")))
+                return VRT_ERR_NOMEM;
+        if (!t->rest_valid) {
+                VRT_CUDA(cudaMemcpyAsync(t->d_tri_rest, t->d_tri_in, bytes, cudaMemcpyDeviceToDevice, t->stream));
+                if (t->d_nrm_in)
+                        VRT_CUDA(cudaMemcpyAsync(t->d_nrm_rest, t->d_nrm_in, bytes, cudaMemcpyDeviceToDevice, t->stream));
+                t->rest_valid = true;
+        }
+        const size_t xb = xf.size() * sizeof(vrt_xform);
+        if (t->xf_buf.reserve(xb))
+                return VRT_ERR_NOMEM;
+        VRT_CUDA(cudaMemcpyAsync(t->xf_buf.p, xf.data(), xb, cudaMemcpyHostToDevice, t->stream));
+        k_apply_xforms<<<(T + 255u) / 256u, 256, 0, t->stream>>>(t->d_tri_rest, t->d_nrm_rest, t->xf_buf.as<vrt_xform>(),
+                                                                 (uint32_t)xf.size(), T, t->d_tri_in, t->d_nrm_in);
+        count_launch();
+        VRT_CUDA(cudaGetLastError());
+        return VRT_OK;
+}
+
+int vrt_update_triangles(vrt_tree* t, const float* tri_xyz, const float* tri_nrm, uint32_t num_tris, int max_depth)
+{
+        return update_triangles(t, tri_xyz, tri_nrm, num_tris, max_depth, false, "vrt_update_triangles");
+}
+
+int vrt_update_triangles_dev(vrt_tree* t, const float* d_tri_xyz, const float* d_tri_nrm, uint32_t num_tris,
+                             int max_depth)
+{
+        return update_triangles(t, d_tri_xyz, d_tri_nrm, num_tris, max_depth, true, "vrt_update_triangles_dev");
+}
+
+int vrt_update_xform(vrt_tree* t, const vrt_xform* xf, uint32_t num_xf, int max_depth)
+{
+        int rc = check_update(t, "vrt_update_xform", max_depth);
+        if (rc)
+                return rc;
+        std::vector<vrt_xform> sorted;
+        rc = sort_xforms(xf, num_xf, t->hdr.num_tris, "vrt_update_xform", &sorted);
+        if (rc)
+                return rc;
+        rc = gi_writer_begin(t);
+        if (!rc)
+                rc = apply_xforms(t, sorted);
+        if (!rc)
+                rc = build_tree(t, max_depth);
+        return gi_writer_end(t, rc);
+}
+
 // ---- single-process multi-GPU render (SURVEY.md 8e; replaces render_mt camera.h:41-68 over N devices) -------
 // A C / C++ host (main.cc) owns ONE process: vrt_mgpu_create replicates a built octree onto the given devices
 // (peer copies of the blob over NVLink), vrt_mgpu_render_async deals the film's 8-row bands round-robin to the
@@ -1525,6 +1742,21 @@ void vrt_mgpu_free(vrt_mgpu* m)
         }
         cudaSetDevice(cur);
         delete m;
+}
+
+// the input triangles of `src` (the pose its octree was built from) as the inputs of replica `rep`, whose device is
+// current: the rest pose of vrt_mgpu_update_xform, which rebuilds on the first replica
+static int copy_inputs(vrt_tree* rep, const vrt_tree* src)
+{
+        const size_t bytes = (size_t)std::max<uint32_t>(src->hdr.num_tris, 1) * 36;
+        if (!cuda_ok(cudaMalloc(&rep->d_tri_in, bytes), "cudaMalloc(tri)") ||
+            (src->d_nrm_in && !cuda_ok(cudaMalloc(&rep->d_nrm_in, bytes), "cudaMalloc(nrm)")))
+                return VRT_ERR_NOMEM;
+        VRT_CUDA(cudaMemcpyPeer(rep->d_tri_in, rep->device, src->d_tri_in, src->device, bytes));
+        if (src->d_nrm_in)
+                VRT_CUDA(cudaMemcpyPeer(rep->d_nrm_in, rep->device, src->d_nrm_in, src->device, bytes));
+        rep->unit_normals = src->unit_normals;
+        return VRT_OK;
 }
 
 int vrt_mgpu_create(const vrt_tree* tree, int num_devices, const int* devices, vrt_mgpu** out)
@@ -1579,8 +1811,12 @@ int vrt_mgpu_create(const vrt_tree* tree, int num_devices, const int* devices, v
                                 cudaFree(tmp);
                         }
                 }
+                if (!rc && i == 0 && tree->d_tri_in)
+                        rc = copy_inputs(rep, tree);
                 if (!rc)
                         m->trees.push_back(rep);
+                else
+                        vrt_tree_free(rep);
         }
         cudaSetDevice(src_dev);
         if (rc) {
@@ -1722,6 +1958,84 @@ int vrt_mgpu_gi_render_aov(vrt_mgpu* m, const vrt_camera* cam, const float kd[3]
         int rc = vrt_mgpu_gi_render_aov_async(m, cam, kd, res, film_full_or_null, aov_full);
         const int rs = vrt_mgpu_sync(m);
         return rc ? rc : rs;
+}
+
+// ---- animated geometry on the replicas: the first replica rebuilds (the build synchronises the host at every level,
+// so builds on the others would run one after another anyway), then every other replica takes a copy of its blob --
+// the path of vrt_mgpu_create: peer copy, bind, compute_hulls -- between its own GI writer pair.
+static int replica_take_blob(vrt_tree* t, const vrt_tree* src)
+{
+        const uint64_t b = src->hdr.bytes;
+        VRT_CUDA(cudaStreamSynchronize(t->stream));  // every frame that reads the old blob has finished
+        if (t->blob_bytes < b) {
+                cudaFree(t->blob);
+                t->blob = nullptr;
+                if (cudaMalloc(&t->blob, b) != cudaSuccess) {
+                        cudaGetLastError();
+                        set_error("cudaMalloc(%llu) for a replica's blob failed", (unsigned long long)b);
+                        return VRT_ERR_NOMEM;
+                }
+                t->blob_bytes = b;
+        }
+        VRT_CUDA(cudaMemcpyPeerAsync(t->blob, t->device, src->blob, src->device, b, t->stream));
+        VRT_CUDA(cudaStreamSynchronize(t->stream));
+        t->hdr = src->hdr;
+        tree_bind_views(t);
+        return compute_hulls(t);
+}
+
+static int mgpu_replicate(vrt_mgpu* m)
+{
+        const vrt_tree* src = m->trees[0];
+        return mgpu_each(m, [&](int i, vrt_tree* t) {
+                if (i == 0)
+                        return (int)VRT_OK;
+                int rc = gi_writer_begin(t);
+                if (!rc)
+                        rc = replica_take_blob(t, src);
+                return gi_writer_end(t, rc);
+        });
+}
+
+int vrt_mgpu_update_triangles(vrt_mgpu* m, const float* tri_xyz, const float* tri_nrm, uint32_t num_tris, int max_depth)
+{
+        const char* fn = "vrt_mgpu_update_triangles";
+        if (!m || m->trees.empty()) {
+                set_error("null multi-GPU handle");
+                return VRT_ERR_ARG;
+        }
+        vrt_tree* t0 = m->trees[0];
+        if (max_depth < 1 || max_depth > (int)VRT_MAX_DEPTH) {
+                set_error("%s: max_depth %d out of range [1,%u]", fn, max_depth, VRT_MAX_DEPTH);
+                return VRT_ERR_ARG;
+        }
+        // a replica set made from a tree without input triangles takes its first inputs here, normals or not
+        int rc = check_update_triangles(t0, fn, tri_xyz, tri_nrm != nullptr, t0->d_tri_in != nullptr, num_tris);
+        if (rc)
+                return rc;
+        rc = mgpu_each(m, [&](int i, vrt_tree* t) {
+                if (i)
+                        return (int)VRT_OK;
+                const size_t bytes = (size_t)std::max<uint32_t>(num_tris, 1) * 36;
+                if (!t->d_tri_in && (!cuda_ok(cudaMalloc(&t->d_tri_in, bytes), "cudaMalloc(tri)") ||
+                                     (tri_nrm && !cuda_ok(cudaMalloc(&t->d_nrm_in, bytes), "cudaMalloc(nrm)")))) {
+                        cudaFree(t->d_tri_in);
+                        t->d_tri_in = nullptr;
+                        return (int)VRT_ERR_NOMEM;
+                }
+                return update_triangles(t, tri_xyz, tri_nrm, num_tris, max_depth, false, fn);
+        });
+        return rc ? rc : mgpu_replicate(m);
+}
+
+int vrt_mgpu_update_xform(vrt_mgpu* m, const vrt_xform* xf, uint32_t num_xf, int max_depth)
+{
+        if (!m || m->trees.empty()) {
+                set_error("null multi-GPU handle");
+                return VRT_ERR_ARG;
+        }
+        const int rc = mgpu_each(m, [&](int i, vrt_tree* t) { return i ? (int)VRT_OK : vrt_update_xform(t, xf, num_xf, max_depth); });
+        return rc ? rc : mgpu_replicate(m);
 }
 
 double vrt_mgpu_mean_kernel_ms(vrt_mgpu* m, int index, int last_n)

@@ -1038,6 +1038,19 @@ static int assemble_blob(vrt_tree* t, int L, uint64_t n, const uint64_t* level_n
                 t->own_blob = true;
         }
         char* base = static_cast<char*>(t->blob);
+        // zero the header's tail and the alignment gaps between the sections: every byte up to h.bytes is then a
+        // function of the inputs alone, so a rebuild into a reused blob (vrt_rebuild, vrt_update_*) equals a fresh
+        // build byte for byte
+        const uint64_t gaps[][2] = { { sizeof h, h.off_nodes },
+                                     { h.off_nodes + h.num_nodes * 8, h.off_leaf_morton },
+                                     { h.off_leaf_morton + num_leaves * 8, h.off_leaf_refs },
+                                     { h.off_leaf_refs + n * 4, h.off_tri4 },
+                                     { h.off_tri4 + (uint64_t)T * 48, h.off_nrm },
+                                     { h.off_nrm + (uint64_t)T * 36, h.off_axis_tab },
+                                     { h.off_axis_tab + 3 * h.axis_tab_stride * 8, h.bytes } };
+        for (const auto& g : gaps)
+                if (g[1] > g[0])
+                        VRT_CUDA(cudaMemsetAsync(base + g[0], 0, g[1] - g[0], s));
         VRT_CUDA(cudaMemcpyAsync(h.root_aabb, d_root6, 24, cudaMemcpyDeviceToHost, s));
         uint2* nodes = reinterpret_cast<uint2*>(base + h.off_nodes);
         for (int l = 0; l < L; ++l) {

@@ -143,6 +143,12 @@ struct vrt_tree {
         float* d_tri_in = nullptr;  // [T][9] as given
         float* d_nrm_in = nullptr;  // [T][9] as given, or null
         bool unit_normals = false;  // VRT_BUILD_UNIT_NORMALS: d_nrm_in is stored verbatim
+        // rest pose of vrt_update_xform, allocated on its first call ([T][9] each; d_nrm_rest only with d_nrm_in);
+        // rest_valid false: the rest pose is d_tri_in / d_nrm_in themselves (after a build or a full update)
+        float* d_tri_rest = nullptr;
+        float* d_nrm_rest = nullptr;
+        bool rest_valid = false;
+        vrt::Scratch xf_buf;  // sorted transform table of the last vrt_update_xform
         // build scratch
         vrt::Scratch keys_a, keys_b, tmp_a, tmp_b, tmp_c, hist, refs_s, tab_s, level_morton[VRT_MAX_DEPTH + 1],
             level_first[VRT_MAX_DEPTH + 1], level_mask[VRT_MAX_DEPTH + 1];
