@@ -323,7 +323,14 @@ uint64_t vrt_debug_general_order_calls(void);
  *      One untextured material: kd = tinyobj material_t::diffuse (voxel_octree.cc:474-476).
  *      Per-node state (coverage, illum[6]) lives beside the node array; it belongs to one
  *      build: call vrt_gi_init again after vrt_rebuild, vrt_update_triangles(_dev) or
- *      vrt_update_xform (and their vrt_mgpu_* forms). ------------------------------------- */
+ *      vrt_update_xform (and their vrt_mgpu_* forms).
+ *      `res` (cone_trace's min_voxel_size) must be finite and >= FLT_MIN: every entry point
+ *      that takes it returns VRT_ERR_ARG otherwise, before it looks at its other arguments.
+ *      For a normal res every step of a cone grows its distance by at least 11.5 %, so the
+ *      march ends (in about 1,600 steps even for res = FLT_MIN and an infinite root box); for
+ *      0, a negative or a subnormal res the distance stops advancing and the march never ends.
+ *      main.cc's Res (min over axes of root size / 2^max_depth) is 0 for a planar scene: take
+ *      the minimum over the axes of non-zero size. ------------------------------------------ */
 /* Materials (Triangle::get_albedo, voxel_octree.cc:471-484): tri_uv[T][3][2] per-vertex texture
  * coordinates, tri_mtl[T] material ids, per material kd[m][3] (tinyobj material_t::diffuse) and
  * mtl_tex[m] = index into tex[] or -1 (empty diffuse_texname).  Textures are the bytes stbi_load

@@ -10,6 +10,7 @@ Only tests/, ``__graft_entry__.smoke()`` and bench.py's ``cpu_baseline`` /
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 import os
 import subprocess
@@ -107,12 +108,24 @@ class Port:
         L.orc_gi_dump_level.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]
         L.orc_gi_cone_trace.argtypes = [C.c_void_p, _f32p, _f32p, C.c_uint64, C.c_float, _f32p]
         L.orc_gi_render.argtypes = [C.c_void_p, _f32p, C.c_float, C.c_int, C.c_int, C.c_int, C.c_float, _f32p, _f32p]
+        L.orc_gi_set_exact_log2.argtypes = [C.c_int]
         # materials / textures (SURVEY.md 8f row 3)
         L.orc_set_materials.argtypes = [C.c_void_p, _f32p, _u32p, C.c_uint32, _f32p, C.c_void_p, C.c_uint32, C.c_void_p,
                                         C.c_void_p]
         L.orc_film_rgb8.argtypes = [_f32p, C.c_uint64, _u8p]
         L.orc_film_rgbe.argtypes = [_f32p, C.c_uint64, _u8p]
         L.orc_albedo.argtypes = [C.c_void_p, _u32p, _f32p, C.c_uint64, _f32p, _f32p]
+
+    @contextlib.contextmanager
+    def exact_log2(self):
+        """Within the block the cone trace (gi_cone_trace, gi_render) takes split_level = int(log2f(x)) with the
+        correctly rounded log2f, (float)log2((double)x), instead of libm's -- the definition the device evaluates,
+        so GPU results compare bit for bit.  Outside it the oracle keeps the reference's libm expression."""
+        self.lib.orc_gi_set_exact_log2(1)
+        try:
+            yield self
+        finally:
+            self.lib.orc_gi_set_exact_log2(0)
 
     # -- film export ----------------------------------------------------------
     def film_rgb8(self, film):

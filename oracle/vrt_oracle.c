@@ -1041,6 +1041,12 @@ static uint64_t g_cone_counts[3];
 void orc_gi_counters_reset(void) { memset(g_cone_counts, 0, sizeof g_cone_counts); }
 void orc_gi_counters(uint64_t out[3]) { memcpy(out, g_cone_counts, sizeof g_cone_counts); }
 
+/* split_level = (int)log2f(x) with libm's log2f (the reference's own expression; default), or -- exact mode -- with
+ * the correctly rounded log2f, (float)log2((double)x): the definition the device evaluates in closed form
+ * (vrt_gi.cuh gi_split_level), so that the GPU's cone trace can be compared bit for bit. */
+static int g_exact_log2;
+void orc_gi_set_exact_log2(int on) { g_exact_log2 = on != 0; }
+
 static void orc_cone_trace_one(const orc_tree* t, const float o[3], const float d[3], float min_voxel_size,
                                float out[3])
 {
@@ -1057,7 +1063,8 @@ static void orc_cone_trace_one(const orc_tree* t, const float o[3], const float 
                 float diam = std_maxf(mindist, aperture * 2.f * dist);
                 if (maxdist < diam)
                         break;
-                int split_level = (int)log2f(maxdist / diam);
+                const float ratio = maxdist / diam;
+                int split_level = g_exact_log2 ? (int)(float)log2((double)ratio) : (int)log2f(ratio);
                 const orc_node* tree = root;
                 g_cone_counts[0]++;
                 while (tree->child[0] >= 0 && split_level) {

@@ -109,6 +109,44 @@ def gi_res(root_aabb, max_depth):
     return np.float32(((root[3:] - root[:3]) / np.float32(2.0 ** max_depth)).min())
 
 
+def gi_maxdist(root_aabb):
+    """cone_trace's maxdist = length(root.aabb.size()), float32 with jql::dot's order (voxel_octree.cc:250)."""
+    root = np.asarray(root_aabb, np.float32)
+    s = (root[3:] - root[:3]).astype(np.float32)
+    d = np.float32(0)
+    for k in range(3):
+        d = np.float32(d + np.float32(s[k] * s[k]))
+    return np.sqrt(d, dtype=np.float32)
+
+
+def gi_march(maxdist, res, limit=100000):
+    """The march of cone_trace (voxel_octree.cc:252-281) in float32: the level int(log2f(maxdist / diam)) sampled at
+    each step (log2f correctly rounded; None where the ratio is not a positive float), and whether the march ends --
+    False when dist stops advancing (0, negative or subnormal res) or `limit` steps pass.  It depends on res and the
+    root box only, not on the cone."""
+    f32 = np.float32
+    with np.errstate(over="ignore", invalid="ignore", divide="ignore"):
+        maxdist, res = f32(maxdist), f32(res)
+        mindist = f32(f32(1.414) * res)
+        ap2 = f32(f32(0.577350269) * f32(2))
+        dist = mindist
+        levels = []
+        while dist < maxdist:
+            a = f32(ap2 * dist)
+            diam = a if mindist < a else mindist
+            if maxdist < diam:
+                break
+            if len(levels) == limit:
+                return levels, False
+            q = f32(maxdist / diam)
+            levels.append(int(f32(np.log2(np.float64(q)))) if 0 < q < np.inf else None)
+            nxt = f32(dist + f32(f32(0.1) * diam))
+            if not nxt > dist:
+                return levels, False
+            dist = nxt
+    return levels, True
+
+
 GI_KD = np.array([0.7, 0.6, 0.5], np.float32)  # the scene's single untextured material (material_t::diffuse)
 
 

@@ -4,9 +4,10 @@ indirect light, the ISect normal and the 16-byte hit records, from the film's ow
 The planes are pinned three ways: the film is bytewise the film of gi_render (so nothing else changed), every term is
 bit-exact against the point entry points of the library evaluated on trace_camera's hits (albedo, gi_cone_trace,
 the hit normal, and compute_illum of the hit leaf's light-map row) accumulated like the film, and the terms agree
-with the oracle's restatement of main.cc's trace() loop (the indirect term up to the log2f caveat of
-test_gpu_gi.py).  The oracle side is the loop of the oracle's orc_gi_render built from the oracle's own ray march,
-albedo, cone trace and light-map rows, with VoxelOctree::compute_illum restated below in float32."""
+bit for bit with the oracle's restatement of main.cc's trace() loop (the indirect term with the oracle's correctly
+rounded log2f, Port.exact_log2, as in test_gpu_gi.py).  The oracle side is the loop of the oracle's orc_gi_render
+built from the oracle's own ray march, albedo, cone trace and light-map rows, with VoxelOctree::compute_illum
+restated below in float32."""
 import os
 import subprocess
 
@@ -14,7 +15,7 @@ import numpy as np
 import pytest
 
 from tests.common import CAM_LIGHT, CAM_MAIN, CAM_SPHERE, GI_KD, assert_bits_equal, gi_res
-from tests.test_gpu_gi import _lit, mostly_bits_equal
+from tests.test_gpu_gi import _lit
 from tests.test_gpu_gi_mgpu import _write_obj
 from voxelraytrace20190722_b200 import scenes
 
@@ -196,10 +197,10 @@ def test_gi_planes_exact(gpu, port, lit, name, spp):
         assert_bits_equal(pl[n].reshape(-1, 3), _accumulate(terms[n], spp), f"{name} {n} vs point entry points")
     assert pl["indirect"].max() > 0 and pl["direct"].max() > 0
     # 4. against the oracle's trace() loop
-    ref = _oracle_planes(port, orc, depth, cam10, NX, NY, spp, res)
-    for n in ("albedo", "normal", "direct"):
+    with port.exact_log2():
+        ref = _oracle_planes(port, orc, depth, cam10, NX, NY, spp, res)
+    for n in FLOAT_PLANES:
         assert_bits_equal(pl[n], ref[n], f"{name} {n} vs oracle")
-    mostly_bits_equal(pl["indirect"].reshape(-1, 3), ref["indirect"].reshape(-1, 3), f"{name} indirect vs oracle")
     # 5. one sample per pixel: the film is albedo * (indirect + direct) on hits, the sky elsewhere
     if spp == 1:
         hit = h16["hit"].reshape(NY, NX).astype(bool)

@@ -70,6 +70,11 @@ def test_gi_golden(port):
     assert_bits_equal(tree.gi_cone_trace(z["cone_pos"], z["cone_nrm"], res), z["cone"], "cone_trace")
     nx, ny, spp = (int(v) for v in z["dims"])
     assert_bits_equal(tree.gi_render(z["cam10"], 1.0, nx, ny, spp, res, z["kd"]), z["film"], "trace() film")
+    # the correctly rounded log2f of the device (Port.exact_log2) takes the same split levels on these vectors
+    with port.exact_log2():
+        assert_bits_equal(tree.gi_cone_trace(z["cone_pos"], z["cone_nrm"], res), z["cone"], "exact-mode cone_trace")
+        assert_bits_equal(tree.gi_render(z["cam10"], 1.0, nx, ny, spp, res, z["kd"]), z["film"],
+                          "exact-mode trace() film")
 
 
 def test_textured_golden(port):

@@ -196,9 +196,12 @@ int main(int argc, char** argv)
                         std::printf("filtering...\n");
                         gi::cone_trace_init_filter(&root);
                         std::printf("cone tracing...\n");
+                        // main.cc's Res over the axes of non-zero size: a planar scene's Res would be 0, which the GI
+                        // entry points refuse (the cone march would not advance)
                         float res = 3.4e38f;
                         for (int k = 0; k < 3; ++k)
-                                res = std::min(res, (root.aabb.max[k] - root.aabb.min[k]) / std::pow(2.f, (float)depth));
+                                if (root.aabb.max[k] > root.aabb.min[k])
+                                        res = std::min(res, (root.aabb.max[k] - root.aabb.min[k]) / std::pow(2.f, (float)depth));
                         Film gfilm(1.f, 1.f, nx, ny);
                         render_gi_gpu(&gfilm, cam, &root, 4, kd, res);
                         if (hit) {
@@ -275,7 +278,9 @@ int main(int argc, char** argv)
                                 gi::cone_trace_init_filter(&root);
                                 float res = 3.4e38f;
                                 for (int a = 0; a < 3; ++a)
-                                        res = std::min(res, (root.aabb.max[a] - root.aabb.min[a]) / std::pow(2.f, (float)depth));
+                                        if (root.aabb.max[a] > root.aabb.min[a])
+                                                res = std::min(res, (root.aabb.max[a] - root.aabb.min[a]) /
+                                                                            std::pow(2.f, (float)depth));
                                 Film afilm(1.f, 1.f, nx, ny);
                                 render_gi_gpu(&afilm, cam, &root, 4, kd, res);
                                 write_hdr((std::string(animate) + "." + std::to_string(k) + ".hdr").c_str(), afilm);

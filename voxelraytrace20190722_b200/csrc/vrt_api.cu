@@ -539,6 +539,22 @@ static int check_camera(const vrt_camera* cam, int x0, int y0, int x1, int y1)
         return VRT_OK;
 }
 
+// cone_trace's min_voxel_size.  The march advances by 0.1 * max(1.414 res, 1.1547 dist): for a normal res every step
+// grows dist by at least 11.5 % and the march ends (1,608 steps at res = FLT_MIN even for an infinite root box); for
+// 0, a negative or a subnormal res the increment rounds away and every cone would loop forever on the device.  NaN
+// and +-inf would end at once (zeros) but are never meant.  The first check of every entry point that takes res, so
+// a rejected call has touched neither the handle nor any stream.
+static int check_gi_res(float res)
+{
+        if (!(res >= FLT_MIN) || !(res <= FLT_MAX)) {
+                set_error("res %g outside [FLT_MIN, FLT_MAX]: the cone march ends only for a finite res >= FLT_MIN "
+                          "(main.cc's Res is 0 for a planar scene: take it from the axes of non-zero size)",
+                          (double)res);
+                return VRT_ERR_ARG;
+        }
+        return VRT_OK;
+}
+
 }  // namespace vrt
 
 using namespace vrt;
@@ -1509,6 +1525,8 @@ int vrt_render_bands_async(const vrt_tree* t, const vrt_camera* cam, const vrt_s
 int vrt_gi_render_bands_async(const vrt_tree* t, const vrt_camera* cam, const float kd[3], float res,
                               const vrt_bands* b, float* film_rgb_full)
 {
+        if (const int rc = check_gi_res(res))
+                return rc;
         if (!kd) {
                 set_error("null argument");
                 return VRT_ERR_ARG;
@@ -1535,6 +1553,8 @@ static int check_gi_aov_request(const float kd[3], const vrt_gi_aov* aov)
 int vrt_gi_render_aov_bands_async(const vrt_tree* t, const vrt_camera* cam, const float kd[3], float res,
                                   const vrt_bands* b, float* film_full_or_null, const vrt_gi_aov* aov_full)
 {
+        if (const int rc = check_gi_res(res))
+                return rc;
         const int rc = check_gi_aov_request(kd, aov_full);
         if (rc)
                 return rc;
@@ -1927,6 +1947,8 @@ int vrt_mgpu_gi_filter(vrt_mgpu* m)
 
 int vrt_mgpu_gi_render_async(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_rgb_full)
 {
+        if (const int rc = check_gi_res(res))
+                return rc;
         if (!kd) {
                 set_error("null argument");
                 return VRT_ERR_ARG;
@@ -1937,6 +1959,8 @@ int vrt_mgpu_gi_render_async(vrt_mgpu* m, const vrt_camera* cam, const float kd[
 
 int vrt_mgpu_gi_render(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_rgb_full)
 {
+        if (const int rc = check_gi_res(res))
+                return rc;
         int rc = vrt_mgpu_gi_render_async(m, cam, kd, res, film_rgb_full);
         const int rs = vrt_mgpu_sync(m);
         return rc ? rc : rs;
@@ -1945,6 +1969,8 @@ int vrt_mgpu_gi_render(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], fl
 int vrt_mgpu_gi_render_aov_async(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res,
                                  float* film_full_or_null, const vrt_gi_aov* aov_full)
 {
+        if (const int rc = check_gi_res(res))
+                return rc;
         const int rc = check_gi_aov_request(kd, aov_full);
         if (rc)
                 return rc;
@@ -1955,6 +1981,8 @@ int vrt_mgpu_gi_render_aov_async(vrt_mgpu* m, const vrt_camera* cam, const float
 int vrt_mgpu_gi_render_aov(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_full_or_null,
                            const vrt_gi_aov* aov_full)
 {
+        if (const int rc = check_gi_res(res))
+                return rc;
         int rc = vrt_mgpu_gi_render_aov_async(m, cam, kd, res, film_full_or_null, aov_full);
         const int rs = vrt_mgpu_sync(m);
         return rc ? rc : rs;
@@ -2137,6 +2165,8 @@ int vrt_gi_get_level(const vrt_tree* t, int level, float* coverage, float* illum
 
 int vrt_gi_cone_trace(const vrt_tree* tc, const float* pos, const float* nrm, uint64_t n, float res, float* out_rgb)
 {
+        if (const int rc = check_gi_res(res))
+                return rc;
         int rc = check_tree(tc);
         if (rc)
                 return rc;
@@ -2276,6 +2306,8 @@ int vrt_albedo(const vrt_tree* tc, const uint32_t* tri, const float* pos, uint64
 static int gi_render_common(const vrt_tree* tc, const vrt_camera* cam, const float kd[3], float res, int x0, int y0,
                             int x1, int y1, float* film, bool dev)
 {
+        if (const int rc = check_gi_res(res))
+                return rc;
         int rc = check_tree(tc);
         if (rc)
                 return rc;
@@ -2310,6 +2342,8 @@ int vrt_gi_render_camera_dev(const vrt_tree* t, const vrt_camera* cam, const flo
 static int gi_render_aov_common(const vrt_tree* tc, const vrt_camera* cam, const float kd[3], float res, int x0,
                                 int y0, int x1, int y1, float* film, const vrt_gi_aov* aov, bool dev)
 {
+        if (const int rc = check_gi_res(res))
+                return rc;
         int rc = check_tree(tc);
         if (rc)
                 return rc;
