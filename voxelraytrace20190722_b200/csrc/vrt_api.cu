@@ -1078,36 +1078,6 @@ int vrt_trace_rays(const vrt_tree* tc, const vrt_ray* rays, uint64_t n, vrt_hit*
         return VRT_OK;
 }
 
-static int trace_camera_common(const vrt_tree* tc, const vrt_camera* cam, const vrt_shade* sh, int x0, int y0, int x1,
-                               int y1, void* out, OutMode mode, bool dev, const GiArgs* gi = nullptr)
-{
-        int rc = check_tree(tc);
-        if (rc)
-                return rc;
-        rc = check_camera(cam, x0, y0, x1, y1);
-        if (rc)
-                return rc;
-        const uint64_t npix = (uint64_t)(x1 - x0) * (y1 - y0);
-        if (!npix)
-                return VRT_OK;
-        if (!out || (mode == OUT_FILM && !sh)) {
-                set_error("null out/shade pointer");
-                return VRT_ERR_ARG;
-        }
-        if (dev)
-                return launch_trace_camera(tc, cam, sh, x0, y0, x1, y1, out, mode, 0, 0, nullptr, 0, gi);
-        vrt_tree* t = const_cast<vrt_tree*>(tc);
-        const uint64_t bytes = (mode == OUT_FILM || mode == OUT_GI_FILM) ? npix * (uint64_t)vrt_film_pixel_bytes(tc->film_fmt) : npix * cam->spp * (mode == OUT_HIT48 ? 48 : 16);
-        if (t->io_out.reserve(bytes))
-                return VRT_ERR_NOMEM;
-        rc = launch_trace_camera(t, cam, sh, x0, y0, x1, y1, t->io_out.p, mode, 0, 0, nullptr, 0, gi);
-        if (rc)
-                return rc;
-        VRT_CUDA(cudaMemcpyAsync(out, t->io_out.p, bytes, cudaMemcpyDeviceToHost, t->stream));
-        VRT_CUDA(cudaStreamSynchronize(t->stream));
-        return VRT_OK;
-}
-
 int vrt_film_pixel_bytes(int32_t format)
 {
         switch (format) {
@@ -1264,139 +1234,146 @@ static int gi_writer_end(vrt_tree* t, int rc)
         return rc;
 }
 
-// Pipelined frame loop: the kernel of frame k+1 runs while frame k's film crosses PCIe.
-int vrt_render_camera_async(const vrt_tree* tc, const vrt_camera* cam, const vrt_shade* sh, int x0, int y0, int x1,
-                            int y1, float* film_rgb)
+// ---- camera requests --------------------------------------------------------------------------------------------
+// Every film and hit entry point of the camera kernels is one request: a camera and a rectangle or bands, the outputs
+// of its mode and its shade or GI arguments.  check_request refuses it or finds it empty, and render() runs it in the
+// entry point's form.
+enum Form {
+        ONE_SHOT,  // host outputs, in host memory when the call returns
+        DEV,  // device outputs, enqueued on the handle's stream
+        PIPELINED,  // host outputs, enqueued as one frame of the pipelined loop
+        REPLICA,  // PIPELINED on one replica of a vrt_mgpu, whose arguments the replica set has checked
+};
+
+struct CameraRequest {
+        OutMode mode;
+        Form form;
+        const vrt_camera* cam;
+        int x0, y0, x1, y1;  // the rectangle; banded requests: set from the bands by check_request
+        bool banded;  // the rows of the bands b, not the rectangle
+        const vrt_bands* b;
+        void* out;  // the film, or the hit records of the hit modes (OUT_GI_AOV: the film or NULL)
+        const vrt_shade* sh;  // OUT_FILM, OUT_HIT16_FILM
+        const vrt_gi_aov* aov;  // OUT_GI_AOV
+        const float* kd;  // OUT_GI_*
+        float res;  // OUT_GI_*
+        void* out2;  // OUT_HIT16_FILM: the film
+        int film_full;  // OUT_HIT16_FILM: the film is the full frame
+};
+
+static bool is_gi(OutMode m) { return m == OUT_GI_FILM || m == OUT_GI_AOV; }
+static bool is_hit(OutMode m) { return m == OUT_HIT48 || m == OUT_HIT16 || m == OUT_HIT16_FILM; }
+static bool is_empty(const CameraRequest& q) { return q.x1 <= q.x0 || q.y1 <= q.y0; }
+
+static int check_gi_args(const CameraRequest& q)
 {
-        int rc = check_tree(tc);
-        if (rc)
-                return rc;
-        rc = check_camera(cam, x0, y0, x1, y1);
-        if (rc)
-                return rc;
-        const uint64_t npix = (uint64_t)(x1 - x0) * (y1 - y0);
-        if (!npix)
-                return VRT_OK;
-        if (!film_rgb || !sh) {
-                set_error("null out/shade pointer");
+        if (!q.kd || (q.mode == OUT_GI_AOV && !q.aov)) {
+                set_error("null argument");
                 return VRT_ERR_ARG;
         }
-        vrt_tree* t = const_cast<vrt_tree*>(tc);
-        rc = async_pipeline_prepare(t);
-        if (rc)
-                return rc;
-        cudaStream_t ks = async_kernel_stream(t);
-        const int k = (int)(t->n_async_frames & 1);
-        const uint64_t bytes = npix * (uint64_t)vrt_film_pixel_bytes(t->film_fmt);
-        if (t->film_dev[k].cap < bytes) {
-                VRT_CUDA(cudaStreamSynchronize(t->copy_stream));  // nothing may still read the old buffer
-                if (t->film_dev[k].reserve(bytes))
-                        return VRT_ERR_NOMEM;
+        const vrt_gi_aov* a = q.aov;
+        if (q.mode == OUT_GI_AOV && !a->albedo && !a->direct && !a->indirect && !a->normal && !a->hits) {
+                set_error("every GI plane is NULL (the film alone is the GI film call)");
+                return VRT_ERR_ARG;
         }
-        if (t->n_async_frames >= 2)  // the copy that last read this device film must be done
-                VRT_CUDA(cudaStreamWaitEvent(ks, t->film_copied[k], 0));
-        t->launch_stream = ks;
-        rc = launch_trace_camera(t, cam, sh, x0, y0, x1, y1, t->film_dev[k].p, OUT_FILM);
-        t->launch_stream = nullptr;
-        if (rc)
-                return rc;
-        VRT_CUDA(cudaEventRecord(t->film_ready[k], ks));
-        VRT_CUDA(cudaStreamWaitEvent(t->copy_stream, t->film_ready[k], 0));
-        VRT_CUDA(cudaMemcpyAsync(film_rgb, t->film_dev[k].p, bytes, cudaMemcpyDeviceToHost, t->copy_stream));
-        VRT_CUDA(cudaEventRecord(t->film_copied[k], t->copy_stream));
-        t->n_async_frames++;
         return VRT_OK;
 }
 
-int vrt_trace_camera(const vrt_tree* t, const vrt_camera* cam, int x0, int y0, int x1, int y1, vrt_hit* out)
+// The checks a request makes before its handle: res first in every GI form (a refused call touches no handle and no
+// stream), then kd and the planes in the pipelined ones.
+static int check_request_args(const CameraRequest& q)
 {
-        return trace_camera_common(t, cam, nullptr, x0, y0, x1, y1, out, OUT_HIT48, false);
-}
-int vrt_trace_camera_dev(const vrt_tree* t, const vrt_camera* cam, int x0, int y0, int x1, int y1, vrt_hit* d_out)
-{
-        return trace_camera_common(t, cam, nullptr, x0, y0, x1, y1, d_out, OUT_HIT48, true);
-}
-int vrt_trace_camera16_dev(const vrt_tree* t, const vrt_camera* cam, int x0, int y0, int x1, int y1, vrt_hit16* d_out)
-{
-        return trace_camera_common(t, cam, nullptr, x0, y0, x1, y1, d_out, OUT_HIT16, true);
-}
-int vrt_render_camera(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, int x0, int y0, int x1, int y1,
-                      float* film_rgb)
-{
-        return trace_camera_common(t, cam, sh, x0, y0, x1, y1, film_rgb, OUT_FILM, false);
-}
-int vrt_render_camera_dev(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, int x0, int y0, int x1,
-                          int y1, float* d_film_rgb)
-{
-        return trace_camera_common(t, cam, sh, x0, y0, x1, y1, d_film_rgb, OUT_FILM, true);
-}
-
-int vrt_count_camera(const vrt_tree* tc, const vrt_camera* cam, int x0, int y0, int x1, int y1, uint64_t counts[8])
-{
-        int rc = check_tree(tc);
-        if (rc)
-                return rc;
-        rc = check_camera(cam, x0, y0, x1, y1);
-        if (rc)
-                return rc;
-        if (!counts) {
-                set_error("null counts");
-                return VRT_ERR_ARG;
-        }
-        vrt_tree* t = const_cast<vrt_tree*>(tc);
-        if (t->io_out.reserve(64))
-                return VRT_ERR_NOMEM;
-        VRT_CUDA(cudaMemsetAsync(t->io_out.p, 0, 64, t->stream));
-        memset(counts, 0, 8 * sizeof(uint64_t));
-        if (x1 > x0 && y1 > y0) {
-                rc = launch_trace_camera(t, cam, nullptr, x0, y0, x1, y1, t->io_out.p, OUT_COUNT);
-                if (rc)
-                        return rc;
-        }
-        VRT_CUDA(cudaMemcpyAsync(counts, t->io_out.p, 64, cudaMemcpyDeviceToHost, t->stream));
-        VRT_CUDA(cudaStreamSynchronize(t->stream));
-        return VRT_OK;
-}
-
-int vrt_band_rows(const vrt_camera* cam, const vrt_bands* b)
-{
-        if (!cam || !b || b->band_h < 1 || b->band_stride < 1 || b->band_first < 0) {
-                set_error("bad band description");
-                return VRT_ERR_ARG;
-        }
-        long rows = 0;
-        for (long k = b->band_first; k * b->band_h < cam->ny; k += b->band_stride)
-                rows += std::min<long>(b->band_h, cam->ny - k * b->band_h);
-        return (int)rows;
-}
-
-static int bands_common(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, const vrt_bands* b, void* d_out,
-                        OutMode mode)
-{
-        int rc = check_tree(t);
-        if (rc)
-                return rc;
-        rc = check_camera(cam, 0, 0, cam ? cam->nx : 0, cam ? cam->ny : 0);
-        if (rc)
-                return rc;
-        const int rows = vrt_band_rows(cam, b);
-        if (rows < 0)
-                return rows;
-        if (rows == 0)
+        if (!is_gi(q.mode))
                 return VRT_OK;
-        if (!d_out || (mode == OUT_FILM && !sh)) {
+        int rc = check_gi_res(q.res);
+        if (!rc && q.form >= PIPELINED)
+                rc = check_gi_args(q);
+        return rc;
+}
+
+// Every check of a camera request, in one order.  VRT_OK for an empty request (is_empty) means nothing to do: the
+// rectangle and banded forms return it before they look at the outputs, the one-shot GI forms only after every check.
+static int check_request(const vrt_tree* t, CameraRequest& q)
+{
+        const bool gi = is_gi(q.mode), one_shot_gi = gi && q.form < PIPELINED;
+        int rc = q.form == REPLICA ? VRT_OK : check_request_args(q);
+        if (!rc)
+                rc = check_tree(t);
+        if (!rc)
+                rc = q.banded ? check_camera(q.cam, 0, 0, q.cam ? q.cam->nx : 0, q.cam ? q.cam->ny : 0)
+                         : check_camera(q.cam, q.x0, q.y0, q.x1, q.y1);
+        if (!rc && q.banded) {  // the rows of a banded request: [0, nx) x [y0_film, y0_film + rows)
+                const int rows = vrt_band_rows(q.cam, q.b);
+                if (rows < 0)
+                        return rows;
+                q.x1 = q.cam->nx;
+                q.y0 = rows ? q.b->band_first * q.b->band_h : 0;
+                q.y1 = q.y0 + rows;
+        }
+        if (rc || (is_empty(q) && !one_shot_gi))
+                return rc;
+        if (one_shot_gi && (rc = check_gi_args(q)))
+                return rc;
+        const bool shade = q.mode == OUT_FILM || q.mode == OUT_HIT16_FILM;
+        if ((q.mode != OUT_GI_AOV && !q.out) || (q.mode == OUT_HIT16_FILM && !q.out2) || (shade && !q.sh)) {
                 set_error("null out/shade pointer");
                 return VRT_ERR_ARG;
         }
-        const int y0 = b->band_first * b->band_h;
-        return launch_trace_camera(t, cam, sh, 0, y0, cam->nx, y0 + rows, d_out, mode, b->band_h,
-                                   b->band_stride * b->band_h);
+        if (gi && !t->dev.gi) {
+                set_error("vrt_gi_init has not been called on this tree");
+                return VRT_ERR_ARG;
+        }
+        return VRT_OK;
 }
 
-int vrt_render_bands_dev(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, const vrt_bands* b,
-                         float* d_film_rgb)
+// The outputs of a request, in this order: film, albedo, direct, indirect, normal, hit records (NULL: not requested).
+// Host requests lay them out in one device buffer, each part 256-byte aligned after the one before it.
+struct Layout {
+        char* part[6];
+        size_t row_bytes[6];
+        uint64_t off[6], bytes;
+        void place(char* base, char* d[6]) const  // the parts in the device buffer at `base`
+        {
+                for (int i = 0; i < 6; ++i)
+                        d[i] = part[i] ? base + off[i] : nullptr;
+        }
+};
+
+static Layout layout(const vrt_tree* t, const CameraRequest& q)
 {
-        return bands_common(t, cam, sh, b, d_film_rgb, OUT_FILM);
+        const vrt_gi_aov a = q.mode == OUT_GI_AOV ? *q.aov : vrt_gi_aov{};
+        const bool hit = is_hit(q.mode);
+        const void* const part[6] = { hit ? q.out2 : q.out, a.albedo, a.direct, a.indirect, a.normal,
+                                      hit ? q.out : a.hits };
+        const size_t w = (size_t)(q.x1 - q.x0), plane = w * 12;
+        const size_t row_bytes[6] = { w * (size_t)vrt_film_pixel_bytes(t->film_fmt), plane, plane, plane, plane,
+                                      w * q.cam->spp * (q.mode == OUT_HIT48 ? sizeof(vrt_hit) : sizeof(vrt_hit16)) };
+        Layout lo{};
+        for (int i = 0; i < 6; ++i) {
+                lo.part[i] = static_cast<char*>(const_cast<void*>(part[i]));
+                lo.row_bytes[i] = row_bytes[i];
+                if (part[i]) {
+                        lo.off[i] = align256(lo.bytes);
+                        lo.bytes = lo.off[i] + (uint64_t)(q.y1 - q.y0) * row_bytes[i];
+                }
+        }
+        return lo;
+}
+
+// The launch of a checked request whose outputs are at the device pointers d[] (Layout order).
+static int launch_request(const vrt_tree* t, const CameraRequest& q, char* const d[6], cudaStream_t s)
+{
+        const vrt_gi_aov aov = { reinterpret_cast<float*>(d[1]), reinterpret_cast<float*>(d[2]),
+                                 reinterpret_cast<float*>(d[3]), reinterpret_cast<float*>(d[4]),
+                                 reinterpret_cast<vrt_hit16*>(d[5]) };
+        const bool hit = is_hit(q.mode);
+        CameraLaunch l{ q.cam, q.x0, q.y0, q.x1, q.y1, q.banded ? q.b->band_h : 0,
+                        q.banded ? q.b->band_stride * q.b->band_h : 0,
+                        q.mode, hit ? d[5] : d[0], hit ? d[0] : nullptr, q.film_full,
+                        q.mode == OUT_GI_AOV ? aov : vrt_gi_aov{}, q.sh, {}, q.res, s };
+        for (int c = 0; c < 3 && q.kd; ++c)
+                l.kd[c] = q.kd[c];
+        return launch_trace_camera(t, l);
 }
 
 // One output's compact band rows (src: this rank's rows, band after band) to their final rows of the full host
@@ -1422,92 +1399,69 @@ static int copy_bands_to_host(char* dst_full, const char* src, size_t row_bytes,
         return VRT_OK;
 }
 
-// Multi-GPU frame loop to HOST memory: this rank's bands are rendered into one of two device
-// band buffers and copied by one strided DMA (cudaMemcpy2DAsync: one row per band) straight to
-// their final rows of the full host frame, which every rank of the node maps (shared + pinned),
-// so the N ranks use their N PCIe links in parallel and the copy of frame k overlaps the kernel
-// of frame k+1 -- the N-GPU counterpart of vrt_render_camera_async.  mode OUT_FILM: the harness
-// film (sh); OUT_GI_FILM: the cone-traced GI film (gi->kd, gi->res; the step table is filled on
-// the frame's kernel stream); OUT_GI_AOV: the GI film (film_rgb_full may be NULL) plus the planes
-// of aov_full (host frames), whose compact band rows share the frame slot's one device buffer.
-static int bands_async_common(const vrt_tree* tc, const vrt_camera* cam, const vrt_shade* sh, const GiArgs* gi,
-                              const vrt_gi_aov* aov_full, const vrt_bands* b, float* film_rgb_full, OutMode mode)
+// Each requested output from its device part d[i] to the caller's host memory: a rectangle in one copy, bands to
+// their final rows of the full host frame.
+static int copy_to_host(const CameraRequest& q, const Layout& lo, char* const d[6], cudaStream_t s)
 {
-        int rc = check_tree(tc);
-        if (rc)
-                return rc;
-        rc = check_camera(cam, 0, 0, cam ? cam->nx : 0, cam ? cam->ny : 0);
-        if (rc)
-                return rc;
-        const int rows = vrt_band_rows(cam, b);
-        if (rows < 0)
-                return rows;
-        if (rows == 0)
-                return VRT_OK;
-        if ((mode == OUT_GI_AOV ? !aov_full : !film_rgb_full) || (mode == OUT_FILM ? !sh : !gi)) {
-                set_error("null out/shade pointer");
-                return VRT_ERR_ARG;
-        }
-        if (mode != OUT_FILM && !tc->dev.gi) {
-                set_error("vrt_gi_init has not been called on this tree");
-                return VRT_ERR_ARG;
-        }
-        // the outputs (film, albedo, direct, indirect, normal, hits): full host frames, and the bytes of one row
-        const vrt_gi_aov none = {};
-        const vrt_gi_aov& a = mode == OUT_GI_AOV ? *aov_full : none;
-        char* const dst[6] = { reinterpret_cast<char*>(film_rgb_full), reinterpret_cast<char*>(a.albedo),
-                               reinterpret_cast<char*>(a.direct), reinterpret_cast<char*>(a.indirect),
-                               reinterpret_cast<char*>(a.normal), reinterpret_cast<char*>(a.hits) };
-        const size_t plane_row = (size_t)cam->nx * 12;
-        const size_t row_bytes[6] = { (size_t)cam->nx * (size_t)vrt_film_pixel_bytes(tc->film_fmt), plane_row,
-                                      plane_row, plane_row, plane_row, (size_t)cam->nx * cam->spp * sizeof(vrt_hit16) };
-        // their compact band rows in the frame slot's one device buffer, each part 256-byte aligned
-        uint64_t off[6] = {}, bytes = 0;
-        for (int i = 0; i < 6; ++i)
-                if (dst[i]) {
-                        off[i] = (bytes + 255) & ~255ull;
-                        bytes = off[i] + (uint64_t)rows * row_bytes[i];
+        const int rows = q.y1 - q.y0;
+        for (int i = 0; i < 6; ++i) {
+                if (!lo.part[i])
+                        continue;
+                if (q.banded) {
+                        if (const int rc = copy_bands_to_host(lo.part[i], d[i], lo.row_bytes[i], q.b, rows, s))
+                                return rc;
+                } else {
+                        VRT_CUDA(cudaMemcpyAsync(lo.part[i], d[i], (size_t)rows * lo.row_bytes[i], cudaMemcpyDeviceToHost,
+                                                 s));
                 }
+        }
+        return VRT_OK;
+}
+
+// Checks a request and runs it in its form.  The _dev forms launch into the caller's pointers on the handle's stream.
+// The one-shot forms launch into io_out on the handle's stream, copy and synchronise.  A pipelined frame (the kernel of
+// frame k+1 runs while frame k's outputs cross PCIe) takes frame slot k = the frame's parity: its kernel stream, its
+// device buffer film_dev[k] (grown only after the copy stream has drained: nothing may still read the old buffer), and
+// a wait for the copy that last read that buffer; after the launch the copy stream waits for the kernel
+// (film_ready[k]), copies every output and records film_copied[k].
+static int render(const vrt_tree* tc, CameraRequest q)
+{
+        int rc = check_request(tc, q);
+        if (rc || is_empty(q))
+                return rc;
         vrt_tree* t = const_cast<vrt_tree*>(tc);
+        Layout lo = layout(t, q);
+        if (q.form == DEV)
+                return launch_request(t, q, lo.part, t->stream);
+        char* d[6];
+        if (q.form == ONE_SHOT) {
+                if (t->io_out.reserve(lo.bytes))
+                        return VRT_ERR_NOMEM;
+                lo.place(t->io_out.as<char>(), d);
+                if ((rc = launch_request(t, q, d, t->stream)) || (rc = copy_to_host(q, lo, d, t->stream)))
+                        return rc;
+                VRT_CUDA(cudaStreamSynchronize(t->stream));
+                return VRT_OK;
+        }
         rc = async_pipeline_prepare(t);
         if (rc)
                 return rc;
         cudaStream_t ks = async_kernel_stream(t);
         const int k = (int)(t->n_async_frames & 1);
-        if (t->film_dev[k].cap < bytes) {
-                VRT_CUDA(cudaStreamSynchronize(t->copy_stream));  // nothing may still read the old buffer
-                if (t->film_dev[k].reserve(bytes))
+        if (t->film_dev[k].cap < lo.bytes) {
+                VRT_CUDA(cudaStreamSynchronize(t->copy_stream));
+                if (t->film_dev[k].reserve(lo.bytes))
                         return VRT_ERR_NOMEM;
         }
-        if (t->n_async_frames >= 2)  // the copy that last read this device buffer must be done
+        if (t->n_async_frames >= 2)
                 VRT_CUDA(cudaStreamWaitEvent(ks, t->film_copied[k], 0));
-        char* const base = static_cast<char*>(t->film_dev[k].p);
-        vrt_gi_aov d_aov = {};
-        float** const d_planes[4] = { &d_aov.albedo, &d_aov.direct, &d_aov.indirect, &d_aov.normal };
-        for (int i = 0; i < 4; ++i)
-                if (dst[i + 1])
-                        *d_planes[i] = reinterpret_cast<float*>(base + off[i + 1]);
-        if (dst[5])
-                d_aov.hits = reinterpret_cast<vrt_hit16*>(base + off[5]);
-        const int y0 = b->band_first * b->band_h;
-        t->launch_stream = ks;
-        GiArgs ga{};
-        if (mode != OUT_FILM) {
-                ga = *gi;
-                rc = gi_step_table(t, ga.res, &ga.steps);
-        }
-        if (!rc)
-                rc = launch_trace_camera(t, cam, sh, 0, y0, cam->nx, y0 + rows, dst[0] ? base + off[0] : nullptr, mode,
-                                         b->band_h, b->band_stride * b->band_h, nullptr, 0,
-                                         mode == OUT_FILM ? nullptr : &ga, mode == OUT_GI_AOV ? &d_aov : nullptr);
-        t->launch_stream = nullptr;
+        lo.place(t->film_dev[k].as<char>(), d);
+        rc = launch_request(t, q, d, ks);
         if (rc)
                 return rc;
         VRT_CUDA(cudaEventRecord(t->film_ready[k], ks));
         VRT_CUDA(cudaStreamWaitEvent(t->copy_stream, t->film_ready[k], 0));
-        for (int i = 0; i < 6 && !rc; ++i)
-                if (dst[i])
-                        rc = copy_bands_to_host(dst[i], base + off[i], row_bytes[i], b, rows, t->copy_stream);
+        rc = copy_to_host(q, lo, d, t->copy_stream);
         if (rc)
                 return rc;
         VRT_CUDA(cudaEventRecord(t->film_copied[k], t->copy_stream));
@@ -1515,51 +1469,108 @@ static int bands_async_common(const vrt_tree* tc, const vrt_camera* cam, const v
         return VRT_OK;
 }
 
+int vrt_trace_camera(const vrt_tree* t, const vrt_camera* cam, int x0, int y0, int x1, int y1, vrt_hit* out)
+{
+        return render(t, { OUT_HIT48, ONE_SHOT, cam, x0, y0, x1, y1, false, nullptr, out });
+}
+int vrt_trace_camera_dev(const vrt_tree* t, const vrt_camera* cam, int x0, int y0, int x1, int y1, vrt_hit* d_out)
+{
+        return render(t, { OUT_HIT48, DEV, cam, x0, y0, x1, y1, false, nullptr, d_out });
+}
+int vrt_trace_camera16_dev(const vrt_tree* t, const vrt_camera* cam, int x0, int y0, int x1, int y1, vrt_hit16* d_out)
+{
+        return render(t, { OUT_HIT16, DEV, cam, x0, y0, x1, y1, false, nullptr, d_out });
+}
+int vrt_render_camera(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, int x0, int y0, int x1, int y1,
+                      float* film_rgb)
+{
+        return render(t, { OUT_FILM, ONE_SHOT, cam, x0, y0, x1, y1, false, nullptr, film_rgb, sh });
+}
+int vrt_render_camera_dev(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, int x0, int y0, int x1,
+                          int y1, float* d_film_rgb)
+{
+        return render(t, { OUT_FILM, DEV, cam, x0, y0, x1, y1, false, nullptr, d_film_rgb, sh });
+}
+// Pipelined frame loop: the kernel of frame k+1 runs while frame k's film crosses PCIe.
+int vrt_render_camera_async(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, int x0, int y0, int x1,
+                            int y1, float* film_rgb)
+{
+        return render(t, { OUT_FILM, PIPELINED, cam, x0, y0, x1, y1, false, nullptr, film_rgb, sh });
+}
+
+int vrt_count_camera(const vrt_tree* tc, const vrt_camera* cam, int x0, int y0, int x1, int y1, uint64_t counts[8])
+{
+        int rc = check_tree(tc);
+        if (rc)
+                return rc;
+        rc = check_camera(cam, x0, y0, x1, y1);
+        if (rc)
+                return rc;
+        if (!counts) {
+                set_error("null counts");
+                return VRT_ERR_ARG;
+        }
+        vrt_tree* t = const_cast<vrt_tree*>(tc);
+        if (t->io_out.reserve(64))
+                return VRT_ERR_NOMEM;
+        VRT_CUDA(cudaMemsetAsync(t->io_out.p, 0, 64, t->stream));
+        memset(counts, 0, 8 * sizeof(uint64_t));
+        if (x1 > x0 && y1 > y0) {
+                CameraLaunch l{ cam, x0, y0, x1, y1, 0, 0, OUT_COUNT, t->io_out.p };
+                l.stream = t->stream;
+                rc = launch_trace_camera(t, l);
+                if (rc)
+                        return rc;
+        }
+        VRT_CUDA(cudaMemcpyAsync(counts, t->io_out.p, 64, cudaMemcpyDeviceToHost, t->stream));
+        VRT_CUDA(cudaStreamSynchronize(t->stream));
+        return VRT_OK;
+}
+
+int vrt_band_rows(const vrt_camera* cam, const vrt_bands* b)
+{
+        if (!cam || !b || b->band_h < 1 || b->band_stride < 1 || b->band_first < 0) {
+                set_error("bad band description");
+                return VRT_ERR_ARG;
+        }
+        long rows = 0;
+        for (long k = b->band_first; k * b->band_h < cam->ny; k += b->band_stride)
+                rows += std::min<long>(b->band_h, cam->ny - k * b->band_h);
+        return (int)rows;
+}
+
+int vrt_render_bands_dev(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, const vrt_bands* b,
+                         float* d_film_rgb)
+{
+        return render(t, { OUT_FILM, DEV, cam, 0, 0, 0, 0, true, b, d_film_rgb, sh });
+}
+
+// Multi-GPU frame loop to HOST memory: this rank's bands are rendered into one of two device
+// band buffers and copied by one strided DMA (cudaMemcpy2DAsync: one row per band) straight to
+// their final rows of the full host frame, which every rank of the node maps (shared + pinned),
+// so the N ranks use their N PCIe links in parallel and the copy of frame k overlaps the kernel
+// of frame k+1 -- the N-GPU counterpart of vrt_render_camera_async.
 int vrt_render_bands_async(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, const vrt_bands* b,
                            float* film_rgb_full)
 {
-        return bands_async_common(t, cam, sh, nullptr, nullptr, b, film_rgb_full, OUT_FILM);
+        return render(t, { OUT_FILM, PIPELINED, cam, 0, 0, 0, 0, true, b, film_rgb_full, sh });
 }
 
 // The cone-traced GI film (vrt_gi_render_camera) through the same banded, pipelined path.
 int vrt_gi_render_bands_async(const vrt_tree* t, const vrt_camera* cam, const float kd[3], float res,
                               const vrt_bands* b, float* film_rgb_full)
 {
-        if (const int rc = check_gi_res(res))
-                return rc;
-        if (!kd) {
-                set_error("null argument");
-                return VRT_ERR_ARG;
-        }
-        const GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
-        return bands_async_common(t, cam, nullptr, &ga, nullptr, b, film_rgb_full, OUT_GI_FILM);
+        return render(t, { OUT_GI_FILM, PIPELINED, cam, 0, 0, 0, 0, true, b,
+                           film_rgb_full, nullptr, nullptr, kd, res });
 }
 
-// kd and the planes of a banded plane request: VRT_ERR_ARG for a null pointer or a request without any plane
-static int check_gi_aov_request(const float kd[3], const vrt_gi_aov* aov)
-{
-        if (!kd || !aov) {
-                set_error("null argument");
-                return VRT_ERR_ARG;
-        }
-        if (!aov->albedo && !aov->direct && !aov->indirect && !aov->normal && !aov->hits) {
-                set_error("every GI plane is NULL (the film alone is the banded GI film call)");
-                return VRT_ERR_ARG;
-        }
-        return VRT_OK;
-}
-
-// The GI film and its planes (vrt_gi_render_aov) through the same banded, pipelined path.
+// The GI film and its planes (vrt_gi_render_aov) through the same banded, pipelined path: the compact band rows of
+// every requested output share the frame slot's one device buffer.
 int vrt_gi_render_aov_bands_async(const vrt_tree* t, const vrt_camera* cam, const float kd[3], float res,
                                   const vrt_bands* b, float* film_full_or_null, const vrt_gi_aov* aov_full)
 {
-        if (const int rc = check_gi_res(res))
-                return rc;
-        const int rc = check_gi_aov_request(kd, aov_full);
-        if (rc)
-                return rc;
-        const GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
-        return bands_async_common(t, cam, nullptr, &ga, aov_full, b, film_full_or_null, OUT_GI_AOV);
+        return render(t, { OUT_GI_AOV, PIPELINED, cam, 0, 0, 0, 0, true, b,
+                           film_full_or_null, nullptr, aov_full, kd, res });
 }
 
 // ---- animated geometry: new input triangles, then the build of vrt_rebuild ---------------------------------------
@@ -1874,22 +1885,34 @@ int mgpu_each(vrt_mgpu* m, F&& f)
 }  // namespace
 }  // extern "C++"
 
-// one frame: the 8-row bands dealt round-robin, each replica through its bands_async_common pipeline
-static int mgpu_bands_async(vrt_mgpu* m, const vrt_camera* cam, const vrt_shade* sh, const GiArgs* gi,
-                            const vrt_gi_aov* aov_full, float* film_rgb_full, OutMode mode)
+// one frame: the 8-row bands dealt round-robin, each replica through its own pipelined frame loop; the arguments are
+// checked once, before the replica set
+static int mgpu_bands_async(vrt_mgpu* m, const CameraRequest& q)
 {
+        if (const int rc = check_request_args(q))
+                return rc;
         const int n = m ? (int)m->trees.size() : 0;
         return mgpu_each(m, [&](int i, vrt_tree* t) {
-                if (cam && (long)i * m->band_h >= cam->ny)
+                if (q.cam && (long)i * m->band_h >= q.cam->ny)
                         return (int)VRT_OK;  // more devices than bands
                 const vrt_bands b = { m->band_h, i, n };
-                return bands_async_common(t, cam, sh, gi, aov_full, &b, film_rgb_full, mode);
+                CameraRequest r = q;
+                r.b = &b;
+                return render(t, r);
         });
+}
+
+// the synchronous forms: the frame, then vrt_mgpu_sync (also after a refused frame: replicas before the refusing one
+// have enqueued their bands); a null handle keeps the frame's error message
+static int mgpu_sync_after(vrt_mgpu* m, int rc)
+{
+        const int rs = m ? vrt_mgpu_sync(m) : VRT_OK;
+        return rc ? rc : rs;
 }
 
 int vrt_mgpu_render_async(vrt_mgpu* m, const vrt_camera* cam, const vrt_shade* sh, float* film_rgb_full)
 {
-        return mgpu_bands_async(m, cam, sh, nullptr, nullptr, film_rgb_full, OUT_FILM);
+        return mgpu_bands_async(m, { OUT_FILM, REPLICA, cam, 0, 0, 0, 0, true, nullptr, film_rgb_full, sh });
 }
 
 int vrt_mgpu_sync(vrt_mgpu* m)
@@ -1914,9 +1937,7 @@ int vrt_mgpu_sync(vrt_mgpu* m)
 
 int vrt_mgpu_render(vrt_mgpu* m, const vrt_camera* cam, const vrt_shade* sh, float* film_rgb_full)
 {
-        int rc = vrt_mgpu_render_async(m, cam, sh, film_rgb_full);
-        const int rs = vrt_mgpu_sync(m);
-        return rc ? rc : rs;
+        return mgpu_sync_after(m, vrt_mgpu_render_async(m, cam, sh, film_rgb_full));
 }
 
 // ---- GI film on the replicas.  vrt_mgpu_create copies the geometry blob only; materials and the per-node GI state
@@ -1947,45 +1968,26 @@ int vrt_mgpu_gi_filter(vrt_mgpu* m)
 
 int vrt_mgpu_gi_render_async(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_rgb_full)
 {
-        if (const int rc = check_gi_res(res))
-                return rc;
-        if (!kd) {
-                set_error("null argument");
-                return VRT_ERR_ARG;
-        }
-        const GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
-        return mgpu_bands_async(m, cam, nullptr, &ga, nullptr, film_rgb_full, OUT_GI_FILM);
+        return mgpu_bands_async(m, { OUT_GI_FILM, REPLICA, cam, 0, 0, 0, 0, true, nullptr,
+                                     film_rgb_full, nullptr, nullptr, kd, res });
 }
 
 int vrt_mgpu_gi_render(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_rgb_full)
 {
-        if (const int rc = check_gi_res(res))
-                return rc;
-        int rc = vrt_mgpu_gi_render_async(m, cam, kd, res, film_rgb_full);
-        const int rs = vrt_mgpu_sync(m);
-        return rc ? rc : rs;
+        return mgpu_sync_after(m, vrt_mgpu_gi_render_async(m, cam, kd, res, film_rgb_full));
 }
 
 int vrt_mgpu_gi_render_aov_async(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res,
                                  float* film_full_or_null, const vrt_gi_aov* aov_full)
 {
-        if (const int rc = check_gi_res(res))
-                return rc;
-        const int rc = check_gi_aov_request(kd, aov_full);
-        if (rc)
-                return rc;
-        const GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
-        return mgpu_bands_async(m, cam, nullptr, &ga, aov_full, film_full_or_null, OUT_GI_AOV);
+        return mgpu_bands_async(m, { OUT_GI_AOV, REPLICA, cam, 0, 0, 0, 0, true, nullptr,
+                                     film_full_or_null, nullptr, aov_full, kd, res });
 }
 
 int vrt_mgpu_gi_render_aov(vrt_mgpu* m, const vrt_camera* cam, const float kd[3], float res, float* film_full_or_null,
                            const vrt_gi_aov* aov_full)
 {
-        if (const int rc = check_gi_res(res))
-                return rc;
-        int rc = vrt_mgpu_gi_render_aov_async(m, cam, kd, res, film_full_or_null, aov_full);
-        const int rs = vrt_mgpu_sync(m);
-        return rc ? rc : rs;
+        return mgpu_sync_after(m, vrt_mgpu_gi_render_aov_async(m, cam, kd, res, film_full_or_null, aov_full));
 }
 
 // ---- animated geometry on the replicas: the first replica rebuilds (the build synchronises the host at every level,
@@ -2084,7 +2086,7 @@ double vrt_mgpu_mean_kernel_ms(vrt_mgpu* m, int index, int last_n)
 
 int vrt_trace_bands16_dev(const vrt_tree* t, const vrt_camera* cam, const vrt_bands* b, vrt_hit16* d_out)
 {
-        return bands_common(t, cam, nullptr, b, d_out, OUT_HIT16);
+        return render(t, { OUT_HIT16, DEV, cam, 0, 0, 0, 0, true, b, d_out });
 }
 
 double vrt_last_kernel_ms(const vrt_tree* t)
@@ -2303,121 +2305,33 @@ int vrt_albedo(const vrt_tree* tc, const uint32_t* tri, const float* pos, uint64
         return VRT_OK;
 }
 
-static int gi_render_common(const vrt_tree* tc, const vrt_camera* cam, const float kd[3], float res, int x0, int y0,
-                            int x1, int y1, float* film, bool dev)
-{
-        if (const int rc = check_gi_res(res))
-                return rc;
-        int rc = check_tree(tc);
-        if (rc)
-                return rc;
-        if (!cam || !kd || !film) {
-                set_error("null argument");
-                return VRT_ERR_ARG;
-        }
-        if (!tc->dev.gi) {
-                set_error("vrt_gi_init has not been called on this tree");
-                return VRT_ERR_ARG;
-        }
-        GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
-        rc = gi_step_table(tc, res, &ga.steps);
-        if (rc)
-                return rc;
-        return trace_camera_common(tc, cam, nullptr, x0, y0, x1, y1, film, OUT_GI_FILM, dev, &ga);
-}
-
 int vrt_gi_render_camera(const vrt_tree* t, const vrt_camera* cam, const float kd[3], float res, int x0, int y0, int x1,
                          int y1, float* film_rgb)
 {
-        return gi_render_common(t, cam, kd, res, x0, y0, x1, y1, film_rgb, false);
+        return render(t, { OUT_GI_FILM, ONE_SHOT, cam, x0, y0, x1, y1, false, nullptr,
+                           film_rgb, nullptr, nullptr, kd, res });
 }
 
 int vrt_gi_render_camera_dev(const vrt_tree* t, const vrt_camera* cam, const float kd[3], float res, int x0, int y0,
                              int x1, int y1, float* d_film_rgb)
 {
-        return gi_render_common(t, cam, kd, res, x0, y0, x1, y1, d_film_rgb, true);
+        return render(t, { OUT_GI_FILM, DEV, cam, x0, y0, x1, y1, false, nullptr,
+                           d_film_rgb, nullptr, nullptr, kd, res });
 }
 
 // The GI film plus its planes (vrt_gi_aov) in one OUT_GI_AOV launch; host pointers go through one device buffer.
-static int gi_render_aov_common(const vrt_tree* tc, const vrt_camera* cam, const float kd[3], float res, int x0,
-                                int y0, int x1, int y1, float* film, const vrt_gi_aov* aov, bool dev)
-{
-        if (const int rc = check_gi_res(res))
-                return rc;
-        int rc = check_tree(tc);
-        if (rc)
-                return rc;
-        if (!cam || !kd || !aov) {
-                set_error("null argument");
-                return VRT_ERR_ARG;
-        }
-        float* const planes[4] = { aov->albedo, aov->direct, aov->indirect, aov->normal };
-        if (!planes[0] && !planes[1] && !planes[2] && !planes[3] && !aov->hits) {
-                set_error("vrt_gi_render_aov: every plane is NULL (the film alone is vrt_gi_render_camera)");
-                return VRT_ERR_ARG;
-        }
-        if (!tc->dev.gi) {
-                set_error("vrt_gi_init has not been called on this tree");
-                return VRT_ERR_ARG;
-        }
-        rc = check_camera(cam, x0, y0, x1, y1);
-        if (rc)
-                return rc;
-        const uint64_t npix = (uint64_t)(x1 - x0) * (y1 - y0);
-        if (!npix)
-                return VRT_OK;
-        GiArgs ga = { { kd[0], kd[1], kd[2] }, res };
-        rc = gi_step_table(tc, res, &ga.steps);
-        if (rc)
-                return rc;
-        if (dev)
-                return launch_trace_camera(tc, cam, nullptr, x0, y0, x1, y1, film, OUT_GI_AOV, 0, 0, nullptr, 0, &ga, aov);
-        // one device buffer: film, the four float planes, the hit records (each part 256-byte aligned)
-        auto up = [](uint64_t b) { return (b + 255) & ~255ull; };
-        const uint64_t film_bytes = npix * (uint64_t)vrt_film_pixel_bytes(tc->film_fmt), plane_bytes = npix * 12,
-                       hit_bytes = npix * cam->spp * sizeof(vrt_hit16);
-        uint64_t off[6] = { 0 };
-        off[1] = off[0] + (film ? up(film_bytes) : 0);
-        for (int i = 0; i < 4; ++i)
-                off[i + 2] = off[i + 1] + (planes[i] ? up(plane_bytes) : 0);
-        const uint64_t total = off[5] + (aov->hits ? hit_bytes : 0);
-        vrt_tree* t = const_cast<vrt_tree*>(tc);
-        if (t->io_out.reserve(total))
-                return VRT_ERR_NOMEM;
-        char* const base = static_cast<char*>(t->io_out.p);
-        vrt_gi_aov d_aov = {};
-        float** const d_planes[4] = { &d_aov.albedo, &d_aov.direct, &d_aov.indirect, &d_aov.normal };
-        for (int i = 0; i < 4; ++i)
-                if (planes[i])
-                        *d_planes[i] = reinterpret_cast<float*>(base + off[i + 1]);
-        if (aov->hits)
-                d_aov.hits = reinterpret_cast<vrt_hit16*>(base + off[5]);
-        rc = launch_trace_camera(t, cam, nullptr, x0, y0, x1, y1, film ? base : nullptr, OUT_GI_AOV, 0, 0, nullptr, 0,
-                                 &ga, &d_aov);
-        if (rc)
-                return rc;
-        if (film)
-                VRT_CUDA(cudaMemcpyAsync(film, base, film_bytes, cudaMemcpyDeviceToHost, t->stream));
-        for (int i = 0; i < 4; ++i)
-                if (planes[i])
-                        VRT_CUDA(cudaMemcpyAsync(planes[i], base + off[i + 1], plane_bytes, cudaMemcpyDeviceToHost,
-                                                 t->stream));
-        if (aov->hits)
-                VRT_CUDA(cudaMemcpyAsync(aov->hits, base + off[5], hit_bytes, cudaMemcpyDeviceToHost, t->stream));
-        VRT_CUDA(cudaStreamSynchronize(t->stream));
-        return VRT_OK;
-}
-
 int vrt_gi_render_aov(const vrt_tree* t, const vrt_camera* cam, const float kd[3], float res, int x0, int y0, int x1,
                       int y1, float* film_or_null, const vrt_gi_aov* aov)
 {
-        return gi_render_aov_common(t, cam, kd, res, x0, y0, x1, y1, film_or_null, aov, false);
+        return render(t, { OUT_GI_AOV, ONE_SHOT, cam, x0, y0, x1, y1, false, nullptr,
+                           film_or_null, nullptr, aov, kd, res });
 }
 
 int vrt_gi_render_aov_dev(const vrt_tree* t, const vrt_camera* cam, const float kd[3], float res, int x0, int y0,
                           int x1, int y1, float* d_film_or_null, const vrt_gi_aov* d_aov)
 {
-        return gi_render_aov_common(t, cam, kd, res, x0, y0, x1, y1, d_film_or_null, d_aov, true);
+        return render(t, { OUT_GI_AOV, DEV, cam, x0, y0, x1, y1, false, nullptr,
+                           d_film_or_null, nullptr, d_aov, kd, res });
 }
 
 int vrt_debug_param_check(uint64_t out[2])
@@ -2499,39 +2413,18 @@ int vrt_tree_sync(const vrt_tree* t)
         return VRT_OK;
 }
 
-static int frame_common(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, const vrt_bands* b,
-                        vrt_hit16* d_hits, float* d_film_rgb, int film_full)
-{
-        int rc = check_tree(t);
-        if (rc)
-                return rc;
-        rc = check_camera(cam, 0, 0, cam ? cam->nx : 0, cam ? cam->ny : 0);
-        if (rc)
-                return rc;
-        const int rows = vrt_band_rows(cam, b);
-        if (rows < 0)
-                return rows;
-        if (rows == 0)
-                return VRT_OK;
-        if (!d_hits || !d_film_rgb || !sh) {
-                set_error("null out/shade pointer");
-                return VRT_ERR_ARG;
-        }
-        const int y0 = b->band_first * b->band_h;
-        return launch_trace_camera(t, cam, sh, 0, y0, cam->nx, y0 + rows, d_hits, OUT_HIT16_FILM, b->band_h,
-                                   b->band_stride * b->band_h, d_film_rgb, film_full);
-}
-
 int vrt_frame_bands_dev(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, const vrt_bands* b,
                         vrt_hit16* d_hits, float* d_film_rgb)
 {
-        return frame_common(t, cam, sh, b, d_hits, d_film_rgb, 0);
+        return render(t, { OUT_HIT16_FILM, DEV, cam, 0, 0, 0, 0, true, b,
+                           d_hits, sh, nullptr, nullptr, 0.f, d_film_rgb, 0 });
 }
 
 int vrt_frame_bands_peer_dev(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, const vrt_bands* b,
                              vrt_hit16* d_hits, float* d_frame_rgb)
 {
-        return frame_common(t, cam, sh, b, d_hits, d_frame_rgb, 1);
+        return render(t, { OUT_HIT16_FILM, DEV, cam, 0, 0, 0, 0, true, b,
+                           d_hits, sh, nullptr, nullptr, 0.f, d_frame_rgb, 1 });
 }
 
 int vrt_dev_alloc(uint64_t bytes, void** d_ptr)

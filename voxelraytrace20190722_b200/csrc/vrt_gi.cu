@@ -90,9 +90,11 @@ int gi_splat_camera(vrt_tree* t, const vrt_camera* cam, const float kd[3])
                 return VRT_ERR_NOMEM;
         // the light map changes: the filtered levels are stale until the next gi_filter (TreeDev::gi_ok)
         VRT_CUDA(cudaMemsetAsync(const_cast<uint32_t*>(t->dev.gi_ok), 0, 4, t->stream));
-        const GiArgs ga = { { kd[0], kd[1], kd[2] }, 0.f };
-        int rc = launch_trace_camera(t, cam, nullptr, 0, 0, cam->nx, cam->ny, t->keys_a.p, OUT_SPLAT, 0, 0, t->gi_recs.p, 0,
-                                     &ga);
+        CameraLaunch l{ cam, 0, 0, cam->nx, cam->ny, 0, 0, OUT_SPLAT, t->keys_a.p, t->gi_recs.p };
+        for (int c = 0; c < 3; ++c)
+                l.kd[c] = kd[c];
+        l.stream = t->stream;
+        int rc = launch_trace_camera(t, l);
         if (rc)
                 return rc;
         int lb = 1;
@@ -198,7 +200,7 @@ __global__ void k_gi_step_table(GiRoot6 root, float res, float4* tab)
         gi_step_table_fill(root.v, res, tab);
 }
 
-int gi_step_table(const vrt_tree* t, float res, const float4** d_steps)
+int gi_step_table(const vrt_tree* t, float res, cudaStream_t s, const float4** d_steps)
 {
         *d_steps = nullptr;
         static int on = -1;  // VRT_GI_STEPS=0: every cone evaluates the marching arithmetic itself
@@ -208,7 +210,6 @@ int gi_step_table(const vrt_tree* t, float res, const float4** d_steps)
         }
         if (!on)
                 return VRT_OK;
-        cudaStream_t s = t->launch_stream ? t->launch_stream : t->stream;
         Scratch& tab = t->gi_steps[(t->alt_stream && s == t->alt_stream) ? 1 : 0];
         if (tab.reserve((size_t)(kGiMaxSteps + 2) * sizeof(float4)))  // (+1: the cone loop reads one entry ahead)
                 return VRT_ERR_NOMEM;
@@ -266,7 +267,7 @@ int gi_cone_points(const vrt_tree* t, const float* d_pos, const float* d_nrm, ui
         p.res = res;
         p.out = d_out;
         {
-                const int rc = gi_step_table(t, res, &p.steps);
+                const int rc = gi_step_table(t, res, t->stream, &p.steps);
                 if (rc)
                         return rc;
         }

@@ -171,10 +171,8 @@ struct vrt_tree {
         vrt::Scratch film_dev[2];
         cudaStream_t copy_stream = nullptr;
         // the async frame loops alternate their kernels between `stream` and `alt_stream`, so that the head of
-        // frame k+1 fills the SMs the long-ray tail of frame k leaves idle; launch_stream (when set) overrides
-        // `stream` for the next trace launch
+        // frame k+1 fills the SMs the long-ray tail of frame k leaves idle (CameraLaunch::stream)
         cudaStream_t alt_stream = nullptr;
-        mutable cudaStream_t launch_stream = nullptr;
         cudaEvent_t film_ready[2] = {}, film_copied[2] = {};
         // recorded on `stream` when a GI / material writer returns; alt_stream waits on it (vrt_api.cu gi_writer_end)
         cudaEvent_t gi_written = nullptr;
@@ -226,17 +224,24 @@ int import_leaves(vrt_tree* t, int max_depth, const float root_aabb[6], uint64_t
 enum OutMode { OUT_HIT48 = 0, OUT_HIT16 = 1, OUT_FILM = 2, OUT_COUNT = 3, OUT_HIT16_FILM = 4, OUT_SPLAT = 5, OUT_GI_FILM = 6,
               OUT_GI_AOV = 7 };
 int launch_trace_rays(const vrt_tree* t, const vrt_ray* d_rays, uint64_t n, vrt_hit* d_out);
-// band_h > 0: rows [y0,y1) are LOCAL rows of a banded shard; local row r maps to film row
-// y0_film + (r / band_h) * band_pitch + r % band_h (y0 then carries y0_film, y1 = y0 + local rows).
-struct GiArgs {  // OUT_SPLAT / OUT_GI_FILM / OUT_GI_AOV: default material colour, cone-trace min_voxel_size
-        float kd[3];
-        float res;
-        const float4* steps = nullptr;  // step table of the cone trace for (res, root box), see gi_step_table
+// One launch of the camera kernels (value-initialise, then set what the mode reads).
+struct CameraLaunch {
+        const vrt_camera* cam;
+        int x0, y0, x1, y1;  // pixel rectangle; an empty one launches nothing
+        // band_h > 0: rows [y0,y1) are LOCAL rows of a banded shard; local row r maps to film row
+        // y0_film + (r / band_h) * band_pitch + r % band_h (y0 then carries y0_film, y1 = y0 + local rows).
+        int band_h, band_pitch;
+        OutMode mode;
+        void* out;  // film, hit records, OUT_COUNT's counters or OUT_SPLAT's keys (device)
+        void* out2;  // OUT_HIT16_FILM: the film (film_full: rows are film rows); OUT_SPLAT: the splat records
+        int film_full;
+        vrt_gi_aov aov;  // OUT_GI_AOV: device planes, NULL members not written
+        const vrt_shade* sh;  // OUT_FILM / OUT_HIT16_FILM
+        float kd[3];  // OUT_SPLAT / OUT_GI_*: default material colour
+        float res;  // OUT_GI_*: cone-trace min_voxel_size; the launch fills the step table for it on `stream`
+        cudaStream_t stream;  // every operation of the launch is enqueued here
 };
-int launch_trace_camera(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, int x0,
-                        int y0, int x1, int y1, void* d_out, OutMode mode, int band_h = 0,
-                        int band_pitch = 0, void* d_out2 = nullptr, int film_full = 0,
-                        const GiArgs* gi = nullptr, const vrt_gi_aov* aov = nullptr);
+int launch_trace_camera(const vrt_tree* t, const CameraLaunch& l);
 int launch_film_encode(const vrt_tree* t, const float* d_film, uint64_t npix, int fmt, uint8_t* d_out);
 // mean device time (ms) of the last n trace launches (waits for them)
 int trace_ms_mean(const vrt_tree* t, int last_n, double* ms);
@@ -246,9 +251,9 @@ int hull_stats(unsigned long long* out80);
 int gi_init(vrt_tree* t);
 int gi_splat_camera(vrt_tree* t, const vrt_camera* cam, const float kd[3]);
 int gi_filter(vrt_tree* t);
-// fills the tree's step table for `res` on its launch stream (vrt_gi.cuh) -- the table of that kernel stream --
-// and returns the device pointer
-int gi_step_table(const vrt_tree* t, float res, const float4** d_steps);
+// fills the tree's step table for `res` on stream `s` (vrt_gi.cuh) -- the table of that kernel stream -- and returns
+// the device pointer
+int gi_step_table(const vrt_tree* t, float res, cudaStream_t s, const float4** d_steps);
 int gi_cone_points(const vrt_tree* t, const float* d_pos, const float* d_nrm, uint64_t n, float res, float* d_out);
 int gi_albedo_points(const vrt_tree* t, const uint32_t* d_tri, const float* d_pos, uint64_t n, const float kd[3], float* d_out);
 // sort `n` 64-bit keys held in t->keys_a on bits [lo,hi) with the build's radix sort (vrt_build.cu)

@@ -1802,10 +1802,11 @@ static void camera_eye_host(const vrt_camera* cam, float eye[3])
                 eye[k] = o4[k] / o4[3];
 }
 
-int launch_trace_camera(const vrt_tree* t, const vrt_camera* cam, const vrt_shade* sh, int x0, int y0,
-                        int x1, int y1, void* d_out, OutMode mode, int band_h, int band_pitch, void* d_out2, int film_full,
-                        const GiArgs* gi, const vrt_gi_aov* aov)
+int launch_trace_camera(const vrt_tree* t, const CameraLaunch& l)
 {
+        const vrt_camera* cam = l.cam;
+        const int x0 = l.x0, y0 = l.y0, x1 = l.x1, y1 = l.y1;
+        const OutMode mode = l.mode;
         if (x1 <= x0 || y1 <= y0)
                 return VRT_OK;
         if (int rc = check_hull_records(t))
@@ -1825,28 +1826,24 @@ int launch_trace_camera(const vrt_tree* t, const vrt_camera* cam, const vrt_shad
         p.y0 = y0;
         p.x1 = x1;
         p.y1 = y1;
-        p.band_h = band_h > 0 ? band_h : (y1 - y0);
-        p.band_pitch = band_h > 0 ? band_pitch : 0;
-        p.out = d_out;
-        p.out2 = d_out2;
-        p.film_full = film_full;
+        p.band_h = l.band_h > 0 ? l.band_h : (y1 - y0);
+        p.band_pitch = l.band_h > 0 ? l.band_pitch : 0;
+        p.out = l.out;
+        p.out2 = l.out2;
+        p.film_full = l.film_full;
         p.film_fmt = t->film_fmt;
-        if (gi) {
-                p.kd3[0] = gi->kd[0];
-                p.kd3[1] = gi->kd[1];
-                p.kd3[2] = gi->kd[2];
-                p.gi_res = gi->res;
-                p.gi_steps = gi->steps;
-        }
-        if (aov)
-                p.aov = *aov;
-        if (sh) {
-                p.light[0] = sh->light_dir[0];
-                p.light[1] = sh->light_dir[1];
-                p.light[2] = sh->light_dir[2];
-                p.kd = sh->kd;
-                p.shadow = sh->shadow;
-                p.shadow_eps = sh->shadow_eps;
+        p.kd3[0] = l.kd[0];
+        p.kd3[1] = l.kd[1];
+        p.kd3[2] = l.kd[2];
+        p.gi_res = l.res;
+        p.aov = l.aov;
+        if (l.sh) {
+                p.light[0] = l.sh->light_dir[0];
+                p.light[1] = l.sh->light_dir[1];
+                p.light[2] = l.sh->light_dir[2];
+                p.kd = l.sh->kd;
+                p.shadow = l.sh->shadow;
+                p.shadow_eps = l.sh->shadow_eps;
         }
         const int tw = (cam->spp == 4) ? 4 : 8, th = (cam->spp == 4) ? 2 : 4;
         const uint64_t tiles = (uint64_t)((x1 - x0 + tw - 1) / tw) * (uint64_t)((y1 - y0 + th - 1) / th);
@@ -1899,7 +1896,12 @@ int launch_trace_camera(const vrt_tree* t, const vrt_camera* cam, const vrt_shad
         VRT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int grid = persistent_grid(kern, smem);
         grid = (int)std::min<uint64_t>((uint64_t)grid, (tiles + 3) / 4);
-        cudaStream_t ls = t->launch_stream ? t->launch_stream : t->stream;
+        cudaStream_t ls = l.stream;
+        if (mode == OUT_GI_FILM || mode == OUT_GI_AOV) {
+                const int rc = gi_step_table(t, l.res, ls, &p.gi_steps);
+                if (rc)
+                        return rc;
+        }
         const bool use_rel = mode != OUT_COUNT && t->hdr.num_nodes != 0 && t->dev.L >= 1;
         if (use_rel) {
                 const int rc = tab_rel_for_launch(t, p.eye, ls, p.tabrel);
