@@ -508,6 +508,11 @@ int vrt_debug_param_check(uint64_t out[2]);
 /* Test hook: switch the content-hull pruning of the ray kernels off / on for this handle (the hulls stay
  * allocated), so that the pruned traversal can be compared with the unpruned one on the same tree. */
 int vrt_debug_set_hull(vrt_tree* tree, int on);
+/* Test hook: camera launches of this handle read eye-relative hull records and triangle terms (on, the default) or
+ * subtract the eye per ray (off); both give the same results bit for bit. */
+int vrt_debug_set_eye_rel(vrt_tree* tree, int on);
+/* Test hook: number of camera launches of this handle that read eye-relative records so far. */
+int vrt_debug_eye_rel_launches(const vrt_tree* tree, uint64_t* out);
 /* Diagnostic (libraries built with -DVRT_HULL_STATS only, zeros otherwise): per tree level {node expansions, interior
  * children visited, hull tests, hull prunes} of the per-ray kernel since the last call. */
 int vrt_debug_hull_stats(uint64_t out80[80]);

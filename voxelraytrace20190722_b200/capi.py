@@ -81,7 +81,7 @@ SYMBOLS = [
     "vrt_render_camera", "vrt_render_camera_dev", "vrt_render_camera_async", "vrt_band_rows", "vrt_render_bands_dev", "vrt_render_bands_async",
     "vrt_trace_bands16_dev", "vrt_count_camera", "vrt_frame_bands_dev", "vrt_frame_bands_peer_dev",
     "vrt_dev_alloc", "vrt_dev_free", "vrt_host_register", "vrt_host_unregister", "vrt_ipc_export", "vrt_ipc_open", "vrt_ipc_close", "vrt_tree_sync",
-    "vrt_last_kernel_ms", "vrt_mean_kernel_ms", "vrt_debug_general_order_calls", "vrt_debug_param_check", "vrt_debug_pair_total", "vrt_debug_set_hull", "vrt_debug_hull_stats", "vrt_build_ex", "vrt_mgpu_create", "vrt_mgpu_num_devices",
+    "vrt_last_kernel_ms", "vrt_mean_kernel_ms", "vrt_debug_general_order_calls", "vrt_debug_param_check", "vrt_debug_pair_total", "vrt_debug_set_hull", "vrt_debug_set_eye_rel", "vrt_debug_eye_rel_launches", "vrt_debug_hull_stats", "vrt_build_ex", "vrt_mgpu_create", "vrt_mgpu_num_devices",
     "vrt_mgpu_render_async", "vrt_mgpu_sync", "vrt_mgpu_render", "vrt_mgpu_free", "vrt_set_film_format",
     "vrt_film_pixel_bytes", "vrt_hdr_file", "vrt_mgpu_set_film_format", "vrt_film_encode", "vrt_set_materials", "vrt_albedo", "vrt_gi_init", "vrt_gi_splat_camera", "vrt_gi_filter",
     "vrt_gi_get_level", "vrt_gi_cone_trace", "vrt_gi_render_camera", "vrt_gi_render_camera_dev", "vrt_tribox_batch",
@@ -160,6 +160,8 @@ def load(build_if_missing: bool = True):
     L.vrt_debug_param_check.argtypes = [vp]
     L.vrt_debug_pair_total.argtypes = [vp, u64, vp]
     L.vrt_debug_set_hull.argtypes = [vp, i32]
+    L.vrt_debug_set_eye_rel.argtypes = [vp, i32]
+    L.vrt_debug_eye_rel_launches.argtypes = [vp, vp]
     L.vrt_debug_hull_stats.argtypes = [vp]
     L.vrt_mgpu_create.argtypes = [vp, i32, vp, C.POINTER(vp)]
     L.vrt_mgpu_num_devices.argtypes = [vp]
@@ -508,6 +510,16 @@ class Octree:
     def debug_set_hull(self, on: bool):
         """Test hook: content-hull pruning of the ray kernels off / on for this handle."""
         _check(load().vrt_debug_set_hull(self._h, 1 if on else 0))
+
+    def debug_set_eye_rel(self, on: bool):
+        """Test hook: eye-relative hull records and triangle terms of the camera launches on / off for this handle."""
+        _check(load().vrt_debug_set_eye_rel(self._h, 1 if on else 0))
+
+    def debug_eye_rel_launches(self):
+        """Test hook: camera launches of this handle that read eye-relative records so far."""
+        n = C.c_uint64()
+        _check(load().vrt_debug_eye_rel_launches(self._h, C.byref(n)))
+        return int(n.value)
 
     def mean_kernel_ms(self, last_n):
         return float(load().vrt_mean_kernel_ms(self._h, int(last_n)))

@@ -562,7 +562,7 @@ using namespace vrt;
 uint64_t vrt_tree::scratch_bytes() const
 {
         uint64_t b = keys_a.cap + keys_b.cap + tmp_a.cap + tmp_b.cap + tmp_c.cap + hist.cap + refs_s.cap + tab_s.cap +
-                     io_in.cap + io_out.cap + hull_buf.cap + tri64_buf.cap;
+                     io_in.cap + io_out.cap + hull_buf.cap + tri64_buf.cap + eyerel_buf.cap;
         for (unsigned l = 0; l <= VRT_MAX_DEPTH; ++l)
                 b += level_morton[l].cap + level_first[l].cap + level_mask[l].cap;
         return b;
@@ -657,11 +657,18 @@ void vrt_tree_free(vrt_tree* t)
         t->gi_steps[0].release();
         t->gi_steps[1].release();
         t->tabrel_buf.release();
+        t->eyerel_buf.release();
+        auto free_slot_events = [](vrt_tree::RelSlot& s) {
+                if (s.ev)
+                        cudaEventDestroy(s.ev);
+                for (cudaEvent_t e : s.read_ev)
+                        if (e)
+                                cudaEventDestroy(e);
+        };
         for (auto& rs : t->tabrel_slot)
-                if (rs.ev) {
-                        cudaEventDestroy(rs.ev);
-                        cudaEventDestroy(rs.ev_read);
-                }
+                free_slot_events(rs);
+        for (auto& rs : t->eyerel_slot)
+                free_slot_events(rs);
         t->mat_buf.release();
         t->io_out.release();
         t->film_dev[0].release();
@@ -2363,6 +2370,28 @@ int vrt_debug_set_hull(vrt_tree* t, int on)
                 return rc;
         VRT_CUDA(cudaStreamSynchronize(t->stream));
         t->dev.rec_mask = on ? 0xffffu : 0x00ffu;
+        return VRT_OK;
+}
+
+int vrt_debug_set_eye_rel(vrt_tree* t, int on)
+{
+        int rc = check_tree(t);
+        if (rc)
+                return rc;
+        t->eyerel_on = on != 0;
+        return VRT_OK;
+}
+
+int vrt_debug_eye_rel_launches(const vrt_tree* t, uint64_t* out)
+{
+        int rc = check_tree(t);
+        if (rc)
+                return rc;
+        if (!out) {
+                set_error("null out");
+                return VRT_ERR_ARG;
+        }
+        *out = t->n_eyerel_launches;
         return VRT_OK;
 }
 

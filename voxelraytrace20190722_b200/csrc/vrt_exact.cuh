@@ -399,6 +399,41 @@ __device__ __forceinline__ int ray_triangle3_edges(const double o[3], const doub
         return 1;
 }
 
+// ray_triangle3_edges for a ray whose origin o is known before the launch: tv = o - a, qv = tv x e1 and tq = e2 . qv
+// depend on (o, triangle) only and come precomputed with the same operations (k_tri_eye_rel); branches, the 1/det
+// and the results are those of ray_triangle3_edges.
+__device__ __forceinline__ int ray_triangle3_eye(const double dir[3], const double e1[3], const double e2[3],
+                                                 const double tv[3], const double qv[3], double tq, double& t,
+                                                 double& u, double& v)
+{
+        const double eps = 0.000001;
+        double pv[3];
+        dcross(pv, dir, e2);
+        double det = ddot3(e1, pv);
+        if (det > eps) {
+                u = ddot3(tv, pv);
+                if (u < 0.0 || u > det)
+                        return 0;
+                v = ddot3(dir, qv);
+                if (v < 0.0 || dadd(u, v) > det)
+                        return 0;
+        } else if (det < -eps) {
+                u = ddot3(tv, pv);
+                if (u > 0.0 || u < det)
+                        return 0;
+                v = ddot3(dir, qv);
+                if (v > 0.0 || dadd(u, v) < det)
+                        return 0;
+        } else {
+                return 0;
+        }
+        double inv = __ddiv_rn(1.0, det);
+        t = dmul(tq, inv);
+        u = dmul(u, inv);
+        v = dmul(v, inv);
+        return 1;
+}
+
 // ---------------------------------------------------------------------------
 // AABB<Vec3>::isect(ray, nullptr) (graphics_math.h:1312-1332)
 // ---------------------------------------------------------------------------

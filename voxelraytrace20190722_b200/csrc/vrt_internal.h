@@ -2,6 +2,7 @@
 // translation units of libvrt.so.  Not part of the public ABI.
 #pragma once
 
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <string>
@@ -186,14 +187,20 @@ struct vrt_tree {
         mutable void* l2_window_stream = nullptr;
         mutable const void* l2_window_nodes = nullptr;
         mutable uint64_t l2_window_bytes = 0;
-        // origin-relative axis tables of the camera launches (vrt_trace.cu tab_rel_for_launch)
+        // origin-relative axis tables of the camera launches (vrt_trace.cu tab_rel_for_launch), one per eye
         static constexpr int kRelSlots = 8;
         struct RelSlot {
                 float eye[3] = { 0, 0, 0 };
                 bool valid = false, done = false;
-                cudaEvent_t ev = nullptr, ev_read = nullptr;  // table filled / last launch that reads it enqueued
+                cudaEvent_t ev = nullptr;  // table filled
                 cudaStream_t stream = nullptr;
                 uint64_t last_use = 0;
+                // the launches that read the slot since its fill: per reading stream, an event recorded after that
+                // stream's last reading launch (a refill waits for all of them; vrt_trace.cu rel_slot_read)
+                static constexpr int kReaders = 4;
+                int n_read = 0;
+                cudaStream_t read_stream[kReaders] = {};
+                cudaEvent_t read_ev[kReaders] = {};
         };
         mutable uint64_t tabrel_clock = 0;
         mutable int tabrel_cur = 0;
@@ -201,6 +208,19 @@ struct vrt_tree {
         mutable RelSlot tabrel_slot[kRelSlots];
         mutable const void* tabrel_blob = nullptr;
         mutable uint64_t tabrel_build = ~0ull;
+        // eye-relative hull records and triangle terms of the camera launches (vrt_trace.cu eye_rel_for_launch): two
+        // slots, so that the frames of a moving camera can alternate between the two kernel streams
+        static constexpr int kEyeRelSlots = 2;
+        mutable uint64_t eyerel_clock = 0;
+        mutable int eyerel_cur = 0;
+        mutable vrt::Scratch eyerel_buf;
+        mutable RelSlot eyerel_slot[kEyeRelSlots];
+        mutable const void* eyerel_blob = nullptr;
+        mutable uint64_t eyerel_build = ~0ull;
+        bool eyerel_on = true;  // vrt_debug_set_eye_rel
+        mutable bool eyerel_nomem = false;  // the slots did not fit for (eyerel_blob, eyerel_build): not retried
+        mutable uint64_t n_eyerel_launches = 0;  // camera launches that read the records (vrt_debug_eye_rel_launches)
+        mutable float eyerel_last[3] = { NAN, NAN, NAN };  // eye of the last camera launch (never equal before one)
         uint64_t n_builds = 0;  // bumped whenever the blob's contents change (tree_bind_views)
         int film_fmt = 0;  // VRT_FILM_* of every film this handle's kernels write (vrt_set_film_format)
         double build_ms = 0;

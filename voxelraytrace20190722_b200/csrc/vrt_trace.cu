@@ -41,6 +41,9 @@ namespace vrt {
 #ifndef VRT_EYE_ALL
 #define VRT_EYE_ALL 0
 #endif
+#ifndef VRT_ER_EYE
+#define VRT_ER_EYE 1
+#endif
 constexpr int kTraceThreads = VRT_TRACE_THREADS;
 #ifndef VRT_TILE_BLOCK_LOG
 #define VRT_TILE_BLOCK_LOG 3
@@ -78,6 +81,10 @@ struct TraceParams {
         // (k_tab_rel: the reference's (plane - o) of every slab test, evaluated once per table entry instead of once
         // per ray and node); null: the expansion subtracts itself
         const float4* tabrel[3];
+        // camera modes, k_trace_camera<.., ER = true>: the hull records and the triangle terms relative to eye
+        // (k_hull_eye_rel, k_tri_eye_rel)
+        const float4* hull_eye;
+        const double* tri_eye;
         vrt_gi_aov aov;  // OUT_GI_AOV: the per-pixel planes (include/vrt.h); a null member is not written
 };
 
@@ -99,11 +106,17 @@ struct WorkCount {
         uint32_t n_param, n_tie, n_unsafe;
 };
 
+// Eye-relative triangle terms of a camera launch (k_tri_eye_rel): per triangle 14 doubles (112 bytes, seven 16-byte
+// loads) e2, e1, tv = eye - v0, qv = tv x e1, tq = e2 . qv, pad.
+constexpr uint32_t kTriEyeDoubles = 14;
+
 // Triangle::isect + ray_march_isect for one leaf (voxel_octree.cc:99-129,438-460); rec = the leaf's node
-// record {first reference, reference count}.
-template <bool COUNT>
+// record {first reference, reference count}.  EYE: the terms come from tri_eye, the launch's eye-relative triangle
+// terms (o is then the launch's eye).
+template <bool COUNT, bool EYE = false>
 __device__ __forceinline__ bool leaf_isect_rec(const TreeDev& tr, const uint2 rec, const float o[3],
-                                               const float d[3], HitState& hs, WorkCount& wc)
+                                               const float d[3], HitState& hs, WorkCount& wc,
+                                               const double* tri_eye = nullptr)
 {
         if (COUNT) {
                 wc.n_leaf += 1;
@@ -116,7 +129,16 @@ __device__ __forceinline__ bool leaf_isect_rec(const TreeDev& tr, const uint2 re
         for (uint32_t i = 0; i < rec.y; ++i) {
                 const uint32_t ti = __ldg(&tr.leaf_refs[rec.x + i]);
                 double dt, du, dv;
-                {  // v0, e1, e2 already widened and subtracted (k_tri64, every tree with triangles has them)
+                if (EYE) {
+                        const double2* q = reinterpret_cast<const double2*>(tri_eye + kTriEyeDoubles * (uint64_t)ti);
+                        const double2 q0 = __ldg(q), q1 = __ldg(q + 1), q2 = __ldg(q + 2), q3 = __ldg(q + 3);
+                        const double2 q4 = __ldg(q + 4), q5 = __ldg(q + 5);
+                        const double tq = __ldg(tri_eye + kTriEyeDoubles * (uint64_t)ti + 12);
+                        const double e2[3] = { q0.x, q0.y, q1.x }, e1[3] = { q1.y, q2.x, q2.y };
+                        const double tv[3] = { q3.x, q3.y, q4.x }, qv[3] = { q4.y, q5.x, q5.y };
+                        if (ray_triangle3_eye(dd, e1, e2, tv, qv, tq, dt, du, dv) != 1)
+                                continue;
+                } else {  // v0, e1, e2 already widened and subtracted (k_tri64, every tree with triangles has them)
                         const double2* q = reinterpret_cast<const double2*>(tr.tri64 + 10ull * ti);  // 80-byte records
                         const double2 q0 = __ldg(q), q1 = __ldg(q + 1), q2 = __ldg(q + 2), q3 = __ldg(q + 3);
                         const double q4 = __ldg(tr.tri64 + 10ull * ti + 8);
@@ -534,13 +556,15 @@ __device__ unsigned long long g_hull_stats[20][4];
 // over the node's content hull (TreeDev::hull) against the window, as an OVERLAP test: every leaf
 // cell below lies inside the hull plane by plane and rounding is monotone, so a leaf that passes the
 // reference's slab test implies max(t0,tmin) <= min(t1,tmax) here.  false = the subtree cannot
-// produce a hit; skipping it changes no result.
+// produce a hit; skipping it changes no result.  ER: the record is eye-relative (k_hull_eye_rel: the planes already
+// minus the launch's eye, which is o), so only the products remain.
+template <bool ER = false>
 __device__ __forceinline__ bool hull_reachable(const float4 ha, const float4 hb, const float o[3], const float dinv[3],
                                                float tmin, float tmax, float& t0, float& t1)
 {
-        const float2 ax = mul2s(sub2s(ha.z, ha.w, o[0]), dinv[0]);
-        const float2 ay = mul2s(sub2s(hb.x, hb.y, o[1]), dinv[1]);
-        const float2 az = mul2s(sub2s(hb.z, hb.w, o[2]), dinv[2]);
+        const float2 ax = mul2s(ER ? make_float2(ha.z, ha.w) : sub2s(ha.z, ha.w, o[0]), dinv[0]);
+        const float2 ay = mul2s(ER ? make_float2(hb.x, hb.y) : sub2s(hb.x, hb.y, o[1]), dinv[1]);
+        const float2 az = mul2s(ER ? make_float2(hb.z, hb.w) : sub2s(hb.z, hb.w, o[2]), dinv[2]);
         t0 = fmax3(fminf(ax.x, ax.y), fminf(ay.x, ay.y), fminf(az.x, az.y));
         t1 = fmin3(fmaxf(ax.x, ax.y), fmaxf(ay.x, ay.y), fmaxf(az.x, az.y));
         return fmaxf(t0, tmin) <= fminf(t1, tmax);
@@ -558,12 +582,16 @@ __device__ __forceinline__ bool hull_reachable(const float4 ha, const float4 hb,
 // not key-safe (param_safe_levels), the node is expanded by expand_slab instead.  Each cell
 // knows its own t0 (entry breakpoint) and t1 (next breakpoint), so the reference's window test
 // slab_accept(t0,t1,tmin,tmax) is evaluated on the same values.
-template <bool COUNT, bool REL>
+// ER (camera launches, o = the launch's eye): the hull records are read from hull_eye and the leaf tests take
+// their eye-dependent terms from tri_eye (EyeRel below) instead of subtracting the origin per ray.
+template <bool COUNT, bool REL, bool ER>
 __device__ __forceinline__ void trace_one_fast(const TreeDev& tr, const float root[6], const float o[3],
                                                const float d[3], float tmin, float tmax, uint32_t* s_first,
                                                uint32_t* s_meta, uint32_t* s_list, HitState& hs, WorkCount& wc,
-                                               const float4* const* rel)
+                                               const float4* const* rel, const float4* hull_eye,
+                                               const double* tri_eye)
 {
+        const float4* const hull = ER ? hull_eye : tr.hull;
         float dinv[3];
 #pragma unroll
         for (int k = 0; k < 3; ++k)
@@ -604,7 +632,7 @@ __device__ __forceinline__ void trace_one_fast(const TreeDev& tr, const float ro
         // = 0x00ff clears the flags -- the "hulls off" switch of the tests)
         uint2 rec;
         if (!COUNT) {
-                const float4 h0 = __ldg(&tr.hull[0]);
+                const float4 h0 = __ldg(&hull[0]);
                 rec = make_uint2(__float_as_uint(h0.x), __float_as_uint(h0.y) & tr.rec_mask);
         } else {
                 rec = __ldg(&tr.nodes[0]);
@@ -764,7 +792,7 @@ __device__ __forceinline__ void trace_one_fast(const TreeDev& tr, const float ro
                         const uint32_t cy = 2u * y + ((c >> 1) & 1u);
                         const uint32_t cz = 2u * z + (c & 1u);
                         if (level + 1 == L) {
-                                if (leaf_isect<COUNT>(tr, child, o, d, hs, wc)) {
+                                if (leaf_isect_rec<COUNT, ER>(tr, __ldg(&tr.nodes[child]), o, d, hs, wc, tri_eye)) {
                                         hs.hit = true;
                                         hs.leaf = child;
                                         hs.cx = cx - (1u << L);
@@ -784,16 +812,16 @@ __device__ __forceinline__ void trace_one_fast(const TreeDev& tr, const float ro
                         atomicAdd(&g_hull_stats[level][1], 1ull);
 #endif
                         if (!COUNT) {
-                                const float4 ha = __ldg(&tr.hull[2ull * child]);
+                                const float4 ha = __ldg(&hull[2ull * child]);
                                 if ((mask >> (8u + c)) & 1u) {
-                                        const float4 hb = __ldg(&tr.hull[2ull * child + 1]);
+                                        const float4 hb = __ldg(&hull[2ull * child + 1]);
                                         float h0, h1;
 #ifdef VRT_HULL_STATS
                                         atomicAdd(&g_hull_stats[level][2], 1ull);
-                                        if (!hull_reachable(ha, hb, o, dinv, tmin, tmax, h0, h1))
+                                        if (!hull_reachable<ER>(ha, hb, o, dinv, tmin, tmax, h0, h1))
                                                 atomicAdd(&g_hull_stats[level][3], 1ull);
 #endif
-                                        if (!hull_reachable(ha, hb, o, dinv, tmin, tmax, h0, h1))
+                                        if (!hull_reachable<ER>(ha, hb, o, dinv, tmin, tmax, h0, h1))
                                                 continue;
                                 }
                                 rec = make_uint2(__float_as_uint(ha.x), __float_as_uint(ha.y) & tr.rec_mask);
@@ -818,11 +846,12 @@ __device__ __forceinline__ void trace_one_fast(const TreeDev& tr, const float ro
         }
 }
 
-template <bool COUNT, bool REL = false>
+template <bool COUNT, bool REL = false, bool ER = false>
 __device__ __forceinline__ void trace_one(const TreeDev& tr, const float root[6], const float o[3],
                                           const float d[3], float tmin, float tmax, uint32_t* s_first,
                                           uint32_t* s_meta, uint32_t* s_list, HitState& hs, WorkCount& wc,
-                                          const float4* const* rel = nullptr)
+                                          const float4* const* rel = nullptr, const float4* hull_eye = nullptr,
+                                          const double* tri_eye = nullptr)
 {
         hs.hit = false;
         hs.tri = VRT_NO_TRI;
@@ -832,7 +861,8 @@ __device__ __forceinline__ void trace_one(const TreeDev& tr, const float root[6]
         if (tr.num_nodes == 0)
                 return;
         if (ray_is_tame(tr, o, d))
-                trace_one_fast<COUNT, REL>(tr, root, o, d, tmin, tmax, s_first, s_meta, s_list, hs, wc, rel);
+                trace_one_fast<COUNT, REL, ER>(tr, root, o, d, tmin, tmax, s_first, s_meta, s_list, hs, wc, rel, hull_eye,
+                                               tri_eye);
         else
                 trace_one_exact<COUNT>(tr, root, o, d, tmin, tmax, s_first, s_meta, s_list, hs, wc);
 }
@@ -1252,11 +1282,14 @@ k_trace_rays(const __grid_constant__ TraceParams p)
         }
 }
 
-// Every mode runs best at 72 registers (7 CTAs/SM).  Round 1 had the compact outputs at 64 registers (8 CTAs/SM);
+// Round 2: every mode ran best at 72 registers (7 CTAs/SM).  Round 1 had the compact outputs at 64 registers (8 CTAs/SM);
 // since the tiles of an SM are neighbours on the film (per-SM queues below: L1 hit rate 73 -> 87 %) the warps wait
 // less on memory, and the 1/d values that 64 registers push into local memory (re-read in every expansion and hull
 // test) cost more than the eighth CTA hides: hit16 5.92 -> 5.72 ms per headline frame.
-template <int MODE, bool WS>
+template <int MODE, bool WS, bool ER>
+// Round 3: the instantiations with eye-relative records (ER: the film, hit16 and hit16 + film modes) no longer need
+// the origin in registers during the traversal, and one more CTA per SM (64 registers) is faster for them: headline
+// frame 5.51 -> 5.39 ms (B200, DESIGN.md section 5).
 #ifndef VRT_FILM_MIN_BLOCKS
 #define VRT_FILM_MIN_BLOCKS 7
 #endif
@@ -1266,9 +1299,9 @@ template <int MODE, bool WS>
 #ifndef VRT_GI_MIN_BLOCKS
 #define VRT_GI_MIN_BLOCKS 5
 #endif
-__global__ void __launch_bounds__(kTraceThreads, (MODE == OUT_HIT16 || MODE == OUT_COUNT) ? VRT_HIT16_MIN_BLOCKS
+__global__ void __launch_bounds__(kTraceThreads, (MODE == OUT_HIT16 || MODE == OUT_COUNT) ? VRT_HIT16_MIN_BLOCKS + (ER ? 1 : 0)
                                                  : (MODE == OUT_GI_FILM || MODE == OUT_GI_AOV) ? VRT_GI_MIN_BLOCKS
-                                                                                          : VRT_FILM_MIN_BLOCKS)
+                                                                                          : VRT_FILM_MIN_BLOCKS + (ER ? 1 : 0))
 k_trace_camera(const __grid_constant__ TraceParams p)
 {
         extern __shared__ uint32_t s_stack[];
@@ -1424,8 +1457,9 @@ k_trace_camera(const __grid_constant__ TraceParams p)
                 } else if (active) {
                         // the common origin comes precomputed from the host in the record-only modes (-3.5 % there);
                         // the film modes keep computing it (measured: with it precomputed ptxas spills more in those
-                        // instantiations and the frame step gets 5 % slower)
-                        if (VRT_EYE_ALL || MODE == OUT_HIT16 || MODE == OUT_HIT48) {
+                        // instantiations and the frame step gets 5 % slower) unless the eye-relative records are in use
+                        // (ER: the traversal then needs the origin only in the rare slab fallback and the hit distance)
+                        if (VRT_EYE_ALL || MODE == OUT_HIT16 || MODE == OUT_HIT48 || (ER && VRT_ER_EYE)) {
                                 o[0] = p.eye[0];
                                 o[1] = p.eye[1];
                                 o[2] = p.eye[2];
@@ -1434,8 +1468,9 @@ k_trace_camera(const __grid_constant__ TraceParams p)
                                 gen_ray(p.cam, px, py, s, o, d);
                         }
                         // (every camera launch carries the origin-relative plane table, see launch_trace_camera)
-                        trace_one<MODE == OUT_COUNT, MODE != OUT_COUNT>(p.tree, p.root, o, d, p.cam.tmin, p.cam.tmax, s_first,
-                                                                        s_meta, s_list, hs, wc, p.tabrel);
+                        trace_one<MODE == OUT_COUNT, MODE != OUT_COUNT, ER>(p.tree, p.root, o, d, p.cam.tmin, p.cam.tmax,
+                                                                            s_first, s_meta, s_list, hs, wc, p.tabrel,
+                                                                            p.hull_eye, p.tri_eye);
                 }
                 const unsigned long long pix = (unsigned long long)ry * W + (px - p.x0);
                 if (MODE == OUT_HIT48) {
@@ -1562,51 +1597,77 @@ __global__ void __launch_bounds__(256) k_tab_rel(const float4* __restrict__ tab,
         rel[i] = make_float4(fsub(t.x, e), fsub(t.y, e), fsub(t.z, e), fsub(t.w, e));
 }
 
-// The table for (tree contents, eye), cached per handle: a frame loop with a fixed camera builds it once.  Slots are
-// reused round-robin by launch number (launches of consecutive frames may overlap on two streams); a launch on
-// another stream than the one that filled the slot waits for the fill through the slot's event.
-static int tab_rel_for_launch(const vrt_tree* t, const float eye[3], cudaStream_t ls, const float4* out[3])
+// Eye-relative hull records of a camera launch: the records of TreeDev::hull (n interior nodes) with their six planes
+// minus the eye -- fsub, the (plane - o) of hull_reachable rounded once -- and the first-child and mask words unchanged,
+// so that a record is still the node record of the expansion.
+__global__ void __launch_bounds__(256) k_hull_eye_rel(const float4* __restrict__ hull, uint64_t n, float ex, float ey,
+                                                      float ez, float4* __restrict__ out)
 {
-        const uint64_t n4 = t->hdr.axis_tab_stride / 2;  // float4 entries per axis
-        const uint64_t slot_bytes = 3 * n4 * sizeof(float4);
-        if (t->tabrel_buf.cap < vrt_tree::kRelSlots * slot_bytes || t->tabrel_blob != t->blob ||
-            t->tabrel_build != t->n_builds) {
-                VRT_CUDA(cudaDeviceSynchronize());  // (first launch after a build: nothing may still read the old tables)
-                if (t->tabrel_buf.reserve(vrt_tree::kRelSlots * slot_bytes))
-                        return VRT_ERR_NOMEM;
-                for (auto& s : t->tabrel_slot)
-                        s.valid = false;
-                t->tabrel_blob = t->blob;
-                t->tabrel_build = t->n_builds;
-        }
+        const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+        if (i >= n)
+                return;
+        const float4 a = hull[2 * i], b = hull[2 * i + 1];
+        out[2 * i] = make_float4(a.x, a.y, fsub(a.z, ex), fsub(a.w, ex));
+        out[2 * i + 1] = make_float4(fsub(b.x, ey), fsub(b.y, ey), fsub(b.z, ez), fsub(b.w, ez));
+}
+
+// Eye-relative triangle terms (kTriEyeDoubles per triangle, see leaf_isect_rec): from tri64's v0, e1, e2 the tv, qv and
+// e2 . qv that ray_triangle3_edges evaluates for a ray from the eye, with its operations in its order.
+__global__ void __launch_bounds__(256) k_tri_eye_rel(const double* __restrict__ tri64, uint32_t T, float ex, float ey,
+                                                     float ez, double* __restrict__ out)
+{
+        const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+        if (t >= T)
+                return;
+        const double* q = tri64 + 10ull * t;
+        const double a[3] = { q[0], q[1], q[2] }, e1[3] = { q[3], q[4], q[5] }, e2[3] = { q[6], q[7], q[8] };
+        const double o[3] = { (double)ex, (double)ey, (double)ez };
+        double tv[3], qv[3];
+#pragma unroll
+        for (int k = 0; k < 3; ++k)
+                tv[k] = dsub(o[k], a[k]);
+        dcross(qv, tv, e1);
+        const double r[kTriEyeDoubles] = { e2[0], e2[1], e2[2], e1[0], e1[1], e1[2], tv[0],
+                                           tv[1], tv[2], qv[0], qv[1], qv[2], ddot3(e2, qv), 0.0 };
+        double2* w = reinterpret_cast<double2*>(out + kTriEyeDoubles * (uint64_t)t);
+#pragma unroll
+        for (int k = 0; k < (int)kTriEyeDoubles / 2; ++k)
+                w[k] = make_double2(r[2 * k], r[2 * k + 1]);
+}
+
+// The slot of `slots` whose records are those of `eye`: a slot that holds them, else the least recently used one,
+// refilled on `ls` by fill(k) once every launch that read it since its last fill (on any stream, rel_slot_read) is
+// done.  Launches of consecutive frames may overlap on two streams: a launch on another stream than the one that
+// filled the slot waits for the fill through the slot's event.
+template <class Fill>
+static int rel_slot_for_launch(vrt_tree::RelSlot* slots, int n, uint64_t& clock, const float eye[3], cudaStream_t ls,
+                               Fill fill, int* out)
+{
         int k = -1;
-        for (int i = 0; i < vrt_tree::kRelSlots; ++i)
-                if (t->tabrel_slot[i].valid && memcmp(t->tabrel_slot[i].eye, eye, 12) == 0)
+        for (int i = 0; i < n; ++i)
+                if (slots[i].valid && memcmp(slots[i].eye, eye, 12) == 0)
                         k = i;
         if (k < 0) {
-                // least recently used slot; its last reader (possibly queued on the other stream) goes first
                 k = 0;
-                for (int i = 1; i < vrt_tree::kRelSlots; ++i)
-                        if (t->tabrel_slot[i].last_use < t->tabrel_slot[k].last_use)
+                for (int i = 1; i < n; ++i)
+                        if (slots[i].last_use < slots[k].last_use)
                                 k = i;
-                auto& s = t->tabrel_slot[k];
-                if (!s.ev) {
+                auto& s = slots[k];
+                if (!s.ev)
                         VRT_CUDA(cudaEventCreateWithFlags(&s.ev, cudaEventDisableTiming));
-                        VRT_CUDA(cudaEventCreateWithFlags(&s.ev_read, cudaEventDisableTiming));
-                } else if (s.valid) {
-                        VRT_CUDA(cudaStreamWaitEvent(ls, s.ev_read, 0));
-                }
-                float4* dst = reinterpret_cast<float4*>(static_cast<char*>(t->tabrel_buf.p) + k * slot_bytes);
-                k_tab_rel<<<(unsigned)((3 * n4 + 255) / 256), 256, 0, ls>>>(t->dev.tab4[0], (uint32_t)n4, eye[0], eye[1], eye[2], dst);
-                count_launch();
-                VRT_CUDA(cudaGetLastError());
+                for (int i = 0; i < s.n_read; ++i)
+                        VRT_CUDA(cudaStreamWaitEvent(ls, s.read_ev[i], 0));
+                s.n_read = 0;
+                s.valid = false;
+                if (int rc = fill(k))
+                        return rc;
                 VRT_CUDA(cudaEventRecord(s.ev, ls));
                 memcpy(s.eye, eye, 12);
                 s.valid = true;
                 s.done = false;
                 s.stream = ls;
         }
-        auto& s = t->tabrel_slot[k];
+        auto& s = slots[k];
         if (!s.done) {
                 if (cudaEventQuery(s.ev) == cudaSuccess)
                         s.done = true;
@@ -1614,11 +1675,130 @@ static int tab_rel_for_launch(const vrt_tree* t, const float eye[3], cudaStream_
                         VRT_CUDA(cudaStreamWaitEvent(ls, s.ev, 0));
                 cudaGetLastError();  // (cudaErrorNotReady is not an error here)
         }
-        s.last_use = ++t->tabrel_clock;
+        s.last_use = ++clock;
+        *out = k;
+        return VRT_OK;
+}
+
+// After a launch on `ls` that reads slot s: the slot's read event of that stream is recorded behind it.  When every
+// entry belongs to another stream, this stream takes over entry 0 after waiting for its event, so that the new event
+// still completes only after that stream's readers.
+static int rel_slot_read(vrt_tree::RelSlot& s, cudaStream_t ls)
+{
+        int i = 0;
+        while (i < s.n_read && s.read_stream[i] != ls)
+                ++i;
+        if (i == vrt_tree::RelSlot::kReaders) {
+                i = 0;
+                VRT_CUDA(cudaStreamWaitEvent(ls, s.read_ev[0], 0));
+        } else if (i == s.n_read) {
+                s.n_read++;
+        }
+        if (!s.read_ev[i])
+                VRT_CUDA(cudaEventCreateWithFlags(&s.read_ev[i], cudaEventDisableTiming));
+        s.read_stream[i] = ls;
+        VRT_CUDA(cudaEventRecord(s.read_ev[i], ls));
+        return VRT_OK;
+}
+
+// The origin-relative axis tables for (tree contents, eye), cached per handle: a frame loop with a fixed camera builds
+// them once.
+static int tab_rel_for_launch(const vrt_tree* t, const float eye[3], cudaStream_t ls, const float4* out[3])
+{
+        const uint64_t n4 = t->hdr.axis_tab_stride / 2;  // float4 entries per axis
+        const uint64_t slot_bytes = 3 * n4 * sizeof(float4);
+        if (t->tabrel_buf.cap < vrt_tree::kRelSlots * slot_bytes || t->tabrel_blob != t->blob ||
+            t->tabrel_build != t->n_builds) {
+                VRT_CUDA(cudaDeviceSynchronize());  // (first launch after a build: nothing may still read the old tables)
+                for (auto& s : t->tabrel_slot) {
+                        s.valid = false;
+                        s.n_read = 0;
+                }
+                if (t->tabrel_buf.reserve(vrt_tree::kRelSlots * slot_bytes))
+                        return VRT_ERR_NOMEM;
+                t->tabrel_blob = t->blob;
+                t->tabrel_build = t->n_builds;
+        }
+        auto fill = [&](int k) -> int {
+                float4* dst = reinterpret_cast<float4*>(static_cast<char*>(t->tabrel_buf.p) + k * slot_bytes);
+                k_tab_rel<<<(unsigned)((3 * n4 + 255) / 256), 256, 0, ls>>>(t->dev.tab4[0], (uint32_t)n4, eye[0], eye[1], eye[2], dst);
+                count_launch();
+                VRT_CUDA(cudaGetLastError());
+                return VRT_OK;
+        };
+        int k = 0;
+        if (int rc = rel_slot_for_launch(t->tabrel_slot, vrt_tree::kRelSlots, t->tabrel_clock, eye, ls, fill, &k))
+                return rc;
         t->tabrel_cur = k;
         const float4* base = reinterpret_cast<const float4*>(static_cast<const char*>(t->tabrel_buf.p) + k * slot_bytes);
         for (int a = 0; a < 3; ++a)
                 out[a] = base + a * n4;
+        return VRT_OK;
+}
+
+// The eye-relative hull records and triangle terms for (tree contents, eye), cached per handle like the tables above
+// (fewer slots: a slot is 32 bytes per interior node and 112 per triangle).  vrt_update_* rebuilds, which bumps n_builds.
+// VRT_ERR_NOMEM: no room for the slots; the caller launches with the absolute records instead, and the reservation is
+// not tried again before the next build.
+static uint64_t eye_rel_hull_bytes(const vrt_tree* t)
+{
+        return align256((t->hdr.num_nodes - t->hdr.num_leaves) * 2 * sizeof(float4));
+}
+static uint64_t eye_rel_slot_bytes(const vrt_tree* t)
+{
+        return eye_rel_hull_bytes(t) + align256((uint64_t)t->hdr.num_tris * kTriEyeDoubles * sizeof(double));
+}
+static bool eye_rel_cached(const vrt_tree* t, const float eye[3])
+{
+        if (t->eyerel_blob != t->blob || t->eyerel_build != t->n_builds)
+                return false;
+        for (const auto& s : t->eyerel_slot)
+                if (s.valid && memcmp(s.eye, eye, 12) == 0)
+                        return true;
+        return false;
+}
+static int eye_rel_for_launch(const vrt_tree* t, const float eye[3], cudaStream_t ls, const float4** hull_eye,
+                              const double** tri_eye)
+{
+        const uint64_t interior = t->hdr.num_nodes - t->hdr.num_leaves, T = t->hdr.num_tris;
+        const uint64_t hull_bytes = eye_rel_hull_bytes(t), slot_bytes = eye_rel_slot_bytes(t);
+        const bool current = t->eyerel_blob == t->blob && t->eyerel_build == t->n_builds;
+        if (current && t->eyerel_nomem)
+                return VRT_ERR_NOMEM;
+        if (!current || t->eyerel_buf.cap < vrt_tree::kEyeRelSlots * slot_bytes) {
+                VRT_CUDA(cudaDeviceSynchronize());  // (first launch after a build: nothing may still read the old records)
+                for (auto& s : t->eyerel_slot) {
+                        s.valid = false;
+                        s.n_read = 0;
+                }
+                t->eyerel_blob = t->blob;
+                t->eyerel_build = t->n_builds;
+                t->eyerel_nomem = t->eyerel_buf.reserve(vrt_tree::kEyeRelSlots * slot_bytes) != 0;
+                if (t->eyerel_nomem)
+                        return VRT_ERR_NOMEM;
+        }
+        auto fill = [&](int k) -> int {
+                char* base = static_cast<char*>(t->eyerel_buf.p) + k * slot_bytes;
+                if (interior) {
+                        k_hull_eye_rel<<<(unsigned)((interior + 255) / 256), 256, 0, ls>>>(t->dev.hull, interior, eye[0], eye[1],
+                                                                                          eye[2], reinterpret_cast<float4*>(base));
+                        count_launch();
+                }
+                if (T) {
+                        k_tri_eye_rel<<<(unsigned)((T + 255) / 256), 256, 0, ls>>>(t->dev.tri64, (uint32_t)T, eye[0], eye[1], eye[2],
+                                                                                  reinterpret_cast<double*>(base + hull_bytes));
+                        count_launch();
+                }
+                VRT_CUDA(cudaGetLastError());
+                return VRT_OK;
+        };
+        int k = 0;
+        if (int rc = rel_slot_for_launch(t->eyerel_slot, vrt_tree::kEyeRelSlots, t->eyerel_clock, eye, ls, fill, &k))
+                return rc;
+        t->eyerel_cur = k;
+        const char* base = static_cast<const char*>(t->eyerel_buf.p) + k * slot_bytes;
+        *hull_eye = reinterpret_cast<const float4*>(base);
+        *tri_eye = reinterpret_cast<const double*>(base + hull_bytes);
         return VRT_OK;
 }
 
@@ -1878,33 +2058,59 @@ int launch_trace_camera(const vrt_tree* t, const CameraLaunch& l)
                 use_ws = (e && e[0] == '1') ? 1 : 0;
         }
         const bool ws = use_ws != 0;
+        cudaStream_t ls = l.stream;
+        // every camera launch but the counting mode reads the origin-relative tables; the per-ray kernels of the film
+        // and hit16 modes (the ones measured with them) also the eye-relative hull records and triangle terms, unless
+        // they are switched off or do not fit in memory
+        const bool use_rel = mode != OUT_COUNT && t->hdr.num_nodes != 0 && t->dev.L >= 1;
+        const bool er_mode = mode == OUT_HIT16 || mode == OUT_HIT16_FILM || mode == OUT_FILM;
+        bool er = false;
+        if (use_rel) {
+                const int rc = tab_rel_for_launch(t, p.eye, ls, p.tabrel);
+                if (rc)
+                        return rc;
+                // (launches with shadow rays keep them off: measured on config 5, 2048^3 8K orbit + shadow rays, with
+                // them the frame went from 56.28 to 56.59 ms on B200, DESIGN.md section 5)
+                if (!ws && er_mode && t->eyerel_on && !(l.sh && l.sh->shadow)) {
+                        // a slot fill reads and writes about a slot's bytes; it pays for itself from about one ray per
+                        // 13 slot bytes (B200, DESIGN.md section 5: the 2048^3 tree's 595 MB slot costs 0.22 ms, a ray
+                        // saves 5 ps).  Smaller launches with a new eye keep the per-ray subtraction; an eye seen by the
+                        // previous launch (a fixed camera) is filled on its second launch and reused from then on.
+                        const uint64_t rays = (uint64_t)(x1 - x0) * (uint64_t)(y1 - y0) * (uint64_t)cam->spp;
+                        if (rays * 13 >= eye_rel_slot_bytes(t) || memcmp(t->eyerel_last, p.eye, 12) == 0 ||
+                            eye_rel_cached(t, p.eye)) {
+                                const int rc2 = eye_rel_for_launch(t, p.eye, ls, &p.hull_eye, &p.tri_eye);
+                                if (rc2 && rc2 != VRT_ERR_NOMEM)
+                                        return rc2;
+                                er = rc2 == VRT_OK;
+                        }
+                        memcpy(t->eyerel_last, p.eye, 12);
+                }
+        }
         p.lut_off = (uint32_t)stack_bytes(t, mode);
         const size_t smem = stack_bytes(t, mode) + (ws ? (size_t)kWsLutBytes : 0);
         const void* kern = nullptr;
-#define VRT_PICK(M) kern = ws ? (const void*)k_trace_camera<M, true> : (const void*)k_trace_camera<M, false>
+#define VRT_PICK(M) kern = ws ? (const void*)k_trace_camera<M, true, false> : (const void*)k_trace_camera<M, false, false>
+#define VRT_PICK_ER(M) \
+        kern = er ? (const void*)k_trace_camera<M, false, true> : ws ? (const void*)k_trace_camera<M, true, false> \
+                                                                      : (const void*)k_trace_camera<M, false, false>
         switch (mode) {
         case OUT_HIT48: VRT_PICK(OUT_HIT48); break;
-        case OUT_HIT16: VRT_PICK(OUT_HIT16); break;
+        case OUT_HIT16: VRT_PICK_ER(OUT_HIT16); break;
         case OUT_COUNT: VRT_PICK(OUT_COUNT); break;
-        case OUT_HIT16_FILM: VRT_PICK(OUT_HIT16_FILM); break;
+        case OUT_HIT16_FILM: VRT_PICK_ER(OUT_HIT16_FILM); break;
         case OUT_SPLAT: VRT_PICK(OUT_SPLAT); break;
         case OUT_GI_FILM: VRT_PICK(OUT_GI_FILM); break;
         case OUT_GI_AOV: VRT_PICK(OUT_GI_AOV); break;
-        default: VRT_PICK(OUT_FILM); break;
+        default: VRT_PICK_ER(OUT_FILM); break;
         }
+#undef VRT_PICK_ER
 #undef VRT_PICK
         VRT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int grid = persistent_grid(kern, smem);
         grid = (int)std::min<uint64_t>((uint64_t)grid, (tiles + 3) / 4);
-        cudaStream_t ls = l.stream;
         if (mode == OUT_GI_FILM || mode == OUT_GI_AOV) {
                 const int rc = gi_step_table(t, l.res, ls, &p.gi_steps);
-                if (rc)
-                        return rc;
-        }
-        const bool use_rel = mode != OUT_COUNT && t->hdr.num_nodes != 0 && t->dev.L >= 1;
-        if (use_rel) {
-                const int rc = tab_rel_for_launch(t, p.eye, ls, p.tabrel);
                 if (rc)
                         return rc;
         }
@@ -1919,8 +2125,15 @@ int launch_trace_camera(const vrt_tree* t, const CameraLaunch& l)
         VRT_CUDA(cudaLaunchKernel(kern, dim3(grid), dim3(kTraceThreads), args, smem, ls));
         count_launch();
         VRT_CUDA(cudaEventRecord(t->ring1[slot], ls));
-        if (use_rel)  // (a later launch that re-fills this table slot waits for this reader)
-                VRT_CUDA(cudaEventRecord(t->tabrel_slot[t->tabrel_cur].ev_read, ls));
+        // (a later launch that re-fills these slots waits for this reader)
+        if (use_rel)
+                if (int rc = rel_slot_read(t->tabrel_slot[t->tabrel_cur], ls))
+                        return rc;
+        if (er) {
+                if (int rc = rel_slot_read(t->eyerel_slot[t->eyerel_cur], ls))
+                        return rc;
+                t->n_eyerel_launches++;
+        }
         t->n_trace_launches++;
         return VRT_OK;
 }
